@@ -2,7 +2,7 @@
 """bench.py — CSR SpMM throughput on B200 (BASELINE.json: "SpMM GFLOP/s & HBM GB/s (% roofline)
 at K=32/256, 1/2/4/8 B200 vs host CPU").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload reddit_k256] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload reddit_k256] [--impl reference] [--dump-outputs DIR]
 
 A step is one SpMM (C = A·B) of the named synthetic graph: every kernel `spmm_b200_run`
 launches, through the C ABI. For N > 1 (torchrun) A's rows are partitioned by nnz over the ranks
@@ -18,6 +18,9 @@ over NVLink (multimem.st / peer stores), every rank downloads its own block of C
 With N > 1 the line also carries, under `also`, BASELINE config 5: the products-shaped graph over the same
 ranks (SpMM alone, strong scaling) and two stacked layers with the all-gather of C done by NCCL (all-gather-v)
 and by the kernel's own epilogue (peer / multicast stores), bit-compared.
+
+`--dump-outputs DIR` (GPU arm only) writes C as the last timed step left it to DIR/C.npy, with its row numbers in
+DIR/C_rows.npy; above DUMP_BYTES a fixed, seeded sample of rows (see dump_outputs).
 
 `--impl reference` times the CPU restatement of the reference's SpMM (oracle/spmm_oracle.c,
 OpenMP over rows — the reference itself has no CPU path: PA4/handout/src/spmm_ref.cu is a CUDA
@@ -53,6 +56,7 @@ WORKLOADS = {
 SEED = 123
 L2_BYTES = 126 << 20
 NVLINK_PEER_GBS = 770.0   # measured peer copy per direction (B200_PROFILING.md)
+DUMP_BYTES = 48 << 20     # --dump-outputs writes at most this much (C, or a seeded sample of its rows)
 
 
 def bytes_min(m, nnz, k, b_rows=None):
@@ -344,6 +348,27 @@ def timed_steps(ctx, fn, steps, flush):
     return np.asarray([a.elapsed_time(b) for a, b in evs])
 
 
+def dump_outputs(ctx, sh, vout, directory):
+    """--dump-outputs: C = A·B as a caller of the timed path receives it, written as DIR/C.npy (float32, one row of C
+    per line) with the row numbers in DIR/C_rows.npy (float64). A C larger than DUMP_BYTES is a fixed, seeded sample
+    of its rows, so that two builds run with the same arguments can be compared output for output. With N > 1 the
+    ranks' row blocks are all-gathered first (collective: every rank calls this)."""
+    torch = ctx.torch
+    m, k = sh.num_v, sh.feat
+    full = vout
+    if ctx.world > 1:
+        full = torch.empty(m * k, dtype=torch.float32, device=ctx.dev)
+        sh.allgather(vout, full)
+    if ctx.rank != 0:
+        return
+    n = min(m, DUMP_BYTES // (4 * k + 8))
+    rows = np.arange(m) if n == m else np.sort(np.random.default_rng(SEED).choice(m, n, replace=False))
+    c = full[: m * k].view(m, k)[torch.from_numpy(rows).to(ctx.dev)].cpu().numpy()
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "C.npy"), c)
+    np.save(os.path.join(directory, "C_rows.npy"), rows.astype(np.float64))
+
+
 def build_sharded(ctx, H, shape, k, opts, graph=None):
     """Graph, nnz-balanced row partition (SURVEY.md §8e), this rank's operator over its block with B replicated."""
     from hpc_b200.dist import ShardedSpMM
@@ -507,6 +532,8 @@ def run_b200(args):
         wall0 = time.perf_counter()
         step_ms = timed_steps(ctx, lambda: sh.run(vin, vout), args.steps, flush)
         wall = time.perf_counter() - wall0
+    if args.dump_outputs:
+        dump_outputs(ctx, sh, vout, args.dump_outputs)
     ms_per_step, ms_min = ctx.max_over_ranks([step_ms.mean(), step_ms.min()])
     per_rank_ms = ctx.gather_over_ranks(step_ms.mean())
     launches = op.launches_per_run * args.steps
@@ -587,7 +614,7 @@ def run_b200(args):
         ncu, ncu_src = ncu_record(args.workload) if world == 1 else (None, "captures are single-GPU")
         line = {
             "metric": "spmm_gflops", "value": round(flops / ms_per_step / 1e6, 2), "unit": "GFLOP/s",
-            "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": round(ms_per_step, 5),
+            "n_gpus": world, "steps": len(step_ms), "warmup": args.warmup, "ms_per_step": round(ms_per_step, 5),
             "ms_per_step_min": round(ms_min, 5), "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic",
             "config": workload_config(args.workload, ptr),
@@ -699,7 +726,12 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--sustain-seconds", type=float, default=2.0)
     ap.add_argument("--opt", action="append", default=[], help="engine option name=value (tuning runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="GPU arm only: write C of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computes; the reference arm times a sample of rows")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -27,6 +27,13 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_argument_errors():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "c0_k32", *extra], capture_output=True,
+                           text=True, timeout=120, cwd=ROOT)
+        assert r.returncode == 2 and "error:" in r.stderr, (extra, r.stderr[-2000:])
+
+
 def test_byte_accounting():
     sys.path.insert(0, ROOT)
     import bench

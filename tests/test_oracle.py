@@ -1,7 +1,7 @@
 """The CPU oracle (oracle/spmm_oracle.c) against hand-checkable cases, its own literal form,
 and the committed golden vectors. The reference ships no SpMM golden vector (SURVEY.md §8c);
-tests/test_gpu_parity.py pins this oracle bit-for-bit against the reference's own kernel
-rebuilt for sm_100a (oracle/_ref)."""
+tests/test_gpu_parity.py pins this oracle bit-for-bit against the reference kernel's stored
+outputs (tests/golden/make_reference_golden.py)."""
 import json
 import os
 
