@@ -89,6 +89,10 @@ class SpMMB200 : public SpMM {
         return new SpMMB200(t, feat < 0 ? this->feat_in : feat, stream_);
     }
 
+    // SDDMM over this operator's pattern: out[e] = <x_row[row(e)], x_col[idx[e]]> for every nonzero e (out: num_e
+    // floats in CSR position order). With x_row = dC and x_col = B, out is the gradient of C = A*B for the edge values.
+    void sddmm(const float *x_row, const float *x_col, float *out) { check(spmm_b200_sddmm(h_, x_row, x_col, out, stream_), "sddmm"); }
+
     // the same matrix with every row in ascending column order — for CSR inputs whose rows are not column-sorted (they
     // otherwise stay in one column block). Results associate in column order. Delete it before this operator.
     SpMMB200 *column_sorted(int feat = -1) const {

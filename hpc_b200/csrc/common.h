@@ -147,6 +147,9 @@ struct Plan {
     int2 *d_lpanel_all = nullptr, *d_panel_all = nullptr;
     float *d_part_all = nullptr;
     int *d_seg_count_all = nullptr;
+    // spmm_b200_sddmm (sddmm.cu), set up by its first call after preprocess
+    int *d_sddmm_vp = nullptr;      // [n_col_blocks * num_v + 1] band-major prefix of the (band, row) lengths (several blocks)
+    int sddmm_chunk = 0;            // nonzeros per warp (0: not set up yet)
 };
 
 }  // namespace spmm_b200

@@ -70,6 +70,7 @@ void free_plan(Plan &p) {
     release(p.d_pheavy_seg0);
     release(p.d_ctr);
     release(p.d_split);
+    release(p.d_sddmm_vp);
     if (hop) cudaSetDevice(cur);
     p = Plan();
 }

@@ -143,6 +143,16 @@ class SpMMB200(SpMM):
         self._check_io(vin, vout)
         check(lib.spmm_b200_run(self._h, _ptr(vin), _ptr(vout), _stream()))
 
+    def sddmm(self, x_row, x_col, out) -> None:
+        """SDDMM over this operator's pattern (spmm_b200_sddmm): out[e] = <x_row[row(e)], x_col[idx[e]]> for every
+        nonzero e, in CSR position order. x_row: num_v x feat_in, x_col: b_rows x feat_in, out: >= num_e floats.
+        With x_row = dC and x_col = B, out is dL/dval of C = A·B. Asynchronous on the current stream."""
+        for name, t, n in (("x_row", x_row, self.num_v * self.feat_in), ("x_col", x_col, self.b_rows * self.feat_in),
+                           ("out", out, self.num_e)):
+            if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < n:
+                raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {n} elements")
+        check(lib.spmm_b200_sddmm(self._h, _ptr(x_row), _ptr(x_col), _ptr(out), _stream()))
+
     def run_profiled(self, vin, vout) -> float:
         """run + the kernel's device time in ms (synchronises)."""
         self._check_io(vin, vout)

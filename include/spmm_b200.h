@@ -121,6 +121,20 @@ int spmm_b200_set_gather(spmm_b200_t h, int n_targets, float *const *targets, fl
  * destroy it before h. spmm_b200_refresh_values on it re-reads h's current values. Synchronises `stream`. */
 int spmm_b200_create_transposed(spmm_b200_t h, int feat_in, void *stream, spmm_b200_t *out);
 
+/* SDDMM over the operator's sparsity pattern (no reference counterpart; PA4 is forward only). For every nonzero e of
+ * row r (CSR position order, e in [0, num_e)):
+ *     out[e] = sum_j x_row[r * feat_in + j] * x_col[idx[e] * feat_in + j]
+ * in the fixed order documented in hpc_b200/csrc/sddmm.cu (results depend on feat_in only, not on any plan option).
+ * x_row: num_v x feat_in (e.g. dC), x_col: b_rows x feat_in (e.g. B), out: num_e floats, fully overwritten.
+ * With x_row = dC and x_col = B, out is dL/dval of C = A*B. Reads the caller's d_ptr / d_idx (not val), and no
+ * workspace that run uses. Works on any handle (row block, transposed, column-sorted); out follows THAT handle's CSR
+ * positions. x_row / x_col must be 16-byte aligned when feat_in % 4 == 0. num_e == 0: returns 0 without a CUDA call;
+ * feat_in == 0: out is set to +0.0f. Needs preprocess (SPMM_B200_ESTATE otherwise); set_feat, the b_rows option and a
+ * new preprocess invalidate it as they invalidate run. Asynchronous on `stream`. The first call after preprocess on a
+ * plan with several column blocks allocates its band prefix (from the library's pool, on `stream`): make that call
+ * before capturing sddmm into a CUDA graph. */
+int spmm_b200_sddmm(spmm_b200_t h, const float *x_row, const float *x_col, float *out, void *stream);
+
 /* The column-sorted operator (no reference counterpart): a new handle over the SAME matrix with every row stored in
  * ascending column order (stable: equal columns keep their storage order), built on the device. A CSR whose rows are
  * not column-sorted is otherwise kept in ONE column block — splitting an unsorted row at band boundaries would reorder
