@@ -81,9 +81,7 @@ int spmm_b200_set_option(spmm_b200_t h, const char *name, long long value) {
     else if (!strcmp(name, "tune") && value >= 0 && value <= 1) h->opt_tune = value;
     else if (!strcmp(name, "light_steps") && value >= 0 && value <= 65536) h->opt_light_steps = value;
     else if (!strcmp(name, "col_blocks") && value >= 0 && value <= 64) h->opt_col_blocks = value;
-    else if (!strcmp(name, "persistent") && value >= -1 && value <= 1) h->opt_persistent = value;
     else if (!strcmp(name, "row_groups") && value >= 0 && value <= kMaxRowGroups) h->opt_row_groups = value;
-    else if (!strcmp(name, "ticket_batch") && value >= 0 && value <= 16) h->opt_ticket_batch = value;
     else if (!strcmp(name, "split_streams") && value >= -1 && value <= 1) h->opt_split_streams = value;
     else if (!strcmp(name, "host_bands") && (value == 0 || value == 1 || (value >= 10 && value <= 90))) h->opt_host_bands = value;
     else if (!strcmp(name, "zero_copy") && value >= 0 && value <= 1) {
@@ -347,9 +345,9 @@ int spmm_b200_plan_info(spmm_b200_t h, spmm_b200_plan_info_t *info) {
     info->n_col_blocks = p.n_col_blocks;
     info->col_begin = b.col_begin;
     info->col_end = b.col_end;
-    info->persistent = p.persistent ? 1 : 0;
+    info->persistent = 0;
     info->n_row_groups = p.n_groups;
-    info->n_tickets = p.n_ptask;
+    info->n_tickets = 0;
     return 0;
 }
 
@@ -377,8 +375,6 @@ int spmm_b200_plan_copy(spmm_b200_t h, int which, void *host_dst, size_t bytes) 
             src = pl.d_split;
             want = pl.n_col_blocks > 1 ? sizeof(int) * (size_t)(pl.n_col_blocks + 1) * h->num_v : 0;
             break;
-        case 11: src = pl.d_ptask; want = sizeof(int4) * (size_t)pl.n_ptask; break;
-        case 13: src = pl.d_ctr; want = pl.d_ctr ? sizeof(unsigned int) * ctr_words(pl.n_groups) : 0; break;
         case 12: {
             want = pl.group_row.empty() ? 0 : sizeof(int) * pl.group_row.size();
             if (bytes != want) break;

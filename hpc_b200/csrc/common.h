@@ -33,7 +33,7 @@ struct SegDesc {
     int nnz_begin;
 };
 
-constexpr int kMaxBands = 16;    // column blocks one persistent launch can carry
+constexpr int kMaxBands = 16;    // cap of the automatic number of column blocks
 constexpr int kMaxRowGroups = 64;
 
 // What every pass of a run shares.
@@ -77,23 +77,6 @@ struct RunArgs {
     BandArgs b;
 };
 
-// One persistent launch for all column blocks: warps draw tickets; ticket order is band-major. `all` addresses the
-// bands' arrays as ONE set (each array is a single allocation, band after band), and the ticket list carries absolute
-// positions, so nothing in the task bodies is indexed by band.
-struct PersistArgs {
-    CommonArgs c;
-    BandArgs all;             // lpanel / panel / seg_desc / seg_hrow / heavy_seg0 / seg_count / part over all bands
-    const int4 *ptask;        // per ticket: {lpanel offset, or -1 - segment; steps; row group | accumulate << 16 | final << 17;
-                              //              completed tasks of that row group the task waits for}
-    int total;                // tickets
-    unsigned int *ctr;        // counters, one per 128-byte line (kCtrStride words apart): [0] ticket, [1] exited warps,
-                              // [2 + g] completed tasks of row group g — zero between runs — then the watchdog's line
-    int n_groups;
-    int batch;                // tickets a warp draws at once while the launch is far from its end (1 over its last stretch)
-};
-constexpr int kCtrStride = 32;   // words between counters: each on its own L2 line (same-line atomics serialise)
-inline size_t ctr_words(int n_groups) { return (size_t)(2 + n_groups + 1) * kCtrStride; }
-
 // The plan of one column block (the whole matrix when there is a single block).
 struct BlockPlan {
     int col_begin = 0, col_end = 0;   // B rows [col_begin, col_end) are gathered in this pass
@@ -116,7 +99,6 @@ struct BlockPlan {
     int *d_seg_count = nullptr;
     int2 *d_panel = nullptr;
     float *d_part = nullptr;
-    std::vector<int> task_group;   // host: row group of every utask entry (persistent launch)
     int split_task = 0;            // first task of the second half of the row groups (two-stream launches); 0 / n_utask: no split
 };
 
@@ -130,19 +112,9 @@ struct Plan {
     int *d_split = nullptr;   // [(n_col_blocks+1)][num_v] start of each column block inside each row
     std::vector<BlockPlan> blocks;
     int launches = 0;
-    // persistent single launch (all column blocks in one kernel)
-    bool persistent = false;
-    int n_groups = 1;               // row groups: band b+1's tasks of a group wait for band b's tasks of the same group
+    int n_groups = 1;               // row groups: contiguous row ranges planned independently, never spanned by a task
     std::vector<int> group_row;     // [n_groups + 1] first row of each group
-    unsigned int *d_ctr = nullptr;  // ticket, exited warps, per-group completion counters, watchdog (ctr_words)
-    int persist_grid = 0;           // CTAs of the persistent launch (all co-resident)
-    int ticket_batch = 1;           // tickets drawn at once far from the end of the launch
     bool split_streams = false;     // every pass as two launches (row-group halves) on two streams: each tail overlaps the next launch
-    int n_ptask = 0;
-    int4 *d_ptask = nullptr;        // the ticket list
-    SegDesc *d_pseg_desc = nullptr; // segments of all bands with absolute panel offsets
-    int *d_pseg_hrow = nullptr;     // segment -> absolute heavy-row index
-    int *d_pheavy_seg0 = nullptr;   // absolute heavy row -> absolute first segment (n_heavy + 1 entries per band)
     // arenas: one allocation per array kind, band after band (the per-band pointers above point into them)
     int2 *d_lpanel_all = nullptr, *d_panel_all = nullptr;
     float *d_part_all = nullptr;
@@ -160,7 +132,7 @@ struct spmm_b200_handle {
     const float *d_val = nullptr;
     int num_v = 0, num_e = 0, feat = 0;
     long long opt_seg_len = 0, opt_kslice = 0, opt_block = 128, opt_reorder = -1, opt_tune = 0, opt_col_blocks = 0, opt_light_steps = 0,
-              opt_zero_copy = 1, opt_persistent = -1, opt_row_groups = 0, opt_ticket_batch = 0, opt_split_streams = -1, opt_host_bands = 0;
+              opt_zero_copy = 1, opt_row_groups = 0, opt_split_streams = -1, opt_host_bands = 0;
     int plan_select = 0;   // which column block plan_info / plan_copy describe
     spmm_b200::Plan plan;
     float *d_stage_in = nullptr, *d_stage_out = nullptr;
@@ -211,7 +183,6 @@ int refresh_panels(spmm_b200_handle *h, cudaStream_t stream);
 int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t stream,
                 int *launches, const cudaEvent_t *band_ready = nullptr, float *cfinal = nullptr);
 int resident_warps(int lanes, int vec, int tune, int block);
-int persistent_grid(int lanes, int vec, int tune, int block);   // CTAs that are co-resident for the persistent kernel
 int launch_check_cols(const int *d_idx, long long nnz, int b_rows, int *d_bad, cudaStream_t stream);
 // band_begin[0..n_col_blocks]: first B row of every column block (band_begin[n] = b_rows), at most kMaxSplitBands blocks
 constexpr int kMaxSplitBands = 64;
@@ -240,9 +211,7 @@ int launch_xrank_barrier(unsigned int *const *flags, int world, int rank, int ph
 
 // Packs light rows (costs = deg + 1 entries each, in plan order) into stream tasks of `groups` interleaved lane-group
 // lanes with about `steps` entries each; dst[i] = lpanel slot of row i's header. Returns the lpanel length.
-// cut[0..n_cut): ascending row positions before which the open task is closed (row-group boundaries), or NULL.
-long long pack_light_host(const int *cost, int n, int groups, int steps, int *dst, std::vector<int2> &tasks,
-                          const int *cut = nullptr, int n_cut = 0);
+long long pack_light_host(const int *cost, int n, int groups, int steps, int *dst, std::vector<int2> &tasks);
 
 // lanes/vec choice for a slice width (shared by plan + launch)
 inline void shape_for_kslice(int kslice, int *lanes, int *vec) {

@@ -64,11 +64,6 @@ void free_plan(Plan &p) {
     release(p.d_panel_all);
     release(p.d_part_all);
     release(p.d_seg_count_all);
-    release(p.d_ptask);
-    release(p.d_pseg_desc);
-    release(p.d_pseg_hrow);
-    release(p.d_pheavy_seg0);
-    release(p.d_ctr);
     release(p.d_split);
     release(p.d_sddmm_vp);
     if (hop) cudaSetDevice(cur);
@@ -194,8 +189,7 @@ int plan_rows_host(const int *rb, const int *re, int M, int seg_len, int reorder
 // `steps` entries, the task is closed and the row opens the next one. A task's lanes are interleaved in the
 // panel — entry j of lane g sits at off + j*groups + g — and padded with nops to the longest lane rounded up to a
 // multiple of 4 steps (whole gather batches; it also keeps every task on a 16-byte boundary).
-long long pack_light_host(const int *cost, int n, int groups, int steps, int *dst, std::vector<int2> &tasks, const int *cut,
-                          int n_cut) {
+long long pack_light_host(const int *cost, int n, int groups, int steps, int *dst, std::vector<int2> &tasks) {
     tasks.clear();
     std::vector<int> fill((size_t)groups, 0);
     long long off = 0;
@@ -207,19 +201,7 @@ long long pack_light_host(const int *cost, int n, int groups, int steps, int *ds
         off += (long long)mx * groups;
         std::fill(fill.begin(), fill.end(), 0);
     };
-    int ci = 0;
     for (int i = 0; i < n; ++i) {
-        // a row-group boundary: no task spans it (the persistent launch orders column-block passes per row group)
-        bool boundary = false;
-        while (ci < n_cut && cut[ci] <= i) {
-            boundary |= cut[ci] == i;
-            ++ci;
-        }
-        if (boundary) {
-            bool any = false;
-            for (int x : fill) any |= x > 0;
-            if (any) close_task();
-        }
         int g = 0;
         for (int q = 1; q < groups; ++q)
             if (fill[q] < fill[g]) g = q;
@@ -260,12 +242,13 @@ int auto_light_steps(int groups, long long total_cost, long long slots, long lon
 
 // Everything the host works out for one column block before anything is allocated on the device.
 struct HostBlock {
-    std::vector<int> row_perm, heavy_rows, heavy_seg0, seg_hrow, task_group;
+    std::vector<int> row_perm, heavy_rows, heavy_seg0, seg_hrow;
     std::vector<SegDesc> segs;
     std::vector<int4> light;
     std::vector<int2> ltasks, utask;
     long long panel_len = 0, lpanel_len = 0;
     int reorder = 1, light_steps = 0;
+    int split_task = 0;   // first task of the second half of the row groups
     int rc = 0;
     char err[256] = "";
 };
@@ -282,9 +265,6 @@ static int block_reorder(const spmm_b200_handle *h, const int *rb, const int *re
     for (int r = 0; r < h->num_v; ++r) total += re[r] - rb[r] + 1;
     return (p.lanes == 32 && p.slots > 0 && total >= 8ll * p.slots * 64) ? 0 : 1;
 }
-
-static void plan_block_host(const spmm_b200_handle *h, const int *rb, const int *re, int skip_empty, int reorder, const int *group_row,
-                            int n_groups, HostBlock &hb);
 
 // The row groups (contiguous row ranges) are planned independently of each other — a task never spans a group bound, and
 // the row order (natural or degree buckets) applies INSIDE a group — so planning group by group and concatenating
@@ -388,7 +368,7 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
     hb.seg_hrow.resize((size_t)b_seg[n_groups]);
     hb.ltasks.resize((size_t)b_ltask[n_groups]);
     hb.utask.resize((size_t)b_utask[n_groups]);
-    hb.task_group.resize((size_t)b_utask[n_groups]);
+    hb.split_task = (int)b_utask[(n_groups + 1) / 2];   // the groups' tasks are contiguous, in group order
     if (b_heavy[n_groups]) hb.heavy_seg0[(size_t)b_heavy[n_groups]] = (int)b_seg[n_groups];
 #pragma omp parallel for schedule(dynamic, 1)
     for (int g = 0; g < n_groups; ++g) {
@@ -413,96 +393,32 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
         for (size_t i = 0; i < x.utask.size(); ++i) {
             const int2 u = x.utask[i];
             hb.utask[(size_t)b_utask[g] + i] = u.x < 0 ? make_int2(-1 - (sg + (-1 - u.x)), 0) : make_int2(lp + u.x, u.y);
-            hb.task_group[(size_t)b_utask[g] + i] = g;
         }
     }
 }
 
-// Host part of one block: row order, segments, light-stream packing, task order, row group of every task.
-// group_row: NULL, or the n_groups + 1 row-group boundaries (natural order only).
+// Host part of one block: row order, segments, light-stream packing, task order. group_row: the n_groups + 1
+// row-group boundaries. The scalar fallback (K % 4 != 0) keeps every row whole in one group and reads idx/val at run
+// time: its plan is the row order alone.
 static void plan_block_host(const spmm_b200_handle *h, const int *rb, const int *re, int skip_empty, int reorder,
                             const int *group_row, int n_groups, HostBlock &hb) {
     const Plan &p = h->plan;
-    const int M = h->num_v;
-    if (!p.scalar && group_row) {
+    if (!p.scalar) {
         plan_block_groups(h, rb, re, skip_empty, reorder, group_row, n_groups, hb);
         return;
     }
     hb.reorder = reorder;
-    const int pad = p.scalar ? 2 : 4 * (32 / p.lanes);
-    hb.rc = plan_rows_host(rb, re, M, p.seg_len, reorder, skip_empty, pad, hb.row_perm, hb.heavy_rows, hb.heavy_seg0, hb.segs,
+    hb.rc = plan_rows_host(rb, re, h->num_v, p.seg_len, reorder, skip_empty, 2, hb.row_perm, hb.heavy_rows, hb.heavy_seg0, hb.segs,
                            &hb.panel_len);
     if (hb.rc) {
         snprintf(hb.err, sizeof(hb.err), "%s", spmm_b200_last_error());
         return;
     }
-    const int n_light = (int)hb.row_perm.size();
-    std::vector<int> cost((size_t)n_light), dst((size_t)n_light);
-    const int groups = p.scalar ? 1 : 32 / p.lanes;
-    for (int i = 0; i < n_light; ++i) cost[i] = re[hb.row_perm[i]] - rb[hb.row_perm[i]] + 1;
-    // positions in row_perm where a new row group starts (row_perm ascends in natural order)
-    std::vector<int> cut;
-    if (group_row && n_groups > 1)
-        for (int g = 1; g < n_groups; ++g)
-            cut.push_back((int)(std::lower_bound(hb.row_perm.begin(), hb.row_perm.end(), group_row[g]) - hb.row_perm.begin()));
-    if (!p.scalar) {
-        int steps = p.light_steps;
-        if (h->opt_light_steps <= 0) {
-            long long total = 0;
-            for (int c : cost) total += c;
-            steps = auto_light_steps(groups, total, p.slots, (long long)hb.segs.size() * p.n_slices);
-        }
-        hb.light_steps = steps;
-        hb.lpanel_len = pack_light_host(cost.data(), n_light, groups, steps, dst.data(), hb.ltasks, cut.data(), (int)cut.size());
-        if (hb.lpanel_len > 0x7fffffffll) {
-            hb.rc = SPMM_B200_EINVAL;
-            snprintf(hb.err, sizeof(hb.err), "light panel too large");
-            return;
-        }
-    }
-    hb.light.resize((size_t)n_light);
-    for (int i = 0; i < n_light; ++i) {
+    hb.light.resize(hb.row_perm.size());
+    for (size_t i = 0; i < hb.row_perm.size(); ++i) {
         const int r = hb.row_perm[i];
-        hb.light[i] = make_int4(r, rb[r], re[r] - rb[r], p.scalar ? 0 : dst[i]);
+        hb.light[i] = make_int4(r, rb[r], re[r] - rb[r], 0);
     }
-
-    // Scheduling order of the warp tasks. Bucketed rows: heavy segments (the longest rows) first, then the light
-    // tasks. Natural order: light tasks and heavy segments merged by the row they start with, so that a heavy row
-    // runs next to its neighbours (whose B rows it shares in L2) instead of ahead of everything.
-    auto group_of = [&](int row) {
-        if (!group_row || n_groups <= 1) return 0;
-        return (int)(std::upper_bound(group_row, group_row + n_groups + 1, row) - group_row) - 1;
-    };
-    hb.utask.reserve(hb.ltasks.size() + hb.segs.size());
-    hb.task_group.reserve(hb.ltasks.size() + hb.segs.size());
-    if (reorder == 0 && !p.scalar) {
-        size_t li = 0, first_i = 0;   // first_i: index in row_perm of the first row of light task li
-        size_t si = 0;
-        auto light_first_row = [&](size_t t) {
-            while (first_i < (size_t)n_light && dst[first_i] < hb.ltasks[t].x) ++first_i;
-            return first_i < (size_t)n_light ? hb.row_perm[first_i] : 0x7fffffff;
-        };
-        while (li < hb.ltasks.size() || si < hb.segs.size()) {
-            const int lrow = li < hb.ltasks.size() ? light_first_row(li) : 0x7fffffff;
-            const int hrow = si < hb.segs.size() ? hb.segs[si].row : 0x7fffffff;
-            if (si < hb.segs.size() && hrow < lrow) {
-                hb.utask.push_back(make_int2(-1 - (int)si, 0));
-                hb.task_group.push_back(group_of(hrow));
-                ++si;
-            } else {
-                hb.utask.push_back(hb.ltasks[li]);
-                hb.task_group.push_back(group_of(lrow));
-                ++li;
-            }
-        }
-    } else {
-        for (size_t si = 0; si < hb.segs.size(); ++si) hb.utask.push_back(make_int2(-1 - (int)si, 0));
-        for (const int2 &t : hb.ltasks) hb.utask.push_back(t);
-        hb.task_group.assign(hb.utask.size(), 0);
-    }
-    hb.seg_hrow.resize(hb.segs.size());
-    for (int hr = 0; hr < (int)hb.heavy_rows.size(); ++hr)
-        for (int sgm = hb.heavy_seg0[hr]; sgm < hb.heavy_seg0[hr + 1]; ++sgm) hb.seg_hrow[sgm] = hr;
 }
 
 template <class T>
@@ -646,12 +562,9 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
         reorder[b] = h->opt_reorder >= 0 ? (int)h->opt_reorder : (nb > 1 ? 1 : block_reorder(h, row_begin(b), row_end(b)));
         all_natural &= reorder[b] == 0;
     }
-    // One persistent launch for all column blocks (option "persistent": 1 = on, needs a single feature slice; default off:
-    // built and parity-tested, but on the shapes measured the two-stream launches below do better — profiles/r02_notes.md).
-    p.persistent = !p.scalar && p.n_slices == 1 && nb <= kMaxBands && h->opt_persistent == 1;
     // Row groups: contiguous row ranges balanced by nonzeros (the partition rule), planned independently (in parallel) and
     // never spanned by a task. Natural order: 16. Degree buckets with several blocks: 2 — the halves that go out on two
-    // streams (below) and that order the passes inside a persistent launch. Otherwise 1.
+    // streams (below). Otherwise 1.
     {
         long long g = h->opt_row_groups > 0 ? h->opt_row_groups : (all_natural ? 16 : (nb > 1 ? 2 : 1));
         if (p.scalar) g = 1;
@@ -704,9 +617,8 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
     if (pn_total) SB_CUDA(pool_alloc((void **)&p.d_panel_all, sizeof(int2) * (size_t)pn_total, stream));
     if (seg_total) SB_CUDA(pool_alloc((void **)&p.d_part_all, sizeof(float) * (size_t)seg_total * K, stream));
     if (heavy_total) {
-        // n_heavy + 1 slots per band, so that a band's counters sit at its absolute heavy-row base (the persistent
-        // launch addresses them that way, like heavy_seg0)
-        const size_t slots = (size_t)(heavy_total + nb) * p.n_slices;
+        // n_heavy x n_slices counters per band
+        const size_t slots = (size_t)heavy_total * p.n_slices;
         SB_CUDA(pool_alloc((void **)&p.d_seg_count_all, sizeof(int) * slots, stream));
         SB_CUDA(cudaMemsetAsync(p.d_seg_count_all, 0, sizeof(int) * slots, stream));
     }
@@ -729,9 +641,7 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
         bp.lpanel_len = x.lpanel_len;
         bp.n_ltask = (int)x.ltasks.size();
         bp.n_utask = (int)x.utask.size();
-        bp.task_group = x.task_group;
-        // first task of the second half of the row groups (tasks are in row order, so the groups are contiguous)
-        bp.split_task = (int)(std::lower_bound(x.task_group.begin(), x.task_group.end(), (p.n_groups + 1) / 2) - x.task_group.begin());
+        bp.split_task = x.split_task;
         if ((rc = upload_vec(&bp.d_row_perm, x.row_perm, stream))) return rc;
         if ((rc = upload_vec(&bp.d_light_desc, x.light, stream))) return rc;
         if ((rc = upload_vec(&bp.d_utask, x.utask, stream))) return rc;
@@ -745,7 +655,7 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
             if ((rc = upload_vec(&bp.d_heavy_rows, x.heavy_rows, stream))) return rc;
             if ((rc = upload_vec(&bp.d_heavy_seg0, x.heavy_seg0, stream))) return rc;
             if ((rc = upload_vec(&bp.d_seg_desc, x.segs, stream))) return rc;
-            bp.d_seg_count = p.d_seg_count_all + (heavy_off + b) * p.n_slices;
+            bp.d_seg_count = p.d_seg_count_all + heavy_off * p.n_slices;
             bp.d_panel = p.d_panel_all + pn_off;
             bp.d_part = p.d_part_all + seg_off * K;
             if ((rc = launch_build_panel(bp.d_seg_desc, bp.n_seg, K / 4, pad, h->d_idx, h->d_val, bp.d_panel, stream))) return rc;
@@ -757,71 +667,16 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
     }
     tr.lap("uploads + panel kernels queued");
 
-    // Two-stream launches (option "split_streams": -1 auto = whenever there are several blocks and no persistent launch).
-    p.split_streams = !p.scalar && p.n_groups > 1 &&
-                      (h->opt_split_streams == 1 || (h->opt_split_streams < 0 && nb > 1 && !p.persistent));
+    // Two-stream launches (option "split_streams": -1 auto = whenever there are several blocks).
+    p.split_streams = !p.scalar && p.n_groups > 1 && (h->opt_split_streams == 1 || (h->opt_split_streams < 0 && nb > 1));
     if (p.split_streams && !h->aux_stream) {   // created here, not in run: run may be under CUDA-graph capture
         SB_CUDA(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
         SB_CUDA(cudaEventCreateWithFlags(&h->aux_fork, cudaEventDisableTiming));
         SB_CUDA(cudaEventCreateWithFlags(&h->aux_join, cudaEventDisableTiming));
     }
 
-    // ---- the persistent launch's ticket list: band-major, absolute positions, row group and dependency per task ---------
-    std::vector<int4> ptask;
-    std::vector<SegDesc> pseg;
-    std::vector<int> pseg_hrow, pheavy_seg0;
-    if (p.persistent) {
-        ptask.reserve((size_t)task_total);
-        pseg.reserve((size_t)seg_total);
-        pseg_hrow.reserve((size_t)seg_total);
-        pheavy_seg0.reserve((size_t)(heavy_total + nb));
-        std::vector<int> done((size_t)p.n_groups, 0);   // tasks of each group in the bands before the current one
-        long long lp0 = 0, pn0 = 0, seg0 = 0;
-        int hrow0 = 0;   // absolute heavy-row index base: every band contributes n_heavy + 1 entries of heavy_seg0
-        for (int b = 0; b < nb; ++b) {
-            HostBlock &x = hb[b];
-            const int flags = (b > 0 ? 1 << 16 : 0) | (b + 1 == nb ? 1 << 17 : 0);
-            std::vector<int> here((size_t)p.n_groups, 0);
-            for (size_t t = 0; t < x.utask.size(); ++t) {
-                const int2 u = x.utask[t];
-                const int g = x.task_group[t];
-                ++here[g];
-                ptask.push_back(u.x < 0 ? make_int4(-1 - (int)(seg0 + (-1 - u.x)), 0, g | flags, b > 0 ? done[g] : 0)
-                                        : make_int4((int)(lp0 + u.x), u.y, g | flags, b > 0 ? done[g] : 0));
-            }
-            for (int g = 0; g < p.n_groups; ++g) done[g] += here[g];
-            for (size_t sgm = 0; sgm < x.segs.size(); ++sgm) {
-                SegDesc d = x.segs[sgm];
-                d.panel_off += (int)pn0;
-                pseg.push_back(d);
-                pseg_hrow.push_back(hrow0 + x.seg_hrow[sgm]);
-            }
-            for (int v : x.heavy_seg0) pheavy_seg0.push_back((int)seg0 + v);
-            if (x.heavy_seg0.empty()) pheavy_seg0.push_back((int)seg0);   // keep n_heavy + 1 entries per band
-            hrow0 += (int)x.heavy_rows.size() + 1;
-            lp0 += x.lpanel_len;
-            pn0 += x.panel_len;
-            seg0 += (long long)x.segs.size();
-        }
-        p.n_ptask = (int)ptask.size();
-        if ((rc = upload_vec(&p.d_ptask, ptask, stream))) return rc;
-        if ((rc = upload_vec(&p.d_pseg_desc, pseg, stream))) return rc;
-        if ((rc = upload_vec(&p.d_pseg_hrow, pseg_hrow, stream))) return rc;
-        if ((rc = upload_vec(&p.d_pheavy_seg0, pheavy_seg0, stream))) return rc;
-        // ticket, exited warps, per-group completions, watchdog: one 128-byte line each
-        SB_CUDA(pool_alloc((void **)&p.d_ctr, sizeof(unsigned int) * ctr_words(p.n_groups), stream));
-        SB_CUDA(cudaMemsetAsync(p.d_ctr, 0, sizeof(unsigned int) * ctr_words(p.n_groups), stream));
-        p.persist_grid = persistent_grid(p.lanes, p.vec, p.tune, p.block);
-        // Tickets per draw. A batch delays the completion of its last task by the tasks before it, and the next band's
-        // tasks of the same row group wait for that: only bands much longer than the batches of all resident warps
-        // (32 waves) draw four at a time; the ticket counter's L2 line takes one atomic per draw either way.
-        long long shortest = task_total;
-        for (int b = 0; b < nb; ++b) shortest = std::min<long long>(shortest, (long long)hb[b].utask.size());
-        p.ticket_batch = h->opt_ticket_batch > 0 ? (int)h->opt_ticket_batch : (p.slots > 0 && shortest >= 32 * p.slots ? 4 : 1);
-        if (p.persist_grid <= 0) p.persistent = false;   // occupancy could not be queried: one launch per block
-    }
     SB_CUDA(cudaStreamSynchronize(stream));   // host vectors go out of scope
-    tr.lap("ticket list + final sync");
+    tr.lap("final sync");
     p.ready = true;
     return 0;
 }

@@ -4,7 +4,8 @@
 // K and over the row) and the student's SpmmOptKernel (PA4/workspace/src/spmm_opt.cu:9-35:
 // one CTA per <=256-nnz task, atomicAdd into a pre-zeroed vout).
 //
-//   spmm_kernel        one launch per column block. Warp tasks: heavy segments first, then light-row stream tasks.
+//   spmm_kernel        one launch per column block (two, one per row half, with two-stream launches), one warp task per
+//                      warp: heavy segments and light-row stream tasks in the order the plan schedules them.
 //     light stream     rows kept whole are packed (header + {col,val} entries) into a stream panel cut into
 //                      equal-sized warp tasks; LANES lanes cooperate on one row, each owning VEC float4 of the
 //                      feature slice, so a warp walks 32/LANES interleaved lanes of rows at once. The task's
@@ -30,7 +31,6 @@ namespace {
 constexpr unsigned kFull = 0xffffffffu;
 constexpr int kChunk = 128;   // panel entries per TMA stage (1 KB)
 constexpr int kStages = 2;
-constexpr int kWarpSlots = 8;   // words of per-warp bookkeeping in shared memory (persistent kernel)
 
 // ---- memory helpers ------------------------------------------------------------------------
 
@@ -87,23 +87,8 @@ __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
                  "r"(bytes)
                  : "memory");
 }
-// Watchdog of the persistent launch (wd = the last line of a.ctr, NULL elsewhere): a wait that lasts longer than
-// ~2 s of SM clocks records what it was waiting for — {kind, a, b, c, d} — once, and gives up, so a scheduling bug
-// shows up as a wrong result with a diagnosis instead of a hung GPU. kind 1: staged chunk (TMA), 2: row-group dependency.
-constexpr long long kWatchdogClocks = 4000000000ll;
-__device__ __noinline__ void watchdog_trip(unsigned int *wd, unsigned int kind, unsigned int a, unsigned int b, unsigned int c,
-                                           unsigned int d) {
-    if (atomicCAS(wd, 0u, kind) == 0u) {
-        wd[1] = a;
-        wd[2] = b;
-        wd[3] = c;
-        wd[4] = d;
-        __threadfence();
-    }
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, unsigned int *wd = nullptr, unsigned int info = 0) {
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
     uint32_t done;
-    long long t0 = 0;
     do {
         asm volatile(
             "{\n\t.reg .pred p;\n\t"
@@ -112,13 +97,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, unsign
             : "=r"(done)
             : "r"(smem_u32(bar)), "r"(parity)
             : "memory");
-        if (!done && wd) {
-            if (t0 == 0) t0 = clock64();
-            else if (clock64() - t0 > kWatchdogClocks) {
-                watchdog_trip(wd, 1u, info, parity, blockIdx.x, threadIdx.x);
-                break;
-            }
-        }
     } while (!done);
 }
 // 1-D TMA: global -> shared, completion counted in bytes on the mbarrier.
@@ -134,16 +112,9 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst, const void *src, uint32_
 // ---- the SpMM kernel ------------------------------------------------------------------------
 //
 // Warp tasks (equal-sized, TMA-staged spans of a {col,val} panel) are either light-stream tasks or heavy segments, in
-// the order the plan wants them scheduled. Two outer kernels share the task bodies:
-//   spmm_kernel            one launch per column block, one task per warp, scheduled by the hardware (single-block
-//                          plans, and the host-buffer calls, whose passes wait for uploads between launches)
-//   spmm_persistent_kernel ONE launch for all column blocks: a grid of co-resident warps draws tickets from a global
-//                          counter; ticket order is band-major, so the tail of band b overlaps the head of band b+1.
-//                          A task of band b+1 continues chains that band b left in C, so it waits until the tasks of
-//                          band b that own the same ROW GROUP have completed (per-group completion counters; a task
-//                          publishes its completion after its stores are fenced). Waiting is rare — a group's previous
-//                          band ran a whole band earlier — and cannot deadlock: a task only ever waits for smaller
-//                          tickets, which are complete or held by running warps.
+// the order the plan wants them scheduled. spmm_kernel runs one task per warp, scheduled by the hardware; a launch
+// covers one column block (or one row half of it, with two-stream launches), and a later block's pass continues the
+// chains the earlier one left in C because the launches over the same rows are ordered on one stream.
 //
 // TUNE selects the gathers kept in flight per lane group and the register cap (option "tune";
 // measurements in profiles/r01_sweep.md):
@@ -160,14 +131,12 @@ struct Tune {
     static constexpr int kUnroll = TUNE == 1 ? 2 : 4;   // gathers in flight per lane group
 };
 
-// A warp's staging pipeline: kStages chunks of shared memory, one mbarrier each, initialised once per warp. A task
-// waits for chunk k on stage k % kStages with phase parity (k / kStages) & 1 — which assumes both barriers start the
-// task in an even phase. pipe_finish restores that at the end of a task (one plain arrival completes an idle
-// barrier's phase), so the persistent kernel carries nothing from task to task and never re-initialises a barrier.
+// A warp's staging pipeline: kStages chunks of shared memory, one mbarrier each, initialised by the warp before its
+// task. The task waits for chunk k on stage k % kStages with phase parity (k / kStages) & 1: the barriers start in
+// phase 0, and a warp runs exactly one task, so they are never reused.
 struct Pipe {
     int2 *buf;
     uint64_t *bars;
-    unsigned int *wd;   // watchdog words (persistent launch) or NULL
 };
 __device__ __forceinline__ void pipe_init(const Pipe &p, int lane) {
     if (lane == 0) {
@@ -177,7 +146,10 @@ __device__ __forceinline__ void pipe_init(const Pipe &p, int lane) {
     }
     __syncwarp();
 }
-// after the last chunk of a task has been consumed by every lane (the chunk loops end with __syncwarp)
+// After the last chunk of a task has been consumed by every lane (the chunk loops end with __syncwarp): one plain
+// arrival completes each idle barrier's current phase, so both end the task in an even phase. A warp runs one task, so
+// nothing depends on that; the arrivals stay because the code the compiler generates with them is faster: without them
+// reddit K=32 took 0.8246 instead of 0.8195 ms per run (B200, 1000 W), and spmm_kernel<32, 2, 0, false> spills 24 bytes.
 __device__ __forceinline__ void pipe_finish(const Pipe &p, int nchunks, int lane) {
     static_assert(kStages == 2, "phase bookkeeping below is written for two stages");
     if (lane == 0) {
@@ -192,26 +164,19 @@ __device__ __forceinline__ void pipe_issue(const Pipe &p, int k, const int2 *src
 }
 __device__ __forceinline__ const int2 *pipe_wait(const Pipe &p, int k) {
     const int s = k % kStages;
-    mbar_wait(&p.bars[s], (uint32_t)(k / kStages) & 1u, p.wd, (unsigned int)k);
+    mbar_wait(&p.bars[s], (uint32_t)(k / kStages) & 1u);
     return p.buf + s * kChunk;
 }
-
-struct NoHook {
-    __device__ __forceinline__ void start() const {}
-    __device__ __forceinline__ void mid() const {}
-    __device__ __forceinline__ void late() const {}
-};
 
 // Light rows as a stream: a warp walks one task of the light panel, staged through shared
 // memory by 1-D TMA exactly like a heavy segment. Lane group g reads entries g, g+GROUPS, ... of the task:
 // a header starts a new row (the previous row's accumulator is stored first), a nonzero is one B-row gather
 // and one in-order FMA, a nop is padding. Rows never span lane groups, so every row is still one FMA chain in
 // CSR order (bit-exact), but gathers stay in flight across row boundaries and no load depends on a
-// per-row descriptor. `hook.start()` runs once the first chunks are on their way (the persistent kernel publishes the
-// previous task and checks this task's dependency there).
-template <int LANES, int VEC, int TUNE, bool FULL, class Hook>
+// per-row descriptor.
+template <int LANES, int VEC, int TUNE, bool FULL>
 __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs &bd, bool accumulate, bool final, int slice, int2 td,
-                                             int lane, const Pipe &pipe, Hook &&hook) {
+                                             int lane, const Pipe &pipe) {
     constexpr int GROUPS = 32 / LANES;
     constexpr int U = Tune<TUNE, VEC>::kUnroll;
     const int l = lane % LANES;
@@ -224,7 +189,6 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
         pipe_issue(pipe, 0, src, (uint32_t)min(kChunk, len));   // len is a multiple of 4 * GROUPS
         if (nchunks > 1) pipe_issue(pipe, 1, src + kChunk, (uint32_t)min(kChunk, len - kChunk));
     }
-    hook.start();
 
     const int K = c.feat;
     const int col0 = slice * c.kslice + l * 4;
@@ -303,16 +267,14 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
         __syncwarp();   // every lane is done reading this stage before it is refilled
         if (lane == 0 && k + kStages < nchunks)
             pipe_issue(pipe, k + kStages, src + (size_t)(k + kStages) * kChunk, (uint32_t)min(kChunk, len - (k + kStages) * kChunk));
-        if (k == 0) hook.mid();
     }
     pipe_finish(pipe, nchunks, lane);
-    hook.late();
     flush_row();
 }
 
-template <int LANES, int VEC, int TUNE, bool FULL, class Hook>
+template <int LANES, int VEC, int TUNE, bool FULL>
 __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArgs &bd, bool accumulate, bool final, int slice, int seg,
-                                              int lane, const Pipe &pipe, Hook &&hook) {
+                                              int lane, const Pipe &pipe) {
     constexpr int GROUPS = 32 / LANES;
     constexpr int U = Tune<TUNE, VEC>::kUnroll;
     const int l = lane % LANES;
@@ -326,7 +288,6 @@ __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArg
         pipe_issue(pipe, 0, src, (uint32_t)min(kChunk, plen));
         if (nchunks > 1) pipe_issue(pipe, 1, src + kChunk, (uint32_t)min(kChunk, plen - kChunk));
     }
-    hook.start();
 
     const int K = c.feat;
     const int col0 = slice * c.kslice + l * 4;
@@ -370,11 +331,9 @@ __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArg
         __syncwarp();   // every lane is done reading this stage before it is refilled
         if (lane == 0 && k + kStages < nchunks)
             pipe_issue(pipe, k + kStages, src + (size_t)(k + kStages) * kChunk, (uint32_t)min(kChunk, plen - (k + kStages) * kChunk));
-        if (k == 0) hook.mid();
     }
-    pipe_finish(pipe, nchunks, lane);
-    hook.late();
 
+    pipe_finish(pipe, nchunks, lane);
     // combine the lane groups (fixed tree => deterministic)
 #pragma unroll
     for (int off = LANES; off < 32; off <<= 1) {
@@ -438,156 +397,10 @@ __global__ void __launch_bounds__(256, Tune<TUNE, VEC>::kMinBlocks) spmm_kernel(
     if (slice >= a.c.n_slices) return;
     const int2 td = __ldg(a.b.utask + (gw - (long long)slice * a.b.n_utask));
     const Pipe pipe = {reinterpret_cast<int2 *>(smem_raw) + (size_t)warp * kStages * kChunk,
-                       reinterpret_cast<uint64_t *>(smem_raw + (size_t)nwarps * kStages * kChunk * sizeof(int2)) + warp * kStages, nullptr};
+                       reinterpret_cast<uint64_t *>(smem_raw + (size_t)nwarps * kStages * kChunk * sizeof(int2)) + warp * kStages};
     pipe_init(pipe, lane);
-    if (td.x < 0) heavy_segment<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, -1 - td.x, lane, pipe, NoHook());
-    else light_stream<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, td, lane, pipe, NoHook());
-}
-
-__device__ __forceinline__ void red_release_gpu(unsigned int *p) {
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(p) : "memory");
-}
-// The poll of a row group's counter. Not ld.acquire: that compiles to LDG.STRONG.GPU + CCTL.IVALL — an invalidation of
-// the SM's whole L1 per poll. The rows read after a successful poll are read with ld.cg (L2, never L1), so a relaxed
-// poll followed by fence.acq_rel.gpu (MEMBAR.ALL.GPU, no invalidation) gives the ordering that is needed.
-__device__ __forceinline__ unsigned int ld_relaxed_gpu(const unsigned int *p) {
-    unsigned int v;
-    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void fence_acq_rel_gpu() { asm volatile("fence.acq_rel.gpu;" ::: "memory"); }
-#ifdef SPMM_B200_PERSIST_STATS
-#define PSTAT(i, v) atomicAdd(reinterpret_cast<unsigned long long *>(wd + 8) + (i), (unsigned long long)(v))
-#else
-#define PSTAT(i, v) ((void)0)
-#endif
-
-// The persistent warp's bookkeeping around a task.
-//   start()  once the task's first chunks are on their way: settle the next ticket (parked in shared memory while the
-//            task runs) and check the dependency — the tasks of earlier bands that own the same row group must have
-//            completed. Tickets are drawn four at a time while the launch is far from its end and one at a time over
-//            its last stretch (the tail stays fine-grained); the dependency is polled only when the cached count of
-//            that row group does not already cover it (consecutive tasks of a warp mostly share band and group). Both
-//            keep the traffic on the counters' L2 lines — where same-line atomics serialise — far below their limit.
-//   mid()    after the task's first chunk: publish the completion of the PREVIOUS task (one release-add to its row
-//            group's counter). By then the previous task's stores were acknowledged, so the release does not stall;
-//            issued at the start of the task it would wait for the row the warp has just flushed, and issued at the
-//            end of the task it would delay the tasks that wait for it by a whole (possibly long) task.
-//   late()   right before the task's final stores: note this task as finished-but-unpublished.
-// A warp that has to block in start() publishes first: the tasks it waits for can include its own previous one.
-// Lane 0 does the counting; the warp barriers at the end of every chunk and of every task order all lanes' stores
-// before lane 0's release and extend its acquire to them (the pattern of a grid barrier).
-struct PersistHook {
-    unsigned int *ticket;
-    unsigned int *grp_done;        // counter of row group g at grp_done[g * kCtrStride]
-    volatile unsigned int *slot;   // per warp: [0] next ticket, [1] end of the drawn batch, [2] row group of the finished,
-                                   // unpublished task + 1 (0: none), [3] row group whose count is cached + 1, [4] that count
-    unsigned int t;                // this task's ticket
-    int total;
-    int batch;
-    int flags;                     // this task: row group | accumulate << 16 | final << 17
-    int need;                      // completed tasks of that group this task waits for (0: none)
-    int lane;
-    unsigned int *wd;
-    __device__ __forceinline__ void start() const {
-        if (lane == 0) {
-            unsigned int next = t + 1, fresh = 0;
-            const bool draw = next >= slot[1];
-            if (draw) {
-                // far from the end (more than 16 tasks per warp left): four tickets at once
-                fresh = (unsigned int)total > t && (unsigned int)total - t > 16u * gridDim.x * (blockDim.x >> 5) ? (unsigned int)batch : 1u;
-                next = atomicAdd(ticket, fresh);
-            }
-            const unsigned int grp = (unsigned int)(flags & 0xffff);
-            if (need > 0 && !(slot[3] == grp + 1 && (int)slot[4] >= need)) {
-                const unsigned int *cnt = grp_done + grp * kCtrStride;
-                unsigned int seen = ld_relaxed_gpu(cnt);
-                PSTAT(0, 1);
-                if ((int)seen < need) {
-                    const unsigned int p = slot[2];
-                    if (p) {
-                        red_release_gpu(grp_done + (p - 1) * kCtrStride);
-                        slot[2] = 0;
-                    }
-                    const long long t0 = clock64();
-                    while ((int)(seen = ld_relaxed_gpu(cnt)) < need) {
-                        __nanosleep(32);
-                        if (clock64() - t0 > kWatchdogClocks) {
-                            watchdog_trip(wd, 2u, grp, (unsigned int)need, seen, blockIdx.x * blockDim.x + threadIdx.x);
-                            break;
-                        }
-                    }
-                    PSTAT(1, 1);
-                    PSTAT(2, clock64() - t0);
-                }
-                fence_acq_rel_gpu();
-                slot[3] = grp + 1;
-                slot[4] = seen;
-            }
-            slot[0] = next;
-            if (draw) slot[1] = next + fresh;
-        }
-        __syncwarp();   // extends lane 0's acquire to the lanes that read C rows of the earlier band
-    }
-    __device__ __forceinline__ void mid() const {
-        if (lane == 0) {
-            const unsigned int p = slot[2];
-            if (p) {
-                red_release_gpu(grp_done + (p - 1) * kCtrStride);
-                slot[2] = 0;
-            }
-        }
-    }
-    __device__ __forceinline__ void late() const {
-        // this task counts as finished once its final stores are issued (published during the next task)
-        if (lane == 0) slot[2] = ((flags >> 17) & 1) ? 0u : (unsigned int)(flags & 0xffff) + 1u;   // nobody waits for the last band
-    }
-};
-
-template <int LANES, int VEC, int TUNE, bool FULL>
-__global__ void __launch_bounds__(256, Tune<TUNE, VEC>::kMinBlocks) spmm_persistent_kernel(const __grid_constant__ PersistArgs a) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const int nwarps = blockDim.x >> 5;
-    unsigned int *const ticket = a.ctr, *const exited = a.ctr + kCtrStride, *const grp_done = a.ctr + 2 * kCtrStride;
-    const Pipe pipe = {reinterpret_cast<int2 *>(smem_raw) + (size_t)warp * kStages * kChunk,
-                       reinterpret_cast<uint64_t *>(smem_raw + (size_t)nwarps * kStages * kChunk * sizeof(int2)) + warp * kStages,
-                       a.ctr + (2 + a.n_groups) * kCtrStride};
-    // a few words of shared memory per warp (after the barriers): see PersistHook::slot
-    volatile unsigned int *slot =
-        reinterpret_cast<unsigned int *>(smem_raw + (size_t)nwarps * kStages * (kChunk * sizeof(int2) + sizeof(uint64_t))) + kWarpSlots * warp;
-    pipe_init(pipe, lane);
-    unsigned int t = 0;
-    if (lane == 0) {
-        t = atomicAdd(ticket, 1u);
-        slot[1] = t + 1;
-        slot[2] = 0;
-        slot[3] = 0;
-    }
-    t = __shfl_sync(kFull, t, 0);
-    while (t < (unsigned int)a.total) {
-        // {lpanel offset | -1 - segment, steps, row group | accumulate << 16 | final << 17, completions to wait for}
-        const int4 pt = __ldg(a.ptask + t);
-        const bool accumulate = (pt.z >> 16) & 1, final = (pt.z >> 17) & 1;
-        const PersistHook hook = {ticket, grp_done, slot, t, a.total, a.batch, pt.z, pt.w, lane, pipe.wd};
-        if (pt.x < 0) heavy_segment<LANES, VEC, TUNE, FULL>(a.c, a.all, accumulate, final, 0, -1 - pt.x, lane, pipe, hook);
-        else light_stream<LANES, VEC, TUNE, FULL>(a.c, a.all, accumulate, final, 0, make_int2(pt.x, pt.y), lane, pipe, hook);
-        __syncwarp();   // every lane's stores of this task precede whatever lane 0 releases next
-        t = slot[0];
-    }
-    // the last task's completion
-    if (lane == 0 && slot[2]) red_release_gpu(grp_done + (slot[2] - 1) * kCtrStride);
-    // the last warp out returns the counters to zero for the next run (nobody is left to read them)
-    if (lane == 0) {
-        const unsigned int total_warps = gridDim.x * nwarps;
-        if (atomicAdd(exited, 1u) == total_warps - 1) {
-            for (int g = 0; g < a.n_groups; ++g) grp_done[g * kCtrStride] = 0;
-            *ticket = 0;
-            *exited = 0;
-            __threadfence();
-        }
-    }
+    if (td.x < 0) heavy_segment<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, -1 - td.x, lane, pipe);
+    else light_stream<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, td, lane, pipe);
 }
 
 // K % 4 != 0: scalar lanes over the feature columns, one warp per row, same in-order chain.
@@ -729,8 +542,8 @@ __global__ void __launch_bounds__(256) valid_kernel(const float *y, const float 
     if ((threadIdx.x & 31) == 0 && local) atomicAdd(count, (unsigned long long)local);
 }
 
-// per warp: kStages chunks + their mbarriers, and kWarpSlots words of bookkeeping for the persistent kernel
-size_t task_smem(int block) { return (size_t)(block / 32) * (kStages * (kChunk * sizeof(int2) + sizeof(uint64_t)) + kWarpSlots * sizeof(unsigned int)); }
+// per warp: kStages chunks + their mbarriers
+size_t task_smem(int block) { return (size_t)(block / 32) * kStages * (kChunk * sizeof(int2) + sizeof(uint64_t)); }
 
 template <int LANES, int VEC, int TUNE, bool FULL>
 void launch_tuned(const RunArgs &a, int block, cudaStream_t stream) {
@@ -738,33 +551,27 @@ void launch_tuned(const RunArgs &a, int block, cudaStream_t stream) {
     const long long tasks = (long long)a.b.n_utask * a.c.n_slices;
     spmm_kernel<LANES, VEC, TUNE, FULL><<<(unsigned)((tasks + warps - 1) / warps), block, task_smem(block), stream>>>(a);
 }
-template <int LANES, int VEC, int TUNE, bool FULL>
-void launch_tuned(const PersistArgs &a, int block, int grid, cudaStream_t stream) {
-    spmm_persistent_kernel<LANES, VEC, TUNE, FULL><<<(unsigned)grid, block, task_smem(block), stream>>>(a);
-}
 
-// Args = RunArgs (extra = nothing) or PersistArgs (extra = grid)
-template <int LANES, int VEC, class Args, class... Extra>
-void launch_shape(const Args &a, int block, int tune, bool full, cudaStream_t stream, Extra... extra) {
+template <int LANES, int VEC>
+void launch_shape(const RunArgs &a, int block, int tune, bool full, cudaStream_t stream) {
     if (tune == 1) {
-        if (full) launch_tuned<LANES, VEC, 1, true>(a, block, extra..., stream);
-        else launch_tuned<LANES, VEC, 1, false>(a, block, extra..., stream);
+        if (full) launch_tuned<LANES, VEC, 1, true>(a, block, stream);
+        else launch_tuned<LANES, VEC, 1, false>(a, block, stream);
     } else {
-        if (full) launch_tuned<LANES, VEC, 0, true>(a, block, extra..., stream);
-        else launch_tuned<LANES, VEC, 0, false>(a, block, extra..., stream);
+        if (full) launch_tuned<LANES, VEC, 0, true>(a, block, stream);
+        else launch_tuned<LANES, VEC, 0, false>(a, block, stream);
     }
 }
 
-template <class Args, class... Extra>
-int launch_lanes(const Plan &p, const Args &a, bool full, cudaStream_t stream, Extra... extra) {
+int launch_lanes(const Plan &p, const RunArgs &a, bool full, cudaStream_t stream) {
     switch (p.lanes * 10 + p.vec) {
-        case 11: launch_shape<1, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 21: launch_shape<2, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 41: launch_shape<4, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 81: launch_shape<8, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 161: launch_shape<16, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 321: launch_shape<32, 1>(a, p.block, p.tune, full, stream, extra...); break;
-        case 322: launch_shape<32, 2>(a, p.block, p.tune, full, stream, extra...); break;
+        case 11: launch_shape<1, 1>(a, p.block, p.tune, full, stream); break;
+        case 21: launch_shape<2, 1>(a, p.block, p.tune, full, stream); break;
+        case 41: launch_shape<4, 1>(a, p.block, p.tune, full, stream); break;
+        case 81: launch_shape<8, 1>(a, p.block, p.tune, full, stream); break;
+        case 161: launch_shape<16, 1>(a, p.block, p.tune, full, stream); break;
+        case 321: launch_shape<32, 1>(a, p.block, p.tune, full, stream); break;
+        case 322: launch_shape<32, 2>(a, p.block, p.tune, full, stream); break;
         default:
             set_error("unsupported kernel shape lanes=%d vec=%d", p.lanes, p.vec);
             return SPMM_B200_EINVAL;
@@ -773,16 +580,11 @@ int launch_lanes(const Plan &p, const Args &a, bool full, cudaStream_t stream, E
 }
 
 template <int LANES, int VEC>
-int slots_shape(int block, int tune, bool persistent) {
+int slots_shape(int block, int tune) {
     int nb = 0;
     const size_t smem = task_smem(block);
-    cudaError_t e;
-    if (persistent)
-        e = tune == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_persistent_kernel<LANES, VEC, 1, true>, block, smem)
-                      : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_persistent_kernel<LANES, VEC, 0, true>, block, smem);
-    else
-        e = tune == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 1, true>, block, smem)
-                      : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 0, true>, block, smem);
+    const cudaError_t e = tune == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 1, true>, block, smem)
+                                    : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 0, true>, block, smem);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return 0;
@@ -790,15 +592,15 @@ int slots_shape(int block, int tune, bool persistent) {
     return nb;
 }
 
-int ctas_per_sm(int lanes, int vec, int tune, int block, bool persistent) {
+int ctas_per_sm(int lanes, int vec, int tune, int block) {
     switch (lanes * 10 + vec) {
-        case 11: return slots_shape<1, 1>(block, tune, persistent);
-        case 21: return slots_shape<2, 1>(block, tune, persistent);
-        case 41: return slots_shape<4, 1>(block, tune, persistent);
-        case 81: return slots_shape<8, 1>(block, tune, persistent);
-        case 161: return slots_shape<16, 1>(block, tune, persistent);
-        case 321: return slots_shape<32, 1>(block, tune, persistent);
-        case 322: return slots_shape<32, 2>(block, tune, persistent);
+        case 11: return slots_shape<1, 1>(block, tune);
+        case 21: return slots_shape<2, 1>(block, tune);
+        case 41: return slots_shape<4, 1>(block, tune);
+        case 81: return slots_shape<8, 1>(block, tune);
+        case 161: return slots_shape<16, 1>(block, tune);
+        case 321: return slots_shape<32, 1>(block, tune);
+        case 322: return slots_shape<32, 2>(block, tune);
         default: return 0;
     }
 }
@@ -853,32 +655,6 @@ int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t
     *launches = 0;
     if (h->num_v == 0 || h->feat == 0) return 0;
     const bool full = !p.scalar && h->feat % (p.lanes * p.vec * 4) == 0 && p.kslice == p.lanes * p.vec * 4;
-    // One persistent launch for all column blocks — unless the passes wait for uploads between launches (band_ready:
-    // the host-buffer calls, which PCIe bounds anyway).
-    if (p.persistent && !band_ready) {
-        PersistArgs a;
-        fill_common(a.c, h, vin, vout, cfinal);
-        a.all = BandArgs();
-        a.all.lpanel = p.d_lpanel_all;
-        a.all.panel = p.d_panel_all;
-        a.all.seg_desc = p.d_pseg_desc;
-        a.all.seg_hrow = p.d_pseg_hrow;
-        a.all.heavy_seg0 = p.d_pheavy_seg0;
-        a.all.seg_count = p.d_seg_count_all;
-        a.all.part = p.d_part_all;
-        a.ptask = p.d_ptask;
-        a.total = p.n_ptask;
-        a.ctr = p.d_ctr;
-        a.n_groups = p.n_groups;
-        a.batch = p.ticket_batch;
-        if (a.total > 0) {
-            int rc = launch_lanes(p, a, full, stream, p.persist_grid);
-            if (rc) return rc;
-            ++*launches;
-        }
-        SB_CUDA(cudaGetLastError());
-        return 0;
-    }
     // Two-stream launches: every pass goes out as two kernels, the first half of the row groups on the caller's stream and
     // the second half on a stream of the handle's. A pass only depends on the previous pass over the SAME rows, so each
     // stream is its own chain, and while one kernel drains its last wave the other stream's kernel fills the freed SMs:
@@ -931,11 +707,8 @@ int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t
 
 // warps the device keeps resident for this kernel shape (0 when it cannot be queried, e.g. no device)
 int resident_warps(int lanes, int vec, int tune, int block) {
-    return ctas_per_sm(lanes, vec, tune, block, false) * (block / 32) * sm_count();
+    return ctas_per_sm(lanes, vec, tune, block) * (block / 32) * sm_count();
 }
-
-// CTAs of the persistent launch: as many as are co-resident
-int persistent_grid(int lanes, int vec, int tune, int block) { return ctas_per_sm(lanes, vec, tune, block, true) * sm_count(); }
 
 // grid cap for the grid-stride support kernels: 16 CTAs per SM of the current device
 static long long stride_grid_cap() {

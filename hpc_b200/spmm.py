@@ -206,9 +206,7 @@ class SpMMB200(SpMM):
                                (5, "light_desc", info["n_light"] * 4), (6, "seg_hrow", info["n_seg"]),
                                (7, "split", (nb + 1) * self.num_v if nb > 1 else 0),
                                (8, "ltask", info["n_ltask"] * 2), (9, "lpanel", info["lpanel_len"] * 2),
-                               (10, "utask", info["n_utask"] * 2), (11, "ptask", info["n_tickets"] * 4),
-                               (12, "group_row", info["n_row_groups"] + 1),
-                               (13, "counters", (2 + info["n_row_groups"] + 1) * 32 if info["persistent"] else 0)):
+                               (10, "utask", info["n_utask"] * 2), (12, "group_row", info["n_row_groups"] + 1)):
             a = np.empty(n, dtype=np.int32)
             check(lib.spmm_b200_plan_copy(self._h, which, a.ctypes.data_as(C.c_void_p), a.nbytes))
             out[name] = a
@@ -218,7 +216,6 @@ class SpMMB200(SpMM):
         out["ltask"] = out["ltask"].reshape(-1, 2)
         out["utask"] = out["utask"].reshape(-1, 2)
         out["lpanel"] = out["lpanel"].reshape(-1, 2)
-        out["ptask"] = out["ptask"].reshape(-1, 4)
         if nb > 1:
             out["split"] = out["split"].reshape(nb + 1, self.num_v)
         return out

@@ -53,13 +53,9 @@ int spmm_b200_set_feat(spmm_b200_t h, int feat_in);
  *               columns inside each row, otherwise falls back to 1
  *   "split_streams" -1 (default) = with several column blocks every pass goes out as two launches, the two halves of
  *               the rows, on two streams (each tail overlaps the next launch), 0 = one launch per column block, 1 = on
- *   "persistent" 1 = run() is one persistent launch over all column blocks (a grid of co-resident warps draws tasks from
- *               a counter; band b+1's tasks wait for band b's tasks of the same row group). Needs feat_in <= 256.
- *               Default off: measured slower than the two-stream launches (profiles/r02_notes.md)
  *   "row_groups" contiguous row groups, balanced by nonzeros, that no task spans (0 = auto: 16 in natural row order, 2
- *               in bucketed order with several column blocks, else 1; at most 64): the unit of parallel planning, of the
- *               two-stream launches and of the persistent launch's dependencies
- *   "ticket_batch" persistent launch: tickets drawn per atomic while far from the end (0 = auto)
+ *               in bucketed order with several column blocks, else 1; at most 64): the unit of parallel planning and of
+ *               the two-stream launches
  *   "host_bands" 1 = lay the column blocks out for spmm_b200_run_host: the last block takes the last 40 % of B's rows
  *               (its pass is bound by the PCIe transfer of C anyway), the blocks before it share the rest (the first
  *               pass starts sooner, the rest finishes under the upload of B); 10..90 = that percentage instead of 40.
@@ -189,9 +185,10 @@ typedef struct {
     int resident_warps; /* warps the device keeps resident for the kernel shape (sizes small graphs' tasks) */
     int n_col_blocks;   /* passes over A, one per band of B rows (1 = the whole matrix at once) */
     int col_begin, col_end; /* band of B rows of the selected column block */
-    int persistent;     /* 1: run() is ONE persistent launch over all column blocks (tickets drawn from a counter) */
-    int n_row_groups;   /* row groups ordering the column-block passes inside that launch (1 = whole bands) */
-    int n_tickets;      /* tasks of the persistent launch (all column blocks) */
+    int persistent;     /* always 0: the single-launch mode it reported was removed; kept so that the layout of this
+                           struct, and every reader of it, stays as it was */
+    int n_row_groups;   /* row groups: contiguous row ranges balanced by nonzeros that no task spans (1 = whole bands) */
+    int n_tickets;      /* always 0, for the same reason as `persistent` */
 } spmm_b200_plan_info_t;
 
 /* With n_col_blocks > 1 the plan holds one set of arrays per column block; plan_info / plan_copy
@@ -220,13 +217,6 @@ int spmm_b200_plan_info(spmm_b200_t h, spmm_b200_plan_info_t *info);
  *   6 seg_hrow   int32[n_seg]       index into heavy_rows of each segment's row
  *   7 split      int32[(n_col_blocks+1)*num_v]  block-major: CSR position where column block b starts
  *                                   in row r (empty when n_col_blocks == 1)
- *  11 ptask      int32[n_tickets*4]  the persistent launch's ticket list, band-major (not per block): {lpanel offset
- *                                   over all blocks, or -1 - segment over all blocks; steps; row group | accumulate << 16
- *                                   | final << 17; completed tasks of that row group the task waits for}
- *  13 counters   uint32[(2+n_row_groups+1)*32] the persistent launch's counters, one per 128-byte line (word 32*i):
- *                                   ticket, exited warps, completions per row group — all zero between runs — then the
- *                                   watchdog's line {kind, ...}: non-zero kind = a wait inside the launch timed out
- *                                   (1 staged chunk, 2 row-group dependency)
  *  12 group_row  int32[n_row_groups+1] first row of each row group (row g's bound: first row with ptr >= g*nnz/groups)
  * Returns SPMM_B200_EINVAL when `bytes` is not the exact size. */
 int spmm_b200_plan_copy(spmm_b200_t h, int which, void *host_dst, size_t bytes);

@@ -185,7 +185,7 @@ def pack_light(cost, groups: int, steps: int, cuts=()):
     """Light-stream packing. cost[i] = nonzeros + 1 of the i-th light row in plan order. A row goes to the
     least-filled lane of the current task (lowest index on ties); when that lane is non-empty and would exceed
     `steps`, the task is closed first. `cuts`: row positions before which an open task is closed (row-group
-    boundaries of the persistent launch). -> (dst slots, tasks [(offset, steps)], panel length)"""
+    boundaries: the groups are packed one by one). -> (dst slots, tasks [(offset, steps)], panel length)"""
     dst, tasks = [], []
     fill = [0] * groups
     off = 0
@@ -214,7 +214,7 @@ def pack_light(cost, groups: int, steps: int, cuts=()):
 
 def light_stream(plan_dict, idx, val, groups: int, steps: int, k4: int = 1, group_row=None) -> dict:
     """light_desc with header slots, task list and the stream panel for a plan() result. group_row: the row-group
-    bounds of the persistent launch (natural row order): no task spans a bound."""
+    bounds: no task spans a bound."""
     ld = plan_dict["light_desc"].copy()
     grp = row_groups_of(int(ld[:, 0].max()) + 1 if len(ld) else 0, group_row)[ld[:, 0]] if len(ld) else np.zeros(0, np.int64)
     cuts = [i for i in range(1, len(ld)) if grp[i] != grp[i - 1]]     # the light rows are group-major in either order
@@ -254,29 +254,12 @@ def unified_tasks(plan_dict, stream_dict, reorder: bool, group_row=None) -> np.n
     return np.asarray([k[2] for k in keyed], np.int32).reshape(-1, 2)
 
 
-def ticket_list(blocks, group_row) -> np.ndarray:
-    """The persistent launch's ticket list. blocks: per column block (utask, light_desc, seg_desc, lpanel length, panel
-    length) in band order. One int32[4] per task, band-major: {lpanel offset over all blocks | -1 - segment over all
-    blocks, steps, row group | accumulate << 16 | final << 17, tasks of that row group in the earlier bands (the
-    completions the task waits for; 0 in the first band)}. A task's row group is that of the row it starts with."""
-    group_row = np.asarray(group_row, np.int64)
-    ng = len(group_row) - 1
-    out, done = [], [0] * ng
-    lp0 = seg0 = 0
-    nb = len(blocks)
-    for b, (utask, light_desc, seg_desc, lpanel_len, panel_len) in enumerate(blocks):
-        first_row = {int(d): int(r) for r, _, _, d in light_desc}
-        flags = ((1 << 16) if b > 0 else 0) | ((1 << 17) if b + 1 == nb else 0)
-        here = [0] * ng
-        for x, y in utask:
-            row = int(seg_desc[-1 - x][0]) if x < 0 else first_row[int(x)]
-            g = int(np.searchsorted(group_row, row, side="right")) - 1 if ng > 1 else 0
-            here[g] += 1
-            out.append((-1 - (seg0 + (-1 - int(x))) if x < 0 else lp0 + int(x), int(y), g | flags, done[g] if b > 0 else 0))
-        done = [a + c for a, c in zip(done, here)]
-        lp0 += lpanel_len
-        seg0 += len(seg_desc)
-    return np.asarray(out, np.int32).reshape(-1, 4)
+def task_groups(utask, light_desc, seg_desc, group_row) -> np.ndarray:
+    """Row group of every task of one block's utask: that of the row the task starts with (a light task's first row is
+    the row whose header sits at its offset)."""
+    first_row = {int(d): int(r) for r, _, _, d in light_desc}
+    rows = [int(seg_desc[-1 - x][0]) if x < 0 else first_row[int(x)] for x, _ in utask]
+    return np.searchsorted(np.asarray(group_row, np.int64), np.asarray(rows, np.int64), side="right") - 1
 
 
 def student_split_check(ptr, tasks) -> bool:

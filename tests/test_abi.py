@@ -34,6 +34,8 @@ def test_status_codes_without_gpu():
     assert rc == -1 and b"bad arguments" in lib.spmm_b200_last_error()
     assert lib.spmm_b200_create(None, None, None, 0, 0, 32, ctypes.byref(h)) == 0
     assert lib.spmm_b200_set_option(h, b"nonsense", 1) == -1
+    assert lib.spmm_b200_set_option(h, b"persistent", 1) == -1      # removed options are unknown names
+    assert lib.spmm_b200_set_option(h, b"ticket_batch", 1) == -1
     assert lib.spmm_b200_set_option(h, b"kslice", 6) == -1          # not a multiple of 4
     assert lib.spmm_b200_run(h, None, None, None) == -2             # run before preprocess
     assert b"preprocess" in lib.spmm_b200_last_error()

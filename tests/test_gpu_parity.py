@@ -437,7 +437,7 @@ def test_run_host_matches_device_run(opts):
         op.run_host(h_in, h_out)
         assert np.array_equal(h_out.numpy().view(np.int32), got.ravel().view(np.int32))
     info = op.plan_info()
-    want = 1 if info["persistent"] else info["n_col_blocks"] * (2 if info["n_col_blocks"] > 1 else 1)   # row halves on two streams
+    want = info["n_col_blocks"] * (2 if info["n_col_blocks"] > 1 else 1)   # row halves on two streams
     assert op.run_profiled(vin, vout) > 0 and op.launches_per_run == want
     op.close()
 
@@ -517,22 +517,23 @@ def test_column_block_plan_matches_oracle(shape, K, nb, seg_len):
 
 @pytest.mark.parametrize("shape,K,nb,seg_len,groups,natural", [("c0", 256, 3, 32, 4, True), ("arxiv", 256, 4, 0, 16, True), ("c0", 32, 3, 16, 1, False),
                                                                ("c0", 128, 1, 64, 0, True), ("c0", 64, 3, 16, 0, False), ("arxiv", 256, 5, 0, 3, False)])
-def test_persistent_plan_matches_oracle(shape, K, nb, seg_len, groups, natural):
-    """The single persistent launch: row groups, tasks cut at group bounds, band-major ticket list with dependency
-    counts — every array against the numpy restatement (oracle/plan_oracle.py::ticket_list)."""
+def test_row_group_plan_matches_oracle(shape, K, nb, seg_len, groups, natural):
+    """Row groups with column blocks in either row order: tasks cut at group bounds — every array against the numpy
+    restatement — and the launches that the row-group halves give (two per pass on two streams with several blocks)."""
     ptr, idx = H.gen_named_graph(shape)
     g, vin, vout = dev_inputs(ptr, idx, K)
-    op = H.SpMMB200(g, K, col_blocks=nb, seg_len=seg_len, reorder=0 if natural else 1, persistent=1, row_groups=groups)
+    op = H.SpMMB200(g, K, col_blocks=nb, seg_len=seg_len, reorder=0 if natural else 1, row_groups=groups)
     op.preprocess(vin, vout)
     info = op.plan_info(0)
-    assert info["persistent"] == 1 and info["n_col_blocks"] == nb
+    assert info["n_col_blocks"] == nb
     want_groups = groups or (16 if natural else (2 if nb > 1 else 1))
     assert info["n_row_groups"] == want_groups
     M = g.num_v
     val = g.val.cpu().numpy()
     group_row = P.partition_rows(ptr, want_groups)
     split = P.split_rows(ptr, idx, nb, M) if nb > 1 else np.stack([ptr[:-1], ptr[1:]])
-    blocks, n_tasks = [], 0
+    two_streams = nb > 1 and want_groups > 1        # option split_streams = -1 (auto)
+    launches = 0
     for b in range(nb):
         got = op.plan_arrays(b)
         inf = op.plan_info(b)
@@ -544,21 +545,18 @@ def test_persistent_plan_matches_oracle(shape, K, nb, seg_len, groups, natural):
         want["utask"] = P.unified_tasks(want, want, not natural, group_row)
         for k in ("row_perm", "light_desc", "ltask", "lpanel", "heavy_rows", "heavy_seg0", "seg_desc", "seg_hrow", "panel", "utask"):
             assert np.array_equal(got[k], want[k]), (b, k)
-        blocks.append((want["utask"], want["light_desc"], want["seg_desc"], len(want["lpanel"]), len(want["panel"])))
-        n_tasks += len(want["utask"])
-    tickets = P.ticket_list(blocks, group_row)
-    assert info["n_tickets"] == n_tasks == len(tickets)
-    assert np.array_equal(op.plan_arrays(0)["ptask"], tickets)
-    # no light task spans a row-group bound; dependency counts never exceed the tasks issued before the ticket
-    grp, need = tickets[:, 2] & 0xffff, tickets[:, 3]
-    assert np.all(need <= np.arange(len(tickets)))
-    assert np.all(grp < want_groups)
-    # and it computes the right thing, repeatedly (the counters return to zero after every run)
+        # the tasks are group-major: the second stream takes the tasks of the second half of the groups
+        grp = P.task_groups(want["utask"], want["light_desc"], want["seg_desc"], group_row)
+        assert np.all(np.diff(grp) >= 0) and np.all(grp < want_groups)
+        n = len(want["utask"])
+        cut = int(np.searchsorted(grp, (want_groups + 1) // 2)) if two_streams else n
+        launches += (cut > 0) + (n > cut)
+    # and it computes the right thing, repeatedly (the segment counters return to zero after every run)
     for _ in range(3):
         vout.fill_(float("nan"))
         op.run(vin, vout)
     torch.cuda.synchronize()
-    assert op.launches_per_run == 1
+    assert op.launches_per_run == launches
     check_against_oracle(ptr, idx, K, op, g, vin, vout[: M * K].cpu().numpy().reshape(M, K))
     op.close()
 
@@ -644,7 +642,7 @@ def test_auto_row_order_rule():
     op = H.SpMMB200(g, 256, col_blocks=3)
     op.preprocess(vin, vout)
     info = op.plan_info()
-    assert info["reorder"] == 1 and info["n_row_groups"] == 2 and info["persistent"] == 0
+    assert info["reorder"] == 1 and info["n_row_groups"] == 2
     vout.fill_(float("nan"))
     op.run(vin, vout)
     torch.cuda.synchronize()
@@ -891,7 +889,7 @@ def test_feat_zero_is_a_no_op():
 # ---- the transposed operator: dB = A^T dC (SURVEY.md 8f-3; no reference counterpart, parity unpinned) ---------
 
 @pytest.mark.parametrize("shape,K,opts", [("c0", 32, {}), ("c0", 256, {"seg_len": 32}), ("arxiv", 256, {}), ("arxiv", 32, {}),
-                                           ("c0", 33, {}), ("c0", 64, {"col_blocks": 3, "persistent": 1})])
+                                           ("c0", 33, {}), pytest.param("c0", 64, {"col_blocks": 3}, id="c0-64-col_blocks3")])
 def test_transposed_operator_matches_oracle(shape, K, opts):
     ptr, idx = H.gen_named_graph(shape)
     g, vin, vout = dev_inputs(ptr, idx, K)
@@ -1115,10 +1113,10 @@ def test_reference_test_driver_with_engine_dropped_in(tmp_path, shape, K):
     assert len(times) == 2 and all(t > 0 for t in times)          # cuSPARSE, then the engine (test_spmm.cu:46-62)
 
 
-@pytest.mark.parametrize("K,opts", [(32, {}), (64, {"col_blocks": 3}), (64, {"col_blocks": 3, "persistent": 1})])
+@pytest.mark.parametrize("K,opts", [(32, {}), (64, {"col_blocks": 3})])
 def test_run_is_capturable_in_a_cuda_graph(K, opts):
     """run() makes no host synchronisation, so a launch-bound caller can capture it once and replay it — also when the
-    passes go out on two streams (fork / join inside the capture) and as the one persistent launch."""
+    passes go out on two streams (fork / join inside the capture)."""
     ptr, idx = H.gen_named_graph("arxiv")
     g, vin, vout = dev_inputs(ptr, idx, K)
     op = H.SpMMB200(g, K, **opts)

@@ -94,11 +94,11 @@ def test_edge_cases(name, K):
 
 
 OPTION_SETS = [{}, {"col_blocks": 1}, {"col_blocks": 3}, {"reorder": 0}, {"reorder": 1}, {"seg_len": 64},
-               {"kslice": 32}, {"persistent": 1, "col_blocks": 3}, {"split_streams": 0, "col_blocks": 3},
+               {"kslice": 32}, {"split_streams": 0, "col_blocks": 3},
                {"split_streams": 1, "col_blocks": 3}, {"host_bands": 1, "col_blocks": 4}]
 
 
-@pytest.mark.parametrize("K", [32, 256])
+@pytest.mark.parametrize("K", [32, 256], ids=["K32", "K256"])
 def test_same_bits_under_every_option(K):
     ptr, idx = H.gen_named_graph("arxiv")
     first = None
@@ -176,7 +176,7 @@ def test_identity_with_the_forward_product():
     op.close()
 
 
-@pytest.mark.parametrize("opts", [{}, {"col_blocks": 3}, {"persistent": 1, "col_blocks": 3}])
+@pytest.mark.parametrize("opts", [{}, {"col_blocks": 3}])
 def test_run_sddmm_run_and_repeat_are_bit_identical(opts):
     ptr, idx = H.gen_named_graph("arxiv")
     M, K = len(ptr) - 1, 256

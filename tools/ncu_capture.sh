@@ -18,6 +18,5 @@ cap reddit_k256 spmm_kernel 20 5
 cap products_k256 spmm_kernel 4 1 --workload products_k256
 cap arxiv_k256 spmm_kernel 4 1 --workload arxiv_k256
 cap arxiv_k32 spmm_kernel 4 1 --workload arxiv_k32
-cap reddit_k256_persistent spmm_persistent 4 1 --opt persistent=1
 cp $T/r02_prof_products_k256.ncu-rep $O/
 ls -la $O | tail -20

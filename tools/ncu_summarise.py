@@ -13,7 +13,7 @@ import bench
 rows = list(csv.reader(open(sys.argv[1])))
 hdr, units = rows[0], rows[1]
 workload = sys.argv[2]
-pat = re.compile(sys.argv[3] if len(sys.argv) > 3 else r"spmm_(kernel|persistent)")
+pat = re.compile(sys.argv[3] if len(sys.argv) > 3 else r"spmm_kernel")
 kn = hdr.index("Kernel Name")
 sel = [r for r in rows[2:] if pat.search(r[kn])]
 SCALE = {"byte": 1, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9, "Tbyte": 1e12, "ns": 1e-6, "us": 1e-3, "ms": 1.0, "s": 1e3,

@@ -27,9 +27,9 @@ for parts in (8, 4, 2, 1):
     mid = int(H.partition_rows(H.rebase_ptr(ptr, r0, r1), 2)[1]) + r0
     res = {}
     for name, reorder in (("bucketed", 1), ("natural", 0), ("auto", -1)):
-        one, out1, _g = make(r0, r1, persistent=0, split_streams=0, reorder=reorder)
-        a_op, a_out, _ga = make(r0, mid, persistent=0, split_streams=0, reorder=reorder)
-        b_op, b_out, _gb = make(mid, r1, persistent=0, split_streams=0, reorder=reorder)
+        one, out1, _g = make(r0, r1, split_streams=0, reorder=reorder)
+        a_op, a_out, _ga = make(r0, mid, split_streams=0, reorder=reorder)
+        b_op, b_out, _gb = make(mid, r1, split_streams=0, reorder=reorder)
         s1 = torch.cuda.Stream()
         def run_two():
             s1.wait_stream(torch.cuda.current_stream())
