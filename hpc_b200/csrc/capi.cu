@@ -361,14 +361,14 @@ int spmm_b200_plan_copy(spmm_b200_t h, int which, void *host_dst, size_t bytes) 
     const void *src = nullptr;
     size_t want = 0;
     switch (which) {
-        case 0: src = p.d_row_perm; want = sizeof(int) * (size_t)p.n_light; break;
-        case 1: src = p.d_heavy_rows; want = sizeof(int) * (size_t)p.n_heavy; break;
+        case 0: src = p.d_light_desc; want = sizeof(int) * (size_t)p.n_light; break;
+        case 1: src = p.d_seg_desc; want = sizeof(int) * (size_t)p.n_heavy; break;
         case 2: src = p.d_heavy_seg0; want = p.n_heavy ? sizeof(int) * ((size_t)p.n_heavy + 1) : 0; break;
         case 3: src = p.d_seg_desc; want = sizeof(SegDesc) * (size_t)p.n_seg; break;
         case 4: src = p.d_panel; want = sizeof(int2) * (size_t)p.panel_len; break;
         case 5: src = p.d_light_desc; want = sizeof(int4) * (size_t)p.n_light; break;
         case 6: src = p.d_seg_hrow; want = sizeof(int) * (size_t)p.n_seg; break;
-        case 8: src = p.d_ltask; want = sizeof(int2) * (size_t)p.n_ltask; break;
+        case 8: src = p.d_utask; want = sizeof(int2) * (size_t)p.n_ltask; break;
         case 10: src = p.d_utask; want = sizeof(int2) * (size_t)p.n_utask; break;
         case 9: src = p.d_lpanel; want = sizeof(int2) * (size_t)p.lpanel_len; break;
         case 7:
@@ -392,7 +392,30 @@ int spmm_b200_plan_copy(spmm_b200_t h, int which, void *host_dst, size_t bytes) 
         set_error("spmm_b200_plan_copy: array %d is empty", which);
         return SPMM_B200_ESTATE;
     }
-    SB_CUDA(cudaMemcpy(host_dst, src, want, cudaMemcpyDeviceToHost));
+    // No kernel reads arrays 0, 1 and 8, so the device does not keep them. They are projections of the arrays that `src` is:
+    // row_perm[i] == light_desc[i].x; heavy_rows[i] == seg_desc[heavy_seg0[i]].row; ltask == the entries of utask with x >= 0
+    // (not a heavy segment) in their order: planning takes the light tasks in sequence in either row order, and the row
+    // groups' concatenation shifts both arrays by the same offsets.
+    int *out = static_cast<int *>(host_dst);
+    if (which == 0) {
+        std::vector<int4> light((size_t)p.n_light);
+        SB_CUDA(cudaMemcpy(light.data(), src, sizeof(int4) * light.size(), cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < light.size(); ++i) out[i] = light[i].x;
+    } else if (which == 1) {
+        std::vector<SegDesc> segs((size_t)p.n_seg);
+        std::vector<int> seg0((size_t)p.n_heavy);
+        SB_CUDA(cudaMemcpy(segs.data(), src, sizeof(SegDesc) * segs.size(), cudaMemcpyDeviceToHost));
+        SB_CUDA(cudaMemcpy(seg0.data(), p.d_heavy_seg0, sizeof(int) * seg0.size(), cudaMemcpyDeviceToHost));
+        for (size_t i = 0; i < seg0.size(); ++i) out[i] = segs[(size_t)seg0[i]].row;
+    } else if (which == 8) {
+        std::vector<int2> utask((size_t)p.n_utask);
+        SB_CUDA(cudaMemcpy(utask.data(), src, sizeof(int2) * utask.size(), cudaMemcpyDeviceToHost));
+        int2 *ltask = static_cast<int2 *>(host_dst);
+        for (size_t i = 0, n = 0; i < utask.size() && n < (size_t)p.n_ltask; ++i)
+            if (utask[i].x >= 0) ltask[n++] = utask[i];
+    } else {
+        SB_CUDA(cudaMemcpy(host_dst, src, want, cudaMemcpyDeviceToHost));
+    }
     return 0;
 }
 

@@ -34,6 +34,8 @@ struct SegDesc {
 };
 
 constexpr int kMaxBands = 16;    // cap of the automatic number of column blocks
+// Bytes of B per column-block band, and per chunk of run_host_sharded's upload of B, so that chunks and bands coincide
+constexpr long long kBandBytes = 48ll << 20;
 constexpr int kMaxRowGroups = 64;
 
 // What every pass of a run shares.
@@ -77,29 +79,18 @@ struct RunArgs {
     BandArgs b;
 };
 
-// The plan of one column block (the whole matrix when there is a single block).
+// The plan of one column block (the whole matrix when there is a single block): its counts and its device arrays.
 struct BlockPlan {
     int col_begin = 0, col_end = 0;   // B rows [col_begin, col_end) are gathered in this pass
-    int n_light = 0, n_heavy = 0, n_seg = 0;
-    long long panel_len = 0;
-    int *d_row_perm = nullptr;
-    int4 *d_light_desc = nullptr;
-    int2 *d_ltask = nullptr;
-    int2 *d_utask = nullptr;
-    int n_utask = 0;
-    int2 *d_lpanel = nullptr;
-    int n_ltask = 0;
-    int light_steps = 0;
-    int reorder = 1;
-    long long lpanel_len = 0;
-    int *d_heavy_rows = nullptr;
-    int *d_heavy_seg0 = nullptr;
-    SegDesc *d_seg_desc = nullptr;
-    int *d_seg_hrow = nullptr;
-    int *d_seg_count = nullptr;
-    int2 *d_panel = nullptr;
-    float *d_part = nullptr;
+    int reorder = 1, light_steps = 0;
+    int n_light = 0, n_heavy = 0, n_seg = 0, n_ltask = 0, n_utask = 0;
+    long long panel_len = 0, lpanel_len = 0;
     int split_task = 0;            // first task of the second half of the row groups (two-stream launches); 0 / n_utask: no split
+    int4 *d_light_desc = nullptr;
+    int2 *d_utask = nullptr, *d_lpanel = nullptr, *d_panel = nullptr;
+    SegDesc *d_seg_desc = nullptr;
+    int *d_heavy_seg0 = nullptr, *d_seg_hrow = nullptr, *d_seg_count = nullptr;
+    float *d_part = nullptr;
 };
 
 struct Plan {

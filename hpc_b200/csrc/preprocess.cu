@@ -50,11 +50,8 @@ void free_plan(Plan &p) {
     if (p.d_split || !p.blocks.empty()) cudaDeviceSynchronize();
     auto release = [](void *q) { pool_free(q, cudaStreamLegacy); };
     for (BlockPlan &b : p.blocks) {
-        release(b.d_row_perm);
         release(b.d_light_desc);
-        release(b.d_ltask);
         release(b.d_utask);
-        release(b.d_heavy_rows);
         release(b.d_heavy_seg0);
         release(b.d_seg_desc);
         release(b.d_seg_hrow);
@@ -103,8 +100,7 @@ int auto_kslice(int num_v, int feat) {
 int auto_col_blocks(long long b_rows, int feat, long long nnz, int num_v) {
     const long long b_bytes = b_rows * feat * 4ll;
     if (feat % 4 != 0 || num_v <= 0 || b_bytes <= (96ll << 20)) return 1;
-    const long long band = 48ll << 20;
-    long long nb = (b_bytes + band - 1) / band;
+    long long nb = (b_bytes + kBandBytes - 1) / kBandBytes;
     if (nb > 16) return 1;
     if (nnz / num_v / nb < 64) return 1;
     return (int)nb;
@@ -240,31 +236,15 @@ int auto_light_steps(int groups, long long total_cost, long long slots, long lon
     return (int)(st < dflt ? st : dflt);
 }
 
-// Everything the host works out for one column block before anything is allocated on the device.
-struct HostBlock {
-    std::vector<int> row_perm, heavy_rows, heavy_seg0, seg_hrow;
-    std::vector<SegDesc> segs;
+// The host arrays of one column block, from host planning to their upload (the block's counts go to its BlockPlan).
+struct BlockArrays {
     std::vector<int4> light;
-    std::vector<int2> ltasks, utask;
-    long long panel_len = 0, lpanel_len = 0;
-    int reorder = 1, light_steps = 0;
-    int split_task = 0;   // first task of the second half of the row groups
+    std::vector<int2> utask;
+    std::vector<SegDesc> segs;
+    std::vector<int> heavy_seg0, seg_hrow;
     int rc = 0;
-    char err[256] = "";
+    char err[256] = "";   // set_error keeps one message per thread, and the blocks are planned on several
 };
-
-// Row order of a block. Degree buckets (longest first) shorten the tail and keep the lanes of a task balanced; natural
-// order keeps neighbouring rows together, which lets a graph's locality hit in L2. Auto (-1): natural order
-// when a full warp serves each row (no lanes to balance) and the block is at least 8 waves of tasks long (no
-// tail to speak of) — measured 12.2 -> 11.3 ms on the products shape, neutral on reddit, and the opposite
-// (0.14 -> 0.19 ms) on the one-wave arxiv shape, which therefore keeps the buckets (profiles/r01_sweep.md).
-static int block_reorder(const spmm_b200_handle *h, const int *rb, const int *re) {
-    const Plan &p = h->plan;
-    if (h->opt_reorder >= 0) return (int)h->opt_reorder;
-    long long total = 0;
-    for (int r = 0; r < h->num_v; ++r) total += re[r] - rb[r] + 1;
-    return (p.lanes == 32 && p.slots > 0 && total >= 8ll * p.slots * 64) ? 0 : 1;
-}
 
 // The row groups (contiguous row ranges) are planned independently of each other — a task never spans a group bound, and
 // the row order (natural or degree buckets) applies INSIDE a group — so planning group by group and concatenating
@@ -272,11 +252,10 @@ static int block_reorder(const spmm_b200_handle *h, const int *rb, const int *re
 // brings preprocess for the products shape (2.4 M rows) from ~75 ms of serial host work to a few ms. One group is the
 // ungrouped plan.
 static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const int *re, int skip_empty, int reorder, const int *group_row,
-                              int n_groups, HostBlock &hb) {
+                              int n_groups, BlockPlan &bp, BlockArrays &a) {
     const Plan &p = h->plan;
     const int M = h->num_v;
     const int groups = 32 / p.lanes, pad = 4 * groups;
-    hb.reorder = reorder;
     struct Part {
         std::vector<int> row_perm, heavy_rows, heavy_seg0, cost, dst;
         std::vector<SegDesc> segs;
@@ -299,8 +278,8 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
     long long total = 0, n_seg = 0;
     for (Part &x : part) {
         if (x.rc) {
-            hb.rc = x.rc;
-            snprintf(hb.err, sizeof(hb.err), "row planning failed");
+            a.rc = x.rc;
+            snprintf(a.err, sizeof(a.err), "row planning failed");
             return;
         }
         total += x.total_cost;
@@ -308,7 +287,7 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
     }
     int steps = p.light_steps;
     if (h->opt_light_steps <= 0) steps = auto_light_steps(groups, total, p.slots, n_seg * p.n_slices);
-    hb.light_steps = steps;
+    bp.light_steps = steps;
 #pragma omp parallel for schedule(dynamic, 1)
     for (int g = 0; g < n_groups; ++g) {
         Part &x = part[g];
@@ -342,7 +321,7 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
     }
     // concatenate, shifting every offset by what precedes
     std::vector<long long> b_light((size_t)n_groups + 1, 0), b_heavy((size_t)n_groups + 1, 0), b_seg((size_t)n_groups + 1, 0),
-        b_panel((size_t)n_groups + 1, 0), b_lpanel((size_t)n_groups + 1, 0), b_ltask((size_t)n_groups + 1, 0), b_utask((size_t)n_groups + 1, 0);
+        b_panel((size_t)n_groups + 1, 0), b_lpanel((size_t)n_groups + 1, 0), b_utask((size_t)n_groups + 1, 0);
     for (int g = 0; g < n_groups; ++g) {
         const Part &x = part[g];
         b_light[g + 1] = b_light[g] + (long long)x.row_perm.size();
@@ -350,74 +329,69 @@ static void plan_block_groups(const spmm_b200_handle *h, const int *rb, const in
         b_seg[g + 1] = b_seg[g] + (long long)x.segs.size();
         b_panel[g + 1] = b_panel[g] + x.panel_len;
         b_lpanel[g + 1] = b_lpanel[g] + x.lpanel_len;
-        b_ltask[g + 1] = b_ltask[g] + (long long)x.ltasks.size();
         b_utask[g + 1] = b_utask[g] + (long long)x.utask.size();
     }
-    hb.panel_len = b_panel[n_groups];
-    hb.lpanel_len = b_lpanel[n_groups];
-    if (hb.panel_len > 0x7fffffffll || hb.lpanel_len > 0x7fffffffll) {
-        hb.rc = SPMM_B200_EINVAL;
-        snprintf(hb.err, sizeof(hb.err), "panel too large");
+    bp.panel_len = b_panel[n_groups];
+    bp.lpanel_len = b_lpanel[n_groups];
+    if (bp.panel_len > 0x7fffffffll || bp.lpanel_len > 0x7fffffffll) {
+        a.rc = SPMM_B200_EINVAL;
+        snprintf(a.err, sizeof(a.err), "panel too large");
         return;
     }
-    hb.row_perm.resize((size_t)b_light[n_groups]);
-    hb.light.resize((size_t)b_light[n_groups]);
-    hb.heavy_rows.resize((size_t)b_heavy[n_groups]);
-    hb.heavy_seg0.resize(b_heavy[n_groups] ? (size_t)b_heavy[n_groups] + 1 : 0);
-    hb.segs.resize((size_t)b_seg[n_groups]);
-    hb.seg_hrow.resize((size_t)b_seg[n_groups]);
-    hb.ltasks.resize((size_t)b_ltask[n_groups]);
-    hb.utask.resize((size_t)b_utask[n_groups]);
-    hb.split_task = (int)b_utask[(n_groups + 1) / 2];   // the groups' tasks are contiguous, in group order
-    if (b_heavy[n_groups]) hb.heavy_seg0[(size_t)b_heavy[n_groups]] = (int)b_seg[n_groups];
+    bp.n_light = (int)b_light[n_groups];
+    bp.n_heavy = (int)b_heavy[n_groups];
+    bp.n_seg = (int)b_seg[n_groups];
+    bp.n_utask = (int)b_utask[n_groups];
+    bp.n_ltask = bp.n_utask - bp.n_seg;   // every segment is one task
+    bp.split_task = (int)b_utask[(n_groups + 1) / 2];   // the groups' tasks are contiguous, in group order
+    a.light.resize((size_t)bp.n_light);
+    a.heavy_seg0.resize(bp.n_heavy ? (size_t)bp.n_heavy + 1 : 0);
+    a.segs.resize((size_t)bp.n_seg);
+    a.seg_hrow.resize((size_t)bp.n_seg);
+    a.utask.resize((size_t)bp.n_utask);
+    if (bp.n_heavy) a.heavy_seg0[(size_t)bp.n_heavy] = bp.n_seg;
 #pragma omp parallel for schedule(dynamic, 1)
     for (int g = 0; g < n_groups; ++g) {
         const Part &x = part[g];
         const int lp = (int)b_lpanel[g], pn = (int)b_panel[g], sg = (int)b_seg[g], hv = (int)b_heavy[g];
         for (size_t i = 0; i < x.row_perm.size(); ++i) {
             const int r = x.row_perm[i];
-            hb.row_perm[(size_t)b_light[g] + i] = r;
-            hb.light[(size_t)b_light[g] + i] = make_int4(r, rb[r], re[r] - rb[r], lp + x.dst[i]);
+            a.light[(size_t)b_light[g] + i] = make_int4(r, rb[r], re[r] - rb[r], lp + x.dst[i]);
         }
         for (size_t i = 0; i < x.heavy_rows.size(); ++i) {
-            hb.heavy_rows[(size_t)hv + i] = x.heavy_rows[i];
-            hb.heavy_seg0[(size_t)hv + i] = sg + x.heavy_seg0[i];
-            for (int sgm = x.heavy_seg0[i]; sgm < x.heavy_seg0[i + 1]; ++sgm) hb.seg_hrow[(size_t)sg + sgm] = hv + (int)i;
+            a.heavy_seg0[(size_t)hv + i] = sg + x.heavy_seg0[i];
+            for (int sgm = x.heavy_seg0[i]; sgm < x.heavy_seg0[i + 1]; ++sgm) a.seg_hrow[(size_t)sg + sgm] = hv + (int)i;
         }
         for (size_t i = 0; i < x.segs.size(); ++i) {
             SegDesc d = x.segs[i];
             d.panel_off += pn;
-            hb.segs[(size_t)sg + i] = d;
+            a.segs[(size_t)sg + i] = d;
         }
-        for (size_t i = 0; i < x.ltasks.size(); ++i) hb.ltasks[(size_t)b_ltask[g] + i] = make_int2(lp + x.ltasks[i].x, x.ltasks[i].y);
         for (size_t i = 0; i < x.utask.size(); ++i) {
             const int2 u = x.utask[i];
-            hb.utask[(size_t)b_utask[g] + i] = u.x < 0 ? make_int2(-1 - (sg + (-1 - u.x)), 0) : make_int2(lp + u.x, u.y);
+            a.utask[(size_t)b_utask[g] + i] = u.x < 0 ? make_int2(-1 - (sg + (-1 - u.x)), 0) : make_int2(lp + u.x, u.y);
         }
     }
 }
 
-// Host part of one block: row order, segments, light-stream packing, task order. group_row: the n_groups + 1
-// row-group boundaries. The scalar fallback (K % 4 != 0) keeps every row whole in one group and reads idx/val at run
-// time: its plan is the row order alone.
-static void plan_block_host(const spmm_b200_handle *h, const int *rb, const int *re, int skip_empty, int reorder,
-                            const int *group_row, int n_groups, HostBlock &hb) {
+// The scalar fallback (K % 4 != 0) keeps every row whole in one group and reads idx/val at run time: its plan of a block
+// is the row order alone.
+static void plan_block_scalar(const spmm_b200_handle *h, const int *rb, const int *re, int skip_empty, int reorder, BlockPlan &bp,
+                              BlockArrays &a) {
     const Plan &p = h->plan;
-    if (!p.scalar) {
-        plan_block_groups(h, rb, re, skip_empty, reorder, group_row, n_groups, hb);
+    std::vector<int> row_perm, heavy_rows;
+    a.rc = plan_rows_host(rb, re, h->num_v, p.seg_len, reorder, skip_empty, 2, row_perm, heavy_rows, a.heavy_seg0, a.segs, &bp.panel_len);
+    if (a.rc) {
+        snprintf(a.err, sizeof(a.err), "%s", spmm_b200_last_error());
         return;
     }
-    hb.reorder = reorder;
-    hb.rc = plan_rows_host(rb, re, h->num_v, p.seg_len, reorder, skip_empty, 2, hb.row_perm, hb.heavy_rows, hb.heavy_seg0, hb.segs,
-                           &hb.panel_len);
-    if (hb.rc) {
-        snprintf(hb.err, sizeof(hb.err), "%s", spmm_b200_last_error());
-        return;
-    }
-    hb.light.resize(hb.row_perm.size());
-    for (size_t i = 0; i < hb.row_perm.size(); ++i) {
-        const int r = hb.row_perm[i];
-        hb.light[i] = make_int4(r, rb[r], re[r] - rb[r], 0);
+    bp.n_light = (int)row_perm.size();
+    bp.n_heavy = (int)heavy_rows.size();
+    bp.n_seg = (int)a.segs.size();
+    a.light.resize(row_perm.size());
+    for (size_t i = 0; i < row_perm.size(); ++i) {
+        const int r = row_perm[i];
+        a.light[i] = make_int4(r, rb[r], re[r] - rb[r], 0);
     }
 }
 
@@ -426,6 +400,215 @@ static int upload_vec(T **dst, const std::vector<T> &v, cudaStream_t stream) {
     if (v.empty()) return 0;
     SB_CUDA(pool_alloc((void **)dst, sizeof(T) * v.size(), stream));
     SB_CUDA(cudaMemcpyAsync(*dst, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice, stream));
+    return 0;
+}
+
+// Kernel shape (feature slices, lanes x vec per row slice, segment length, resident warps) and the number of column blocks
+// to aim for. The vectorised kernels address B with 32-bit float4 offsets.
+static int plan_shape(spmm_b200_handle *h, int b_rows, int &nb) {
+    Plan &p = h->plan;
+    const int M = h->num_v, K = h->feat;
+    p.block = (int)h->opt_block;
+    p.scalar = (K % 4) != 0;
+    p.kslice = h->opt_kslice > 0 ? (int)h->opt_kslice : auto_kslice(M, K);
+    if (p.scalar) p.kslice = K;
+    if (p.kslice > 256) p.kslice = 256;
+    if (p.kslice > ((K + 3) & ~3)) p.kslice = (K + 3) & ~3;
+    p.n_slices = (K + p.kslice - 1) / p.kslice;
+    if (!p.scalar) shape_for_kslice(p.kslice, &p.lanes, &p.vec);
+    p.seg_len = h->opt_seg_len > 0 ? (int)h->opt_seg_len : auto_seg_len(h->num_e, p.lanes);
+    p.tune = (int)h->opt_tune;
+    p.light_steps = h->opt_light_steps > 0 ? (int)h->opt_light_steps : 0;
+    p.slots = p.scalar ? 0 : resident_warps(p.lanes, p.vec, p.tune, p.block);
+    if (p.scalar) p.seg_len = 0x7fffffff;   // scalar fallback keeps every row whole
+    if (!p.scalar && (long long)b_rows * (K / 4) > 0x7fffffffll) {
+        set_error("B is too large for 32-bit row offsets: b_rows * feat_in / 4 = %lld >= 2^31", (long long)b_rows * (K / 4));
+        return SPMM_B200_EINVAL;
+    }
+    nb = h->opt_col_blocks > 0 ? (int)h->opt_col_blocks : auto_col_blocks(b_rows, K, h->num_e, M);
+    if (p.scalar || nb < 1) nb = 1;
+    if (nb > kMaxBands && h->opt_col_blocks <= 0) nb = kMaxBands;
+    if (nb > b_rows) nb = b_rows > 0 ? b_rows : 1;
+    return 0;
+}
+
+// Band bounds: band b is B rows [bounds[b], bounds[b + 1]). Default: nb equal bands of ceil(b_rows / nb) rows. Option
+// "host_bands" (the plan is meant for the host-buffer call, spmm_b200_run_host): the LAST band takes the last 40 % of B's
+// rows and the bands before it share the rest. The last pass stores final rows over PCIe and is bound by that transfer
+// whatever it computes, so it may as well carry half of the nonzeros (from a band that no longer fits the L2), while the
+// small early bands let the first pass start sooner and finish the rest of the work under the upload of B.
+static std::vector<int> band_bounds(int b_rows, int nb, long long host_bands) {
+    std::vector<int> bounds;
+    if (host_bands && nb >= 3) {
+        // host_bands = 1: the last band is 40 % of B's rows (measured best on the reddit shape: e2e 10.31 -> 9.34 ms;
+        // 30 %: 9.76, 50 %: 9.60, 60 %: 9.98 — profiles/r02_host_bands.jsonl); 10..90: that percentage
+        const long long pct = host_bands >= 10 ? host_bands : 40;
+        const int small = nb - 1, half = (int)((long long)b_rows * (100 - pct) / 100);
+        const int per = (half + small - 1) / small;
+        for (int b = 0; b < small && b * per < half; ++b) bounds.push_back(b * per);
+        bounds.push_back(half);
+        bounds.push_back(b_rows);
+        return bounds;
+    }
+    const int cols_per_block = nb > 1 ? (b_rows + nb - 1) / nb : b_rows;
+    if (nb > 1) nb = (b_rows + cols_per_block - 1) / cols_per_block;   // every band starts inside B (b_rows = 10, 7 bands -> 5 of 2 rows)
+    for (int b = 0; b < nb; ++b) bounds.push_back(b * cols_per_block);
+    bounds.push_back(b_rows);
+    return bounds;
+}
+
+// CSR read and checks: ptr comes to the host and must hold num_e nonzeros in rows of non-negative degree (whatever the row
+// order, a negative degree would turn into out-of-bounds panel slots). Behind the copy, one pass over idx sets flags[0]
+// when a column is outside B; split_at_bands reads the flags back.
+static int read_csr(const spmm_b200_handle *h, int b_rows, int *d_flags, std::vector<int> &ptr, cudaStream_t stream, PrepTrace &tr) {
+    const int M = h->num_v;
+    ptr.assign((size_t)M + 1, 0);
+    SB_CUDA(cudaMemcpyAsync(ptr.data(), h->d_ptr, sizeof(int) * ((size_t)M + 1), cudaMemcpyDeviceToHost, stream));
+    SB_CUDA(cudaMemsetAsync(d_flags, 0, 2 * sizeof(int), stream));
+    const int rc = launch_check_cols(h->d_idx, h->num_e, b_rows, d_flags, stream);
+    if (rc) return rc;
+    SB_CUDA(cudaStreamSynchronize(stream));
+    if (ptr[0] != 0 || ptr[M] != h->num_e) {
+        set_error("CSR ptr is inconsistent: ptr[0]=%d ptr[num_v]=%d num_e=%d", ptr[0], ptr[M], h->num_e);
+        return SPMM_B200_EINVAL;
+    }
+    for (int r = 0; r < M; ++r)
+        if (ptr[r + 1] < ptr[r]) {
+            set_error("CSR ptr decreases at row %d", r);
+            return SPMM_B200_EINVAL;
+        }
+    tr.lap("ptr D2H + check_cols");
+    return 0;
+}
+
+// Row split: with several bands every row is cut at the band bounds on the device (split[b][r]: where band b starts in
+// row r) and the split comes to the host. That needs ascending columns inside a row: an unsorted CSR keeps one block.
+static int split_at_bands(spmm_b200_handle *h, int b_rows, int *d_flags, std::vector<int> &band_begin, std::vector<int> &split,
+                          cudaStream_t stream) {
+    Plan &p = h->plan;
+    const int M = h->num_v, nb = (int)band_begin.size() - 1;
+    if (nb > 1) {
+        SB_CUDA(pool_alloc((void **)&p.d_split, sizeof(int) * (size_t)(nb + 1) * M, stream));
+        const int rc = launch_split_rows(h->d_ptr, h->d_idx, M, nb, band_begin.data(), p.d_split, d_flags + 1, stream);
+        if (rc) return rc;
+        split.resize((size_t)(nb + 1) * M);
+        SB_CUDA(cudaMemcpyAsync(split.data(), p.d_split, sizeof(int) * split.size(), cudaMemcpyDeviceToHost, stream));
+    }
+    int flags[2] = {0, 0};
+    SB_CUDA(cudaMemcpyAsync(flags, d_flags, sizeof(flags), cudaMemcpyDeviceToHost, stream));
+    SB_CUDA(cudaStreamSynchronize(stream));
+    if (flags[0]) {
+        set_error("CSR idx holds a column outside [0, %d)", b_rows);
+        return SPMM_B200_EINVAL;
+    }
+    if (nb > 1 && flags[1]) {
+        pool_free(p.d_split, stream);
+        p.d_split = nullptr;
+        split.clear();
+        band_begin = {0, b_rows};
+    }
+    return 0;
+}
+
+// Row order, one for every block. Degree buckets (longest rows first) shorten the tail of every launch and keep the lanes
+// of a task balanced; natural order keeps neighbouring rows together, which lets a graph's locality hit in L2. Auto (option
+// reorder = -1): natural order only when locality is what is at stake: ONE block (no column blocks — B is either small or
+// far larger than the L2) in a launch of at least 8 waves of tasks with a full warp per row: measured 12.2 -> 11.3 ms on the
+// products shape and the opposite (0.14 -> 0.19 ms) on the one-wave arxiv shape (profiles/r01_sweep.md). With column blocks
+// every pass gathers from an L2-resident band whatever the order, and buckets win at every partition size of the reddit
+// shape (6.04 vs 6.14 ms whole, 0.80 vs 0.92 ms for a 1/8 block: profiles/r02_notes.md).
+// Row groups: contiguous row ranges balanced by nonzeros (the partition rule, spmm_b200_partition_rows), planned
+// independently (in parallel) and never spanned by a task. Natural order: 16. Degree buckets with several blocks: 2 — the
+// halves that go out on two streams. Otherwise 1.
+static int order_rows(spmm_b200_handle *h, const std::vector<int> &ptr, int nb, int &reorder) {
+    Plan &p = h->plan;
+    const int M = h->num_v;
+    const long long entries = (long long)h->num_e + M;   // the light stream of a single block: every nonzero, a header per row
+    const bool natural = h->opt_reorder >= 0 ? h->opt_reorder == 0 : nb == 1 && p.lanes == 32 && p.slots > 0 && entries >= 8ll * p.slots * 64;
+    reorder = !natural;
+    long long g = h->opt_row_groups > 0 ? h->opt_row_groups : (natural ? 16 : (nb > 1 ? 2 : 1));
+    if (p.scalar) g = 1;
+    if (g > kMaxRowGroups) g = kMaxRowGroups;
+    if (g > M) g = M;
+    p.n_groups = (int)g;
+    p.group_row.resize((size_t)p.n_groups + 1);
+    return spmm_b200_partition_rows(ptr.data(), M, p.n_groups, p.group_row.data());
+}
+
+// Host planning of every block, independent of each other: row order, segments, light-stream packing, task order. Block b
+// gathers from B rows [band_begin[b], band_begin[b + 1]) and owns CSR positions [split[b][r], split[b+1][r]) of row r.
+static int plan_blocks_host(spmm_b200_handle *h, const std::vector<int> &ptr, const std::vector<int> &split,
+                            const std::vector<int> &band_begin, int reorder, std::vector<BlockArrays> &arr) {
+    Plan &p = h->plan;
+    const int nb = p.n_col_blocks, M = h->num_v;
+    // (several blocks: one host thread per block; a single block: its row groups in parallel — nested regions stay serial)
+#pragma omp parallel for schedule(dynamic, 1) if (nb > 1)
+    for (int b = 0; b < nb; ++b) {
+        const int *rb = nb > 1 ? split.data() + (size_t)b * M : ptr.data();
+        const int *re = nb > 1 ? split.data() + (size_t)(b + 1) * M : ptr.data() + 1;
+        // passes after the first skip rows without nonzeros in their band — except the last pass, which lists every
+        // row: it is the one that delivers final rows (to C, to the stacked-layer targets, to run_host's host buffer)
+        const bool skip_empty = b > 0 && b + 1 != nb;
+        p.blocks[b].col_begin = band_begin[b];
+        p.blocks[b].col_end = band_begin[b + 1];
+        p.blocks[b].reorder = reorder;
+        if (p.scalar) plan_block_scalar(h, rb, re, skip_empty, reorder, p.blocks[b], arr[b]);
+        else plan_block_groups(h, rb, re, skip_empty, reorder, p.group_row.data(), p.n_groups, p.blocks[b], arr[b]);
+    }
+    for (const BlockArrays &a : arr)
+        if (a.rc) {
+            set_error("%s", a.err);
+            return a.rc;
+        }
+    if (h->opt_light_steps <= 0) p.light_steps = p.blocks[0].light_steps;   // reported by plan_info (block 0)
+    return 0;
+}
+
+// Device upload: one pool allocation per array kind that kernels write (lpanel, panel, part, seg_count), block after block,
+// then the arrays that kernels read, block by block (the host vectors must outlive the synchronisation of `stream`).
+static int upload_plan(Plan &p, int K, const std::vector<BlockArrays> &arr, cudaStream_t stream, PrepTrace &tr) {
+    long long lp_total = 0, pn_total = 0, seg_total = 0, heavy_total = 0, task_total = 0;
+    for (const BlockPlan &bp : p.blocks) {
+        lp_total += bp.lpanel_len;
+        pn_total += bp.panel_len;
+        seg_total += bp.n_seg;
+        heavy_total += bp.n_heavy;
+        task_total += bp.n_utask;
+    }
+    if (lp_total > 0x7fffffffll || pn_total > 0x7fffffffll || task_total * p.n_slices > 0x7fffffffll) {
+        set_error("plan too large for 32-bit panel offsets (%lld light, %lld heavy entries)", lp_total, pn_total);
+        return SPMM_B200_EINVAL;
+    }
+    if (lp_total) {
+        SB_CUDA(pool_alloc((void **)&p.d_lpanel_all, sizeof(int2) * (size_t)lp_total, stream));
+        SB_CUDA(cudaMemsetAsync(p.d_lpanel_all, 0xFF, sizeof(int2) * (size_t)lp_total, stream));   // nop entries
+    }
+    if (pn_total) SB_CUDA(pool_alloc((void **)&p.d_panel_all, sizeof(int2) * (size_t)pn_total, stream));
+    if (seg_total) SB_CUDA(pool_alloc((void **)&p.d_part_all, sizeof(float) * (size_t)seg_total * K, stream));
+    if (heavy_total) {
+        // n_heavy x n_slices counters per band
+        const size_t slots = (size_t)heavy_total * p.n_slices;
+        SB_CUDA(pool_alloc((void **)&p.d_seg_count_all, sizeof(int) * slots, stream));
+        SB_CUDA(cudaMemsetAsync(p.d_seg_count_all, 0, sizeof(int) * slots, stream));
+    }
+    tr.lap("arena allocation");
+    long long lp_off = 0, pn_off = 0, seg_off = 0, heavy_off = 0;
+    for (size_t b = 0; b < arr.size(); ++b) {
+        BlockPlan &bp = p.blocks[b];
+        int rc;
+        if ((rc = upload_vec(&bp.d_light_desc, arr[b].light, stream)) || (rc = upload_vec(&bp.d_utask, arr[b].utask, stream)) ||
+            (rc = upload_vec(&bp.d_seg_hrow, arr[b].seg_hrow, stream)) || (rc = upload_vec(&bp.d_heavy_seg0, arr[b].heavy_seg0, stream)) ||
+            (rc = upload_vec(&bp.d_seg_desc, arr[b].segs, stream)))
+            return rc;
+        bp.d_lpanel = p.d_lpanel_all + lp_off;   // a block's empty slices are never read
+        bp.d_panel = p.d_panel_all + pn_off;
+        bp.d_part = p.d_part_all + seg_off * K;
+        bp.d_seg_count = p.d_seg_count_all + heavy_off * p.n_slices;
+        lp_off += bp.lpanel_len;
+        pn_off += bp.panel_len;
+        seg_off += bp.n_seg;
+        heavy_off += bp.n_heavy;
+    }
     return 0;
 }
 
@@ -447,224 +630,26 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
         return 0;
     }
     SB_CUDA(cudaGetDevice(&p.device));   // the plan's arrays come from this device's pool (pool.cu)
-    p.block = (int)h->opt_block;
-    p.scalar = (K % 4) != 0;
-    p.kslice = h->opt_kslice > 0 ? (int)h->opt_kslice : auto_kslice(M, K);
-    if (p.scalar) p.kslice = K;
-    if (p.kslice > 256) p.kslice = 256;
-    if (p.kslice > ((K + 3) & ~3)) p.kslice = (K + 3) & ~3;
-    p.n_slices = (K + p.kslice - 1) / p.kslice;
-    if (!p.scalar) shape_for_kslice(p.kslice, &p.lanes, &p.vec);
-    p.seg_len = h->opt_seg_len > 0 ? (int)h->opt_seg_len : auto_seg_len(h->num_e, p.lanes);
-    p.tune = (int)h->opt_tune;
-    p.light_steps = h->opt_light_steps > 0 ? (int)h->opt_light_steps : 0;
-    p.slots = p.scalar ? 0 : resident_warps(p.lanes, p.vec, p.tune, p.block);
-    if (p.scalar) p.seg_len = 0x7fffffff;   // scalar fallback keeps every row whole
-    if (!p.scalar && (long long)b_rows * (K / 4) > 0x7fffffffll) {
-        set_error("B is too large for 32-bit row offsets: b_rows * feat_in / 4 = %lld >= 2^31", (long long)b_rows * (K / 4));
-        return SPMM_B200_EINVAL;
-    }
-    int nb = h->opt_col_blocks > 0 ? (int)h->opt_col_blocks : auto_col_blocks(b_rows, K, h->num_e, M);
-    if (p.scalar || nb < 1) nb = 1;
-    if (nb > kMaxBands && h->opt_col_blocks <= 0) nb = kMaxBands;
-    if (nb > b_rows) nb = b_rows > 0 ? b_rows : 1;
+    int nb = 1, rc;
+    if ((rc = plan_shape(h, b_rows, nb))) return rc;
+    std::vector<int> band_begin = band_bounds(b_rows, nb, h->opt_host_bands), ptr, split;
 
-    std::vector<int> ptr((size_t)M + 1, 0);
-    SB_CUDA(cudaMemcpyAsync(ptr.data(), h->d_ptr, sizeof(int) * ((size_t)M + 1), cudaMemcpyDeviceToHost, stream));
-    // columns must address rows of B: one pass over idx, queued behind the copy of ptr
-    int *d_flags = nullptr, flags[2] = {0, 0};   // [0] bad column, [1] unsorted row
-    SB_CUDA(cudaMalloc((void **)&d_flags, sizeof(flags)));
-    auto with_flags = [&](int rc) {
-        cudaFree(d_flags);
-        return rc;
-    };
-    if (cudaMemsetAsync(d_flags, 0, sizeof(flags), stream) != cudaSuccess) return with_flags(cuda_fail(cudaGetLastError(), "cudaMemsetAsync", __FILE__, __LINE__));
-    int rc = launch_check_cols(h->d_idx, h->num_e, b_rows, d_flags, stream);
-    if (rc) return with_flags(rc);
-    if (cudaStreamSynchronize(stream) != cudaSuccess) return with_flags(cuda_fail(cudaGetLastError(), "cudaStreamSynchronize", __FILE__, __LINE__));
-    if (ptr[0] != 0 || ptr[M] != h->num_e) {
-        set_error("CSR ptr is inconsistent: ptr[0]=%d ptr[num_v]=%d num_e=%d", ptr[0], ptr[M], h->num_e);
-        return with_flags(SPMM_B200_EINVAL);
-    }
-    for (int r = 0; r < M; ++r)   // whatever the row order: a negative degree would turn into out-of-bounds panel slots
-        if (ptr[r + 1] < ptr[r]) {
-            set_error("CSR ptr decreases at row %d", r);
-            return with_flags(SPMM_B200_EINVAL);
-        }
-    tr.lap("ptr D2H + check_cols");
-
-    // split every row at the column-block boundaries (needs ascending columns inside a row; a graph
-    // that is not sorted falls back to a single block)
-    std::vector<int> split;
-    // Band bounds. Default: nb equal bands of ceil(b_rows / nb) rows. Option "host_bands" (the plan is meant for the
-    // host-buffer call, spmm_b200_run_host): the LAST band takes the last 40 % of B's rows and the bands before it share
-    // the rest. The last pass stores final rows over PCIe and is bound by that transfer whatever it computes, so it may
-    // as well carry half of the nonzeros (from a band that no longer fits the L2), while the small early bands let the
-    // first pass start sooner and finish the rest of the work under the upload of B.
-    std::vector<int> band_begin;
-    if (nb > 1 && h->opt_host_bands && nb >= 3) {
-        // host_bands = 1: the last band is 40 % of B's rows (measured best on the reddit shape: e2e 10.31 -> 9.34 ms;
-        // 30 %: 9.76, 50 %: 9.60, 60 %: 9.98 — profiles/r02_host_bands.jsonl); 10..90: that percentage
-        const long long pct = h->opt_host_bands >= 10 ? h->opt_host_bands : 40;
-        const int small = nb - 1, half = (int)((long long)b_rows * (100 - pct) / 100);
-        const int per = (half + small - 1) / small;
-        for (int b = 0; b < small && b * per < half; ++b) band_begin.push_back(b * per);
-        band_begin.push_back(half);
-        band_begin.push_back(b_rows);
-        nb = (int)band_begin.size() - 1;
-    } else {
-        const int cols_per_block = nb > 1 ? (b_rows + nb - 1) / nb : b_rows;
-        if (nb > 1) nb = (b_rows + cols_per_block - 1) / cols_per_block;   // every band starts inside B (b_rows = 10, 7 bands -> 5 of 2 rows)
-        for (int b = 0; b < nb; ++b) band_begin.push_back(b * cols_per_block);
-        band_begin.push_back(b_rows);
-    }
-    if (nb > 1) {
-        if (pool_alloc((void **)&p.d_split, sizeof(int) * (size_t)(nb + 1) * M, stream) != cudaSuccess)
-            return with_flags(cuda_fail(cudaGetLastError(), "pool_alloc(split)", __FILE__, __LINE__));
-        rc = launch_split_rows(h->d_ptr, h->d_idx, M, nb, band_begin.data(), p.d_split, d_flags + 1, stream);
-        if (rc) return with_flags(rc);
-        split.resize((size_t)(nb + 1) * M);
-        cudaError_t e = cudaMemcpyAsync(split.data(), p.d_split, sizeof(int) * split.size(), cudaMemcpyDeviceToHost, stream);
-        if (e != cudaSuccess) return with_flags(cuda_fail(e, "cudaMemcpyAsync(split)", __FILE__, __LINE__));
-    }
-    {
-        cudaError_t e = cudaMemcpyAsync(flags, d_flags, sizeof(flags), cudaMemcpyDeviceToHost, stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
-        cudaFree(d_flags);
-        SB_CUDA(e);
-    }
-    if (flags[0]) {
-        set_error("CSR idx holds a column outside [0, %d)", b_rows);
-        return SPMM_B200_EINVAL;
-    }
-    if (nb > 1 && flags[1]) {
-        pool_free(p.d_split, stream);
-        p.d_split = nullptr;
-        split.clear();
-        nb = 1;
-    }
+    int *d_flags = nullptr;   // [0] a column outside B, [1] a row whose columns are not ascending
+    SB_CUDA(pool_alloc((void **)&d_flags, 2 * sizeof(int), stream));
+    if (!(rc = read_csr(h, b_rows, d_flags, ptr, stream, tr))) rc = split_at_bands(h, b_rows, d_flags, band_begin, split, stream);
+    pool_free(d_flags, stream);
+    if (rc) return rc;
     tr.lap("split_rows + D2H");
+
+    nb = (int)band_begin.size() - 1;
     p.n_col_blocks = nb;
     p.blocks.resize(nb);
-    auto row_begin = [&](int b) { return nb > 1 ? split.data() + (size_t)b * M : ptr.data(); };
-    auto row_end = [&](int b) { return nb > 1 ? split.data() + (size_t)(b + 1) * M : ptr.data() + 1; };
-
-    // Row order. Degree buckets (longest rows first) shorten the tail of every launch and keep the lanes of a task
-    // balanced; natural order keeps neighbouring rows together, which lets a graph's locality hit in L2. Natural order
-    // therefore only when locality is what is at stake: ONE block (no column blocks — B is either small or far larger than
-    // the L2) in a launch of at least 8 waves with a full warp per row: measured 12.2 -> 11.3 ms on the products shape and
-    // the opposite (0.14 -> 0.19 ms) on the one-wave arxiv shape (profiles/r01_sweep.md). With column blocks every pass
-    // gathers from an L2-resident band whatever the order, and buckets win at every partition size of the reddit shape
-    // (6.04 vs 6.14 ms whole, 0.80 vs 0.92 ms for a 1/8 block: profiles/r02_notes.md).
-    std::vector<int> reorder(nb);
-    bool all_natural = true;
-    for (int b = 0; b < nb; ++b) {
-        reorder[b] = h->opt_reorder >= 0 ? (int)h->opt_reorder : (nb > 1 ? 1 : block_reorder(h, row_begin(b), row_end(b)));
-        all_natural &= reorder[b] == 0;
-    }
-    // Row groups: contiguous row ranges balanced by nonzeros (the partition rule), planned independently (in parallel) and
-    // never spanned by a task. Natural order: 16. Degree buckets with several blocks: 2 — the halves that go out on two
-    // streams (below). Otherwise 1.
-    {
-        long long g = h->opt_row_groups > 0 ? h->opt_row_groups : (all_natural ? 16 : (nb > 1 ? 2 : 1));
-        if (p.scalar) g = 1;
-        if (g > kMaxRowGroups) g = kMaxRowGroups;
-        if (g > M) g = M;
-        p.n_groups = (int)g;
-    }
-    p.group_row.assign((size_t)p.n_groups + 1, M);
-    p.group_row[0] = 0;
-    for (int g = 1; g < p.n_groups; ++g) {
-        // first row r with ptr[r] >= g * nnz / n_groups — the partition rule (spmm_b200_partition_rows)
-        const long long target = (long long)h->num_e * g / p.n_groups;
-        p.group_row[g] = (int)(std::lower_bound(ptr.begin(), ptr.begin() + M, target, [](int a, long long t) { return (long long)a < t; }) - ptr.begin());
-    }
-
-    // ---- host planning of every block (independent of each other) -------------------------------------------------
-    std::vector<HostBlock> hb((size_t)nb);
-    // (several blocks: one host thread per block; a single block: its row groups in parallel — nested regions stay serial)
-#pragma omp parallel for schedule(dynamic, 1) if (nb > 1)
-    for (int b = 0; b < nb; ++b) {
-        // passes after the first skip rows without nonzeros in their band — except the last pass, which lists every
-        // row: it is the one that delivers final rows (to C, to the stacked-layer targets, to run_host's host buffer)
-        const bool skip_empty = b > 0 && b + 1 != nb;
-        plan_block_host(h, row_begin(b), row_end(b), skip_empty, reorder[b], p.group_row.data(), p.n_groups, hb[b]);
-    }
-    for (int b = 0; b < nb; ++b)
-        if (hb[b].rc) {
-            set_error("%s", hb[b].err);
-            return hb[b].rc;
-        }
+    std::vector<BlockArrays> arr((size_t)nb);
+    int reorder = 1;
+    if ((rc = order_rows(h, ptr, nb, reorder)) || (rc = plan_blocks_host(h, ptr, split, band_begin, reorder, arr))) return rc;
     tr.lap("host planning (all blocks)");
 
-    // ---- device side: one arena per array kind, band after band ------------------------------------------------------
-    long long lp_total = 0, pn_total = 0, seg_total = 0, heavy_total = 0, task_total = 0;
-    for (int b = 0; b < nb; ++b) {
-        lp_total += hb[b].lpanel_len;
-        pn_total += hb[b].panel_len;
-        seg_total += (long long)hb[b].segs.size();
-        heavy_total += (long long)hb[b].heavy_rows.size();
-        task_total += (long long)hb[b].utask.size();
-    }
-    if (lp_total > 0x7fffffffll || pn_total > 0x7fffffffll || task_total * p.n_slices > 0x7fffffffll) {
-        set_error("plan too large for 32-bit panel offsets (%lld light, %lld heavy entries)", lp_total, pn_total);
-        return SPMM_B200_EINVAL;
-    }
-    if (lp_total) {
-        SB_CUDA(pool_alloc((void **)&p.d_lpanel_all, sizeof(int2) * (size_t)lp_total, stream));
-        SB_CUDA(cudaMemsetAsync(p.d_lpanel_all, 0xFF, sizeof(int2) * (size_t)lp_total, stream));   // nop entries
-    }
-    if (pn_total) SB_CUDA(pool_alloc((void **)&p.d_panel_all, sizeof(int2) * (size_t)pn_total, stream));
-    if (seg_total) SB_CUDA(pool_alloc((void **)&p.d_part_all, sizeof(float) * (size_t)seg_total * K, stream));
-    if (heavy_total) {
-        // n_heavy x n_slices counters per band
-        const size_t slots = (size_t)heavy_total * p.n_slices;
-        SB_CUDA(pool_alloc((void **)&p.d_seg_count_all, sizeof(int) * slots, stream));
-        SB_CUDA(cudaMemsetAsync(p.d_seg_count_all, 0, sizeof(int) * slots, stream));
-    }
-    tr.lap("arena allocation");
-    const int groups = p.scalar ? 1 : 32 / p.lanes;
-    const int pad = p.scalar ? 2 : 4 * groups;
-    long long lp_off = 0, pn_off = 0, seg_off = 0, heavy_off = 0;
-    for (int b = 0; b < nb; ++b) {
-        BlockPlan &bp = p.blocks[b];
-        HostBlock &x = hb[b];
-        bp.col_begin = nb > 1 ? band_begin[b] : 0;
-        bp.col_end = nb > 1 ? band_begin[b + 1] : b_rows;
-        bp.reorder = x.reorder;
-        bp.light_steps = x.light_steps;
-        if (b == 0 && h->opt_light_steps <= 0) p.light_steps = x.light_steps;   // reported by plan_info (block 0)
-        bp.n_light = (int)x.row_perm.size();
-        bp.n_heavy = (int)x.heavy_rows.size();
-        bp.n_seg = (int)x.segs.size();
-        bp.panel_len = x.panel_len;
-        bp.lpanel_len = x.lpanel_len;
-        bp.n_ltask = (int)x.ltasks.size();
-        bp.n_utask = (int)x.utask.size();
-        bp.split_task = x.split_task;
-        if ((rc = upload_vec(&bp.d_row_perm, x.row_perm, stream))) return rc;
-        if ((rc = upload_vec(&bp.d_light_desc, x.light, stream))) return rc;
-        if ((rc = upload_vec(&bp.d_utask, x.utask, stream))) return rc;
-        if ((rc = upload_vec(&bp.d_ltask, x.ltasks, stream))) return rc;
-        if (bp.n_ltask > 0) {
-            bp.d_lpanel = p.d_lpanel_all + lp_off;
-            if ((rc = launch_build_lpanel(bp.d_light_desc, bp.n_light, groups, K / 4, h->d_idx, h->d_val, bp.d_lpanel, stream))) return rc;
-        }
-        if (bp.n_heavy > 0) {
-            if ((rc = upload_vec(&bp.d_seg_hrow, x.seg_hrow, stream))) return rc;
-            if ((rc = upload_vec(&bp.d_heavy_rows, x.heavy_rows, stream))) return rc;
-            if ((rc = upload_vec(&bp.d_heavy_seg0, x.heavy_seg0, stream))) return rc;
-            if ((rc = upload_vec(&bp.d_seg_desc, x.segs, stream))) return rc;
-            bp.d_seg_count = p.d_seg_count_all + heavy_off * p.n_slices;
-            bp.d_panel = p.d_panel_all + pn_off;
-            bp.d_part = p.d_part_all + seg_off * K;
-            if ((rc = launch_build_panel(bp.d_seg_desc, bp.n_seg, K / 4, pad, h->d_idx, h->d_val, bp.d_panel, stream))) return rc;
-        }
-        lp_off += x.lpanel_len;
-        pn_off += x.panel_len;
-        seg_off += (long long)x.segs.size();
-        heavy_off += (long long)x.heavy_rows.size();
-    }
+    if ((rc = upload_plan(p, K, arr, stream, tr)) || (rc = refresh_panels(h, stream))) return rc;
     tr.lap("uploads + panel kernels queued");
 
     // Two-stream launches (option "split_streams": -1 auto = whenever there are several blocks).
@@ -681,8 +666,8 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
     return 0;
 }
 
-// Re-stage the {col, val} panels from the caller's idx/val (asynchronous on `stream`): the plan's structure
-// (row order, segments, tasks, slots) depends on ptr only, so new edge values need no new plan.
+// Stage the {col, val} panels from the caller's idx/val (asynchronous on `stream`): at preprocess, and at refresh_values, as
+// the plan's structure (row order, segments, tasks, slots) depends on ptr only: new edge values need no new plan.
 int refresh_panels(spmm_b200_handle *h, cudaStream_t stream) {
     Plan &p = h->plan;
     if (p.scalar || h->feat == 0 || h->num_v == 0) return 0;   // the scalar kernel reads idx/val at run time

@@ -123,11 +123,11 @@ int spmm_b200_set_replicate(spmm_b200_t h, int world, int rank, float *const *pe
 }
 
 // B is cut into n_chunks equal row chunks by a rule every rank evaluates identically (b_rows and feat_in only: about
-// 48 MB each, the column-block band size, so chunks and bands coincide whenever a rank's plan uses column blocks);
+// kBandBytes each, the column-block band size, so chunks and bands coincide whenever a rank's plan uses column blocks);
 // rank g brings in the g-th of `world` equal pieces of every chunk.
 static int replicate_chunks(long long b_rows, int feat) {
-    const long long bytes = b_rows * feat * 4ll, band = 48ll << 20;
-    long long n = (bytes + band - 1) / band;
+    const long long bytes = b_rows * feat * 4ll;
+    long long n = (bytes + kBandBytes - 1) / kBandBytes;
     if (n < 1) n = 1;
     if (n > 16) n = 16;
     if (n > b_rows) n = b_rows > 0 ? b_rows : 1;
