@@ -10,4 +10,4 @@ from .graph import (  # noqa: F401
     write_graph,
 )
 from .mg import MultiGpuSpMM  # noqa: F401
-from .autograd import GraphSpMM  # noqa: F401
+from .autograd import GraphAttention, GraphSpMM  # noqa: F401

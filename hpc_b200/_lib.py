@@ -47,6 +47,8 @@ SIGNATURES = {
     "spmm_b200_run_profiled": (_I, [_P, _P, _P, _P, C.POINTER(C.c_float)]),
     "spmm_b200_create_transposed": (_I, [_P, _I, _P, C.POINTER(_P)]),
     "spmm_b200_sddmm": (_I, [_P, _P, _P, _P, _P]),
+    "spmm_b200_edge_softmax": (_I, [_P, _P, _P, _P]),
+    "spmm_b200_edge_softmax_backward": (_I, [_P, _P, _P, _P, _P]),
     "spmm_b200_create_column_sorted": (_I, [_P, _I, _P, C.POINTER(_P)]),
     "spmm_b200_destroy": (_I, [_P]),
     "spmm_b200_trim_memory": (_I, []),

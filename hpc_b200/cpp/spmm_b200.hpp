@@ -93,6 +93,15 @@ class SpMMB200 : public SpMM {
     // floats in CSR position order). With x_row = dC and x_col = B, out is the gradient of C = A*B for the edge values.
     void sddmm(const float *x_row, const float *x_col, float *out) { check(spmm_b200_sddmm(h_, x_row, x_col, out, stream_), "sddmm"); }
 
+    // softmax over each row's nonzeros (out: num_e floats in CSR position order, not overlapping scores), and its
+    // gradient ds = p * (dp - rowsum(p * dp)) with p the softmax output. Need no preprocess.
+    void edge_softmax(const float *scores, float *out) {
+        check(spmm_b200_edge_softmax(h_, scores, out, stream_), "edge_softmax");
+    }
+    void edge_softmax_backward(const float *p, const float *dp, float *ds) {
+        check(spmm_b200_edge_softmax_backward(h_, p, dp, ds, stream_), "edge_softmax_backward");
+    }
+
     // the same matrix with every row in ascending column order — for CSR inputs whose rows are not column-sorted (they
     // otherwise stay in one column block). Results associate in column order. Delete it before this operator.
     SpMMB200 *column_sorted(int feat = -1) const {

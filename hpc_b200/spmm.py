@@ -153,6 +153,24 @@ class SpMMB200(SpMM):
                 raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {n} elements")
         check(lib.spmm_b200_sddmm(self._h, _ptr(x_row), _ptr(x_col), _ptr(out), _stream()))
 
+    def _check_edges(self, **arrays):
+        for name, t in arrays.items():
+            if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < self.num_e:
+                raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {self.num_e} elements")
+
+    def edge_softmax(self, scores, out) -> None:
+        """Softmax over each row's nonzeros (spmm_b200_edge_softmax), in CSR position order: out[e] = exp(s[e] - m_r) /
+        sum_r exp(s - m_r). A row of -inf scores gives zeros. Needs no preprocess; out must not overlap scores.
+        Asynchronous on the current stream."""
+        self._check_edges(scores=scores, out=out)
+        check(lib.spmm_b200_edge_softmax(self._h, _ptr(scores), _ptr(out), _stream()))
+
+    def edge_softmax_backward(self, p, dp, ds) -> None:
+        """The gradient of edge_softmax (spmm_b200_edge_softmax_backward): ds[e] = p[e] * (dp[e] - sum_r p * dp), with p
+        its output. ds must not overlap p or dp. Asynchronous on the current stream."""
+        self._check_edges(p=p, dp=dp, ds=ds)
+        check(lib.spmm_b200_edge_softmax_backward(self._h, _ptr(p), _ptr(dp), _ptr(ds), _stream()))
+
     def run_profiled(self, vin, vout) -> float:
         """run + the kernel's device time in ms (synchronises)."""
         self._check_io(vin, vout)

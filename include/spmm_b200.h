@@ -131,6 +131,23 @@ int spmm_b200_create_transposed(spmm_b200_t h, int feat_in, void *stream, spmm_b
  * before capturing sddmm into a CUDA graph. */
 int spmm_b200_sddmm(spmm_b200_t h, const float *x_row, const float *x_col, float *out, void *stream);
 
+/* Row-wise softmax over the operator's pattern (no reference counterpart), in h's CSR position order: for every
+ * nonzero e of row r
+ *     out[e] = exp(s[e] - m_r) / sum_{e' in r} exp(s[e'] - m_r),   m_r = max_{e' in r} s[e']
+ * in the fixed order documented in hpc_b200/csrc/edge_softmax.cu: it depends on the row's length alone, not on any
+ * plan option. Special values follow torch.softmax (a -inf score gives 0; a NaN or +inf anywhere in a row makes the
+ * whole row NaN) except that a row whose scores are all -inf gives zeros (masking; torch gives NaN).
+ * Reads only h's ptr (a valid CSR: ptr[0] = 0, nondecreasing, ptr[num_v] = num_e): needs no preprocess, works on every
+ * handle (row block, transposed: normalising over a column of A, column-sorted). scores / out: num_e floats; out must
+ * not overlap scores. Asynchronous on `stream`, allocates nothing (capturable into a CUDA graph). num_e == 0: returns
+ * 0 without a CUDA call. A null handle, or null arrays with num_e > 0: SPMM_B200_EINVAL. */
+int spmm_b200_edge_softmax(spmm_b200_t h, const float *scores, float *out, void *stream);
+
+/* The gradient of spmm_b200_edge_softmax: with p its output and dp = dL/dp,
+ *     ds[e] = p[e] * (dp[e] - sum_{e' in r} p[e'] * dp[e'])
+ * in the same order. ds must not overlap p or dp. Same contract as spmm_b200_edge_softmax otherwise. */
+int spmm_b200_edge_softmax_backward(spmm_b200_t h, const float *p, const float *dp, float *ds, void *stream);
+
 /* The column-sorted operator (no reference counterpart): a new handle over the SAME matrix with every row stored in
  * ascending column order (stable: equal columns keep their storage order), built on the device. A CSR whose rows are
  * not column-sorted is otherwise kept in ONE column block — splitting an unsorted row at band boundaries would reorder
