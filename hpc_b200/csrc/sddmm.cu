@@ -16,7 +16,10 @@
 // 1 of every row, ...": the x_col band in flight stays in the L2, as in the forward passes, and since no output
 // depends on another band the one launch needs no waiting between bands. The prefix of that virtual order (an
 // exclusive scan of the (band, row) lengths from the plan's split array) is built on the device by the first call
-// after preprocess; with one block it is ptr itself.
+// after preprocess; with one block it is ptr itself, and so is it when blocks x rows + 1 exceeds INT_MAX (the walk is
+// then unbanded, with the same bits).
+#include <climits>
+
 #include <cub/device/device_scan.cuh>
 
 #include "common.h"
@@ -202,6 +205,12 @@ __global__ void __launch_bounds__(256) band_len_kernel(const int *split, int num
         len[i] = i < n_seg ? split[i + num_v] - split[i] : 0;
 }
 
+// Band-major walk: several column blocks and a (band, row) segment count whose prefix (n_seg + 1 entries) fits int. Past
+// that the walk is unbanded (vp = start = ptr): the order of each sum depends on K alone, so the bits are the same.
+bool walk_banded(const spmm_b200_handle *h) {
+    return h->plan.n_col_blocks > 1 && (long long)h->plan.n_col_blocks * h->num_v + 1 <= (long long)INT_MAX;
+}
+
 int pow2_lanes(int q) {
     int l = 1;
     while (l < q && l < 32) l <<= 1;
@@ -245,7 +254,7 @@ void *kernel_fn(int K) {
 int prepare(spmm_b200_handle *h, cudaStream_t stream) {
     Plan &p = h->plan;
     const int K = h->feat;
-    if (p.n_col_blocks > 1 && !p.d_sddmm_vp) {
+    if (walk_banded(h) && !p.d_sddmm_vp) {
         const long long n_seg = (long long)p.n_col_blocks * h->num_v;
         int *len = nullptr, *vp = nullptr;
         void *tmp = nullptr;
@@ -321,7 +330,7 @@ extern "C" int spmm_b200_sddmm(spmm_b200_t h, const float *x_row, const float *x
     if (rc) return rc;
     const Plan &p = h->plan;
     SddmmArgs a;
-    const bool banded = p.n_col_blocks > 1;
+    const bool banded = walk_banded(h);
     a.vp = banded ? p.d_sddmm_vp : h->d_ptr;
     a.start = banded ? p.d_split : h->d_ptr;
     a.idx = h->d_idx;
@@ -329,7 +338,7 @@ extern "C" int spmm_b200_sddmm(spmm_b200_t h, const float *x_row, const float *x
     a.x_col = x_col;
     a.out = out;
     a.num_v = h->num_v;
-    a.n_seg = (banded ? p.n_col_blocks : 1) * h->num_v;
+    a.n_seg = banded ? p.n_col_blocks * h->num_v : h->num_v;   // fits int: walk_banded checked the product
     a.nnz = h->num_e;
     a.feat = K;
     a.chunk = p.sddmm_chunk;

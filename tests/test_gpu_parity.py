@@ -159,6 +159,27 @@ def test_subnormal_inputs_flush_like_the_reference(golden_dir):
 
 # ---- engine vs oracle -----------------------------------------------------------------------------
 
+def _spmm_instance_cases():
+    """One case per reachable spmm_kernel<LANES, VEC, TUNE, FULL> (spmm_kernels.cu launch_lanes), chosen through kslice:
+    FULL (K a multiple of a whole lanes x vec x 4 slice) at K = 2 * kslice, and not FULL at a kslice that is not
+    lanes x vec x 4 and a K that leaves a partial last slice (LANES = 1 has no such kslice); each with tune 0 and 1 and
+    segments short enough to give heavy rows. -> (params, {(K, kslice): (lanes, vec, full)})"""
+    cases = [(2 * kslice, kslice, lanes, vec, True) for kslice, lanes, vec in
+             ((4, 1, 1), (8, 2, 1), (16, 4, 1), (32, 8, 1), (64, 16, 1), (128, 32, 1), (256, 32, 2))]
+    cases += [(K, kslice, lanes, vec, False) for kslice, K, lanes, vec in
+              ((8, 20, 2, 1), (12, 28, 4, 1), (24, 52, 8, 1), (48, 100, 16, 1), (96, 196, 32, 1), (192, 388, 32, 2))]
+    params, shapes = [], {}
+    for K, kslice, lanes, vec, full in cases:
+        for tune in (0, 1):
+            opts = {"kslice": kslice, "tune": tune, "seg_len": 32}
+            params.append(pytest.param("c0", K, opts, id=f"c0-K{K}-kslice{kslice}-tune{tune}"))
+            shapes[(K, tuple(sorted(opts.items())))] = (lanes, vec, full)
+    return params, shapes
+
+
+SPMM_INSTANCES, SPMM_INSTANCE_SHAPE = _spmm_instance_cases()
+
+
 @pytest.mark.parametrize("shape,K,opts", [
     ("c0", 32, {}), ("c0", 32, {"seg_len": 16}), ("c0", 32, {"reorder": 0}), ("c0", 256, {"seg_len": 64, "kslice": 64}),
     ("c0", 256, {"kslice": 128}), ("c0", 64, {}), ("c0", 128, {"block": 128}), ("c0", 512, {}), ("c0", 260, {}),
@@ -170,10 +191,16 @@ def test_subnormal_inputs_flush_like_the_reference(golden_dir):
     ("arxiv", 32, {"col_blocks": 2, "reorder": 0}), ("c0", 64, {"col_blocks": 64}),
     ("arxiv", 32, {"tune": 1}), ("arxiv", 256, {"tune": 1}), ("c0", 64, {"tune": 1, "seg_len": 32}), ("c0", 100, {"tune": 1}),
     ("arxiv", 256, {"reorder": 0}), ("arxiv", 32, {"reorder": 1}),
-])
+] + SPMM_INSTANCES)
 def test_engine_matches_oracle(shape, K, opts):
     ptr, idx = H.gen_named_graph(shape)
     op, g, vin, vout, got = run_engine(ptr, idx, K, **opts)
+    want = SPMM_INSTANCE_SHAPE.get((K, tuple(sorted(opts.items()))))
+    if want is not None:   # the kernel instantiation the case is there for is the one that ran
+        info = op.plan_info()
+        lanes, vec, kslice = info["lanes"], info["vec"], info["kslice"]
+        assert (lanes, vec, K % (lanes * vec * 4) == 0 and kslice == lanes * vec * 4) == want
+        assert info["n_heavy"] > 0
     check_against_oracle(ptr, idx, K, op, g, vin, got)
     op.close()
 

@@ -53,7 +53,7 @@ def _bits_equal(a, b):
 
 
 @pytest.mark.parametrize("shape", ["c0", "arxiv"])
-@pytest.mark.parametrize("K", [0, 4, 32, 33, 64, 256, 512])
+@pytest.mark.parametrize("K", [0, 4, 32, 33, 64, 256, 512, 8, 128, 1024])
 def test_matches_oracle(shape, K):
     ptr, idx = H.gen_named_graph(shape)
     got, want = _sddmm(ptr, idx, K)

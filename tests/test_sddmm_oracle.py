@@ -167,3 +167,46 @@ def test_cpp_adapter_sddmm_compiles(tmp_path):
     r = subprocess.run(["nvcc", "-std=c++14", "-w", "-c", "-o", str(tmp_path / "t.o"), "-I", os.path.join(ROOT, "include"),
                         "-I", os.path.join(ROOT, "hpc_b200", "cpp"), str(tu)], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
+
+
+# ---- dispatch coverage of the GPU tests ----------------------------------------------------------------------------
+
+def _pow2_lanes(q):
+    """pow2_lanes of sddmm.cu"""
+    lanes = 1
+    while lanes < q and lanes < 32:
+        lanes <<= 1
+    return lanes
+
+
+def _fast_shape(k):
+    """fast_shape of sddmm.cu: (lanes, float4 per lane) of sddmm_kernel for K % 4 == 0, K <= 512"""
+    q = k // 4
+    lanes = _pow2_lanes(q)
+    need = -(-q // lanes)
+    return lanes, 1 if need <= 1 else 2 if need <= 2 else 4
+
+
+def test_kernel_path_widths_reach_every_sddmm_dispatch_case():
+    """The widths of tests/test_kernel_paths_gpu.py launch every sddmm_kernel<LANES, VEC, U> in sddmm.cu's dispatch table
+    (read from the source, so a new case without a width fails here), each with all float4 slots of its lanes used and,
+    where the lane count leaves room (LANES >= 4), with some unused; sddmm_generic_kernel<true> (K > 512); and
+    sddmm_generic_kernel<false> at every lane count 1 .. 32."""
+    import re
+    import test_kernel_paths_gpu as KP
+    src = open(os.path.join(ROOT, "hpc_b200", "csrc", "sddmm.cu")).read()
+    table = {(int(l), int(v)) for l, v in re.findall(r"case \d+: return fast_fn<(\d+), (\d+), \d+>\(\);", src)}
+    assert len(table) == 8
+    full, partial = set(), set()
+    for k in KP.SDDMM_FAST_WIDTHS:
+        assert k % 4 == 0 and 0 < k <= 512
+        lanes, vec = _fast_shape(k)
+        (full if k // 4 == lanes * vec else partial).add((lanes, vec))
+    assert full == table
+    assert partial == {s for s in table if s[0] >= 4}
+    assert all(k % 4 == 0 and k > 512 for k in KP.SDDMM_GENERIC_V4_WIDTHS)
+    scalar = KP.SDDMM_GENERIC_SCALAR_WIDTHS
+    assert all(k % 4 != 0 for k in scalar)
+    assert {_pow2_lanes(k) for k in scalar} == {1, 2, 4, 8, 16, 32}
+    assert any(_pow2_lanes(k) == 32 and k > 32 for k in scalar)          # a lane walks more than one column
+    assert set(KP.SDDMM_WIDTHS) == set(KP.SDDMM_FAST_WIDTHS + KP.SDDMM_GENERIC_V4_WIDTHS + scalar)
