@@ -49,6 +49,8 @@ SIGNATURES = {
     "spmm_b200_sddmm": (_I, [_P, _P, _P, _P, _P]),
     "spmm_b200_edge_softmax": (_I, [_P, _P, _P, _P]),
     "spmm_b200_edge_softmax_backward": (_I, [_P, _P, _P, _P, _P]),
+    "spmm_b200_reduce": (_I, [_P, _I, _P, _P, _P, _P]),
+    "spmm_b200_reduce_backward": (_I, [_P, _P, _P, _P, _P, _P, _P]),
     "spmm_b200_create_column_sorted": (_I, [_P, _I, _P, C.POINTER(_P)]),
     "spmm_b200_destroy": (_I, [_P]),
     "spmm_b200_trim_memory": (_I, []),

@@ -1,7 +1,9 @@
 """Differentiable SpMM and graph attention as torch.autograd operations over the engine's kernels.
 
 GraphSpMM: forward is `run`; backward gives dB = Aᵀ·dC through the transposed operator and dval (the gradient for A's
-edge values) through `sddmm(dC, B)`, each only when it is needed.
+edge values) through `sddmm(dC, B)`, each only when it is needed. With reduce="amax" / "amin" the forward is `reduce`,
+which also records the winning nonzero of every output, and the backward is `reduce_backward` on the transposed
+operator; reduce="mean" divides the sum by the row's nonzero count.
 
 GraphAttention: scores = sddmm(q, k), alpha = edge_softmax(scores), out = A_alpha·v, with A_alpha the graph's pattern
 carrying alpha as edge values; every step differentiable.
@@ -39,28 +41,67 @@ class _GraphSpMMFn(torch.autograd.Function):
         return None, db, dval
 
 
+class _GraphSpMMReduceFn(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, mod, b, val):
+        # `val` is g.val itself: passing it makes autograd route dval to it
+        c = torch.empty((mod.g.num_v, mod.feat_in), dtype=torch.float32, device=b.device)
+        arg = torch.empty((mod.g.num_v, mod.feat_in), dtype=torch.int32, device=b.device)
+        mod.op.reduce(mod.reduce, b, c, arg)
+        ctx.mod = mod
+        ctx.save_for_backward(b, arg)
+        return c
+
+    @staticmethod
+    def backward(ctx, dc):
+        mod = ctx.mod
+        b, arg = ctx.saved_tensors
+        db = torch.empty_like(b) if ctx.needs_input_grad[1] else None
+        dval = torch.zeros_like(mod.g.val) if ctx.needs_input_grad[2] else None   # entries beyond num_e: zero
+        if db is not None or dval is not None:
+            mod.transposed().reduce_backward(dc.contiguous(), arg, db=db, dval=dval, vin=b if dval is not None else None)
+        return None, db, dval
+
+
+REDUCTIONS = ("sum", "mean", "amax", "amin")
+
+
 class GraphSpMM:
     """C = A·B for the CSR `g` (num_v x b_rows) and a dense B (b_rows x feat_in), differentiable in B and in g.val.
 
+    reduce (torch.sparse.mm's names): "sum" (default), "mean" (the sum over the row's nonzero count; empty rows give 0),
+    "amax" / "amin" (per column, the largest / smallest val[e] * B[idx[e]] of the row; NaN wins, ties go to the
+    smaller CSR position, empty rows give 0; the gradient goes to the winning nonzero alone).
+
     options are passed to the forward operator (SpMMB200), e.g. b_rows for a row block. g.val may require grad
     (learned edge weights); an in-place change of g.val (an optimizer step) is noticed through its version counter and
-    re-staged into the operators before the next forward. Call close() when done (or rely on garbage collection)."""
+    re-staged into the operators before the next forward ("amax" / "amin" read g.val as it is). Call close() when done
+    (or rely on garbage collection)."""
 
-    def __init__(self, g: CSR, feat_in: int, **options):
+    def __init__(self, g: CSR, feat_in: int, reduce: str = "sum", **options):
+        if reduce not in REDUCTIONS:
+            raise ValueError(f"reduce must be one of {REDUCTIONS}, got {reduce!r}")
         self.g = g
         self.feat_in = int(feat_in)
+        self.reduce = reduce
         self.op = SpMMB200(g, self.feat_in, **options)
         self._t = None
         self._staged = None
         self._prepared = False
+        self._deg = None
+
+    def _staged_values(self) -> bool:
+        """run reads the plan's copy of the values; reduce / reduce_backward read g.val itself."""
+        return self.reduce in ("sum", "mean")
 
     def transposed(self) -> SpMMB200:
-        """The operator over Aᵀ (created and planned on first use)."""
+        """The operator over Aᵀ (created on first use; planned when its run is needed)."""
         if self._t is None:
             self._t = self.op.transposed(self.feat_in)
-            dc = torch.empty((self.op.num_v, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
-            db = torch.empty((self.op.b_rows, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
-            self._t.preprocess(dc, db)
+            if self._staged_values():
+                dc = torch.empty((self.op.num_v, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
+                db = torch.empty((self.op.b_rows, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
+                self._t.preprocess(dc, db)
         return self._t
 
     def _stage(self, b: torch.Tensor) -> None:
@@ -69,18 +110,28 @@ class GraphSpMM:
             c = torch.empty((self.g.num_v, self.feat_in), dtype=torch.float32, device=b.device)
             self.op.preprocess(b, c)
             self._prepared = True
-        elif version != self._staged:
+        elif version != self._staged and self._staged_values():
             self.op.refresh_values()
             if self._t is not None:
                 self._t.refresh_values()
         self._staged = version
+
+    def _degrees(self) -> torch.Tensor:
+        """Nonzeros per row as a (num_v, 1) float32 column, empty rows counted as 1 (their sum is 0)."""
+        if self._deg is None:
+            ptr = self.g.ptr[: self.g.num_v + 1]
+            self._deg = (ptr[1:] - ptr[:-1]).clamp(min=1).to(torch.float32).unsqueeze(1)
+        return self._deg
 
     def __call__(self, b: torch.Tensor) -> torch.Tensor:
         if b.dtype != torch.float32 or not b.is_cuda or b.shape != (self.op.b_rows, self.feat_in):
             raise ValueError(f"B: need a CUDA float32 tensor of shape ({self.op.b_rows}, {self.feat_in})")
         b = b.contiguous()
         self._stage(b)
-        return _GraphSpMMFn.apply(self, b, self.g.val)
+        if self.reduce in ("amax", "amin"):
+            return _GraphSpMMReduceFn.apply(self, b, self.g.val)
+        c = _GraphSpMMFn.apply(self, b, self.g.val)
+        return c / self._degrees() if self.reduce == "mean" else c
 
     def close(self) -> None:
         """Releases the transposed operator, then the forward one."""

@@ -102,6 +102,15 @@ class SpMMB200 : public SpMM {
         check(spmm_b200_edge_softmax_backward(h_, p, dp, ds, stream_), "edge_softmax_backward");
     }
 
+    // amax / amin over each row's messages val[e] * vin[idx[e], j] (op: SPMM_B200_REDUCE_AMAX / _AMIN): vout and arg
+    // (the winner's CSR position, may be NULL) are num_v x feat_in. Reads the current edge values; needs preprocess.
+    void reduce(int op, const float *vin, float *vout, int *arg) { check(spmm_b200_reduce(h_, op, vin, vout, arg, stream_), "reduce"); }
+    // on the operator transposed() returned: the gradients of the source's reduce for B (db) and for the edge values
+    // (dval), each optional; vin (the forward's B) is needed only with dval
+    void reduce_backward(const float *dc, const int *arg, const float *vin, float *db, float *dval) {
+        check(spmm_b200_reduce_backward(h_, dc, arg, vin, db, dval, stream_), "reduce_backward");
+    }
+
     // the same matrix with every row in ascending column order — for CSR inputs whose rows are not column-sorted (they
     // otherwise stay in one column block). Results associate in column order. Delete it before this operator.
     SpMMB200 *column_sorted(int feat = -1) const {

@@ -171,6 +171,43 @@ class SpMMB200(SpMM):
         self._check_edges(p=p, dp=dp, ds=ds)
         check(lib.spmm_b200_edge_softmax_backward(self._h, _ptr(p), _ptr(dp), _ptr(ds), _stream()))
 
+    REDUCE_OPS = {"amax": 1, "amin": 2}   # SPMM_B200_REDUCE_AMAX / _AMIN
+
+    @staticmethod
+    def _check_dense(name, t, n, dtype=torch.float32):
+        if not t.is_cuda or t.dtype != dtype or not t.is_contiguous() or t.numel() < n:
+            raise ValueError(f"{name}: need a contiguous CUDA {dtype} tensor of >= {n} elements")
+
+    def reduce(self, op: str, vin, vout, arg=None) -> None:
+        """amax / amin aggregation over this operator's rows (spmm_b200_reduce): vout[r, j] = the winning message
+        val[e] * vin[idx[e], j] over the nonzeros e of row r, arg[r, j] = e (int32, optional). NaN wins; ties go to the
+        smaller CSR position; an empty row gives 0 and arg -1. vin: b_rows x feat_in, vout / arg: num_v x feat_in.
+        Reads the current g.val (no refresh_values needed). Asynchronous on the current stream."""
+        if op not in self.REDUCE_OPS:
+            raise ValueError(f"reduce: op must be one of {sorted(self.REDUCE_OPS)}, got {op!r}")
+        self._check_dense("vin", vin, self.b_rows * self.feat_in)
+        self._check_dense("vout", vout, self.num_v * self.feat_in)
+        if arg is not None:
+            self._check_dense("arg", arg, self.num_v * self.feat_in, torch.int32)
+        check(lib.spmm_b200_reduce(self._h, self.REDUCE_OPS[op], _ptr(vin), _ptr(vout), _ptr(arg), _stream()))
+
+    def reduce_backward(self, dc, arg, db=None, dval=None, vin=None) -> None:
+        """The gradient of the source operator's reduce, on this operator, which must come from transposed()
+        (spmm_b200_reduce_backward): db (the source's b_rows x feat_in) and dval (num_e, in the source's CSR positions),
+        each optional, from dC and the forward's arg (both the source's num_v x feat_in). vin (the forward's B) is
+        needed only with dval. Asynchronous on the current stream."""
+        src_rows = self.b_rows   # this operator is Aᵀ: its b_rows are the source's rows
+        self._check_dense("dc", dc, src_rows * self.feat_in)
+        self._check_dense("arg", arg, src_rows * self.feat_in, torch.int32)
+        if db is not None:
+            self._check_dense("db", db, self.num_v * self.feat_in)
+        if dval is not None:
+            self._check_dense("dval", dval, self.num_e)
+            if vin is None:
+                raise ValueError("reduce_backward: dval needs vin (the forward's B)")
+            self._check_dense("vin", vin, self.num_v * self.feat_in)
+        check(lib.spmm_b200_reduce_backward(self._h, _ptr(dc), _ptr(arg), _ptr(vin), _ptr(db), _ptr(dval), _stream()))
+
     def run_profiled(self, vin, vout) -> float:
         """run + the kernel's device time in ms (synchronises)."""
         self._check_io(vin, vout)

@@ -148,6 +148,38 @@ int spmm_b200_edge_softmax(spmm_b200_t h, const float *scores, float *out, void 
  * in the same order. ds must not overlap p or dp. Same contract as spmm_b200_edge_softmax otherwise. */
 int spmm_b200_edge_softmax_backward(spmm_b200_t h, const float *p, const float *dp, float *ds, void *stream);
 
+/* amax / amin aggregation over the operator's rows (no reference counterpart; torch.sparse.mm(A, B, "amax" | "amin")).
+ * For every row r, column j < feat_in and nonzero e of r the message is m(e, j) = val[e] * vin[idx[e] * feat_in + j]
+ * (one rounded multiply, subnormals flushed to zero); vout[r * feat_in + j] is the message of the winning nonzero and
+ * arg[r * feat_in + j] its CSR position (arg may be NULL). The winner is the maximum of a total order on (message,
+ * position): a NaN ranks above every number (for amax and amin alike, so NaN propagates as in torch.amax); among
+ * numbers the larger (AMAX) or smaller (AMIN) value wins; equal values, -0 == +0 included, go to the smaller CSR
+ * position. The bits therefore depend on no plan option. An empty row gives +0.0f and arg = -1.
+ * vin: b_rows x feat_in, vout / arg: num_v x feat_in, fully overwritten (also when num_e == 0); 16-byte aligned when
+ * feat_in % 4 == 0. feat_in == 0: returns 0 without a CUDA call. Reads the caller's CURRENT d_ptr / d_idx / d_val, not
+ * the plan's staged copy: no spmm_b200_refresh_values is needed after the values change. Needs preprocess (it validates
+ * the columns against b_rows; SPMM_B200_ESTATE otherwise); set_feat, the b_rows option and a new preprocess invalidate
+ * it as they invalidate run. Works on every handle (row block, transposed, column-sorted); outputs follow THAT handle's
+ * CSR positions. With several column blocks it makes one pass per band of B, as run does. Asynchronous on `stream`, no
+ * atomics, allocates nothing (capturable into a CUDA graph). The stacked-layer epilogue (set_gather), run_host and
+ * set_replicate do not apply. A null handle, a bad op, or null arrays with work to do: SPMM_B200_EINVAL. */
+#define SPMM_B200_REDUCE_AMAX 1
+#define SPMM_B200_REDUCE_AMIN 2
+int spmm_b200_reduce(spmm_b200_t h, int op, const float *vin, float *vout, int *arg, void *stream);
+
+/* The gradient of spmm_b200_reduce, on t = spmm_b200_create_transposed(h, feat_in, ...) (any other handle, a
+ * column-sorted one included, gives SPMM_B200_EINVAL; t needs no preprocess). dc: num_v x feat_in of h (dL/dvout), arg:
+ * the forward's arg (required). With A^T row c holding entries k in storage order, e = perm[k] and r = the row of A of
+ * entry k, entry k matches column j when arg[r * feat_in + j] == e:
+ *     db[c, j] = sum over matching entries of val[e] * dc[r * feat_in + j]      (b_rows x feat_in; +0.0f if none)
+ *     dval[e]  = sum over matching columns j of dc[r * feat_in + j] * vin[c * feat_in + j]      (num_e, h's positions)
+ * in the fixed orders documented in hpc_b200/csrc/reduce.cu (db: tiles of 1024 entries; dval: sddmm's order with the
+ * non-matching terms skipped), so the bits do not depend on any option. val is h's CURRENT d_val. db and dval are each
+ * optional (NULL); vin (the forward's B) is needed only with dval. Arrays 16-byte aligned when feat_in % 4 == 0.
+ * Asynchronous on `stream`, no atomics, allocates nothing (capturable into a CUDA graph). */
+int spmm_b200_reduce_backward(spmm_b200_t t, const float *dc, const int *arg, const float *vin, float *db, float *dval,
+                              void *stream);
+
 /* The column-sorted operator (no reference counterpart): a new handle over the SAME matrix with every row stored in
  * ascending column order (stable: equal columns keep their storage order), built on the device. A CSR whose rows are
  * not column-sorted is otherwise kept in ONE column block — splitting an unsorted row at band boundaries would reorder
