@@ -204,14 +204,46 @@ int launch_xrank_barrier(unsigned int *const *flags, int world, int rank, int ph
 // lanes with about `steps` entries each; dst[i] = lpanel slot of row i's header. Returns the lpanel length.
 long long pack_light_host(const int *cost, int n, int groups, int steps, int *dst, std::vector<int2> &tasks);
 
+// The current device's SM count, or the error of the failed query.
+inline cudaError_t query_sm_count(int *sms) {
+    int dev = 0;
+    const cudaError_t e = cudaGetDevice(&dev);
+    return e != cudaSuccess ? e : cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev);
+}
+
+// The current device's SM count, or 0 when it cannot be queried (the error is cleared).
+inline int sm_count() {
+    int sms = 0;
+    if (query_sm_count(&sms) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    return sms;
+}
+
+// Lanes per row slice of q units (float4 or columns): the power of two >= q, at most 32. This is the L of sddmm's
+// summation order (sddmm.cu), which reduce_backward's dval (reduce.cu) must follow bit for bit.
+inline int pow2_lanes(int q) {
+    int l = 1;
+    while (l < q && l < 32) l <<= 1;
+    return l;
+}
+
+// The one-slice lane shape of K % 4 == 0, K <= 512 (sddmm_kernel, reduce.cu's float4 kernels): L lanes of vec float4.
+struct LaneShape {
+    int lanes, vec;   // vec: 1, 2 or 4
+};
+inline LaneShape fast_lane_shape(int K) {
+    const int q = K / 4, l = pow2_lanes(q), need = (q + l - 1) / l;
+    return {l, need <= 1 ? 1 : need <= 2 ? 2 : 4};
+}
+
 // lanes/vec choice for a slice width (shared by plan + launch)
 inline void shape_for_kslice(int kslice, int *lanes, int *vec) {
     // kslice is a multiple of 4; lanes*vec*4 >= kslice, lanes a power of two <= 32
-    int q = (kslice + 3) / 4;   // float4 per row slice
-    int l = 1;
-    while (l < q && l < 32) l <<= 1;
-    *lanes = l;
-    *vec = (q + l - 1) / l;     // 1 for kslice <= 128, 2 for 256
+    const int q = (kslice + 3) / 4;   // float4 per row slice
+    *lanes = pow2_lanes(q);
+    *vec = (q + *lanes - 1) / *lanes;   // 1 for kslice <= 128, 2 for 256
 }
 
 }  // namespace spmm_b200

@@ -25,15 +25,14 @@
 // exp(0) = exp(-0) = 1 exactly (single-edge rows give 1), -inf and every result below FLT_MIN give +0, and every float
 // in [-87.5, 0] is within 2 ulp of the fp64 exp (checked exhaustively by tests/test_edge_softmax_oracle.py).
 //
-// Work split (rows run from 0 to 154 828 nonzeros on the shapes of hpc_b200/shapes.py). Rows of at most 1024
-// nonzeros: one warp each, scores kept in registers (HBM reads every input once); warps take contiguous row ranges
-// of equal rows + nonzeros, found by a binary search over ptr[r] + r. Longer rows: one CTA each (8 warps take the
-// tiles round-robin, tile sums are folded in tile order through shared memory), found by a second launch whose CTAs
-// scan row stripes; the passes after the first re-read the row from the L2. No atomics, no workspace, no allocation.
+// Work split (rows run from 0 to 154 828 nonzeros on the shapes of hpc_b200/shapes.py), as rows.cuh describes. Rows of
+// at most 1024 nonzeros: one warp each, scores kept in registers (HBM reads every input once). Longer rows: one CTA
+// each (8 warps take the tiles round-robin, tile sums are folded in tile order through shared memory); the passes
+// after the first re-read the row from the L2. No atomics, no workspace, no allocation.
 #include <cfloat>
 #include <cstdint>
 
-#include "common.h"
+#include "rows.cuh"
 
 namespace spmm_b200 {
 
@@ -44,11 +43,7 @@ constexpr int kTile = 256;                   // T of the order above
 constexpr int kPer = kTile / 32;             // positions per lane per tile
 constexpr int kRegTiles = 4;                 // a warp keeps rows of up to kRegTiles tiles in registers
 constexpr int kWarpMax = kRegTiles * kTile;  // longer rows go to the CTA path
-constexpr int kBlock = 256;
-constexpr int kWarps = kBlock / 32;
 constexpr int kRound = 64;                   // tile sums folded per round in the CTA path
-constexpr int kWarpWaves = 4;                // row ranges per resident warp (32 per SM assumed): a short tail
-constexpr long long kMinChunk = 256;         // rows + nonzeros per warp at least
 
 struct SoftmaxArgs {
     const int *ptr;
@@ -86,24 +81,12 @@ __device__ __forceinline__ float warp_sum(float c) {
 
 __device__ __forceinline__ bool is_bad(float x) { return x != x || x == INFINITY; }
 
-// first row r in [0, num_v] with ptr[r] + r >= d
-__device__ int first_row(const int *ptr, int num_v, long long d) {
-    int lo = 0, hi = num_v;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if ((long long)__ldg(ptr + mid) + mid >= d) hi = mid;
-        else lo = mid + 1;
-    }
-    return lo;
-}
-
 // Rows of 1 .. kWarpMax nonzeros, one warp each, in contiguous ranges of about `chunk` rows + nonzeros per warp.
 template <bool BWD>
-__global__ void __launch_bounds__(kBlock) softmax_warp_kernel(const __grid_constant__ SoftmaxArgs a) {
+__global__ void __launch_bounds__(kRowBlock) softmax_warp_kernel(const __grid_constant__ SoftmaxArgs a) {
     const int lane = threadIdx.x & 31;
-    const long long w = (long long)blockIdx.x * kWarps + (threadIdx.x >> 5);
-    const int r0 = first_row(a.ptr, a.num_v, w * a.chunk);
-    const int r1 = first_row(a.ptr, a.num_v, (w + 1) * a.chunk);
+    int r0, r1;
+    warp_rows(a, r0, r1);
     int beg = r0 < r1 ? __ldg(a.ptr + r0) : 0;
     for (int r = r0; r < r1; ++r) {
         const int end = __ldg(a.ptr + r + 1);
@@ -190,120 +173,101 @@ __global__ void __launch_bounds__(kBlock) softmax_warp_kernel(const __grid_const
     }
 }
 
-// Rows of more than kWarpMax nonzeros, one CTA each. CTA b scans row stripes b, b + gridDim.x, ... of kBlock rows
-// and takes the long rows of a stripe in row order.
+// Rows of more than kWarpMax nonzeros, one CTA each (the long-row launch of rows.cuh).
 template <bool BWD>
-__global__ void __launch_bounds__(kBlock) softmax_long_kernel(const __grid_constant__ SoftmaxArgs a) {
-    __shared__ unsigned long_mask[kWarps];
-    __shared__ float red_m[kWarps];
-    __shared__ int red_bad[kWarps];
+__global__ void __launch_bounds__(kRowBlock) softmax_long_kernel(const __grid_constant__ SoftmaxArgs a) {
+    __shared__ unsigned long_mask[kRowWarps];
+    __shared__ float red_m[kRowWarps];
+    __shared__ int red_bad[kRowWarps];
     __shared__ float tsum[kRound];
     __shared__ float total;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    for (long long r0 = (long long)blockIdx.x * kBlock; r0 < a.num_v; r0 += (long long)gridDim.x * kBlock) {
-        const long long rr = r0 + threadIdx.x;
-        const bool is_long = rr < a.num_v && __ldg(a.ptr + rr + 1) - __ldg(a.ptr + rr) > kWarpMax;
-        const unsigned bm = __ballot_sync(kFull, is_long);
-        if (lane == 0) long_mask[warp] = bm;
-        __syncthreads();
-        for (int sw = 0; sw < kWarps; ++sw) {
-            for (unsigned rest = long_mask[sw]; rest; rest &= rest - 1) {
-                const int r = (int)r0 + sw * 32 + __ffs(rest) - 1;
-                const int beg = __ldg(a.ptr + r), n = __ldg(a.ptr + r + 1) - beg;
-                const float *x = a.a + beg;
-                const float *dp = BWD ? a.b + beg : nullptr;
-                float *out = a.out + beg;
-                // pass 1 (forward): max and the NaN / +inf flag
-                float m = 0.0f;
-                if (!BWD) {
-                    m = -INFINITY;
-                    int bad = 0;
-                    for (int i = threadIdx.x; i < n; i += kBlock) {
-                        const float s = x[i];
-                        m = fmaxf(m, s);
-                        bad |= is_bad(s);
-                    }
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for_long_rows(a, kWarpMax, long_mask, [&](int r) {
+        const int beg = __ldg(a.ptr + r), n = __ldg(a.ptr + r + 1) - beg;
+        const float *x = a.a + beg;
+        const float *dp = BWD ? a.b + beg : nullptr;
+        float *out = a.out + beg;
+        // pass 1 (forward): max and the NaN / +inf flag
+        float m = 0.0f;
+        if (!BWD) {
+            m = -INFINITY;
+            int bad = 0;
+            for (int i = tid; i < n; i += kRowBlock) {
+                const float s = x[i];
+                m = fmaxf(m, s);
+                bad |= is_bad(s);
+            }
 #pragma unroll
-                    for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(kFull, m, o));
-                    bad = __any_sync(kFull, bad);
-                    if (lane == 0) {
-                        red_m[warp] = m;
-                        red_bad[warp] = bad;
-                    }
-                    __syncthreads();
-                    for (int k = 0; k < kWarps; ++k) {
-                        m = fmaxf(m, red_m[k]);
-                        bad |= red_bad[k];
-                    }
-                    __syncthreads();
-                    if (bad || m == -INFINITY) {
-                        const float fill = bad ? __int_as_float(0x7fffffff) : 0.0f;
-                        for (int i = threadIdx.x; i < n; i += kBlock) out[i] = fill;
-                        continue;
-                    }
-                }
-                // pass 2: tile sums in tile order
-                const int nt = (n + kTile - 1) / kTile;
-                float S = 0.0f;
-                for (int t0 = 0; t0 < nt; t0 += kRound) {
-                    const int t1 = min(nt, t0 + kRound);
-                    for (int t = t0 + warp; t < t1; t += kWarps) {
-                        float xa[kPer], xb[kPer];
-#pragma unroll
-                        for (int j = 0; j < kPer; ++j) {
-                            const int i = t * kTile + j * 32 + lane;
-                            xa[j] = i < n ? x[i] : 0.0f;
-                            if (BWD) xb[j] = i < n ? dp[i] : 0.0f;
-                        }
-                        float c = 0.0f;
-#pragma unroll
-                        for (int j = 0; j < kPer; ++j) {
-                            if (t * kTile + j * 32 + lane < n)
-                                c = BWD ? fmaf(xa[j], xb[j], c) : __fadd_rn(c, sm_exp(__fsub_rn(xa[j], m)));
-                        }
-                        c = warp_sum(c);
-                        if (lane == 0) tsum[t - t0] = c;
-                    }
-                    __syncthreads();
-                    if (threadIdx.x == 0)
-                        for (int t = t0; t < t1; ++t) S = __fadd_rn(S, tsum[t - t0]);
-                    __syncthreads();
-                }
-                if (threadIdx.x == 0) total = S;
-                __syncthreads();
-                S = total;
-                // pass 3: outputs
-                for (int i = threadIdx.x; i < n; i += kBlock)
-                    out[i] = BWD ? __fmul_rn(x[i], __fsub_rn(dp[i], S)) : __fdiv_rn(sm_exp(__fsub_rn(x[i], m)), S);
-                __syncthreads();   // `total` is rewritten by the next row
+            for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(kFull, m, o));
+            bad = __any_sync(kFull, bad);
+            if (lane == 0) {
+                red_m[warp] = m;
+                red_bad[warp] = bad;
+            }
+            __syncthreads();
+            for (int k = 0; k < kRowWarps; ++k) {
+                m = fmaxf(m, red_m[k]);
+                bad |= red_bad[k];
+            }
+            __syncthreads();
+            if (bad || m == -INFINITY) {
+                const float fill = bad ? __int_as_float(0x7fffffff) : 0.0f;
+                for (int i = tid; i < n; i += kRowBlock) out[i] = fill;
+                return;
             }
         }
-        __syncthreads();   // long_mask is rewritten by the next stripe
-    }
+        // pass 2: tile sums in tile order
+        const int nt = (n + kTile - 1) / kTile;
+        float S = 0.0f;
+        for (int t0 = 0; t0 < nt; t0 += kRound) {
+            const int t1 = min(nt, t0 + kRound);
+            for (int t = t0 + warp; t < t1; t += kRowWarps) {
+                float xa[kPer], xb[kPer];
+#pragma unroll
+                for (int j = 0; j < kPer; ++j) {
+                    const int i = t * kTile + j * 32 + lane;
+                    xa[j] = i < n ? x[i] : 0.0f;
+                    if (BWD) xb[j] = i < n ? dp[i] : 0.0f;
+                }
+                float c = 0.0f;
+#pragma unroll
+                for (int j = 0; j < kPer; ++j) {
+                    if (t * kTile + j * 32 + lane < n)
+                        c = BWD ? fmaf(xa[j], xb[j], c) : __fadd_rn(c, sm_exp(__fsub_rn(xa[j], m)));
+                }
+                c = warp_sum(c);
+                if (lane == 0) tsum[t - t0] = c;
+            }
+            __syncthreads();
+            if (tid == 0)
+                for (int t = t0; t < t1; ++t) S = __fadd_rn(S, tsum[t - t0]);
+            __syncthreads();
+        }
+        if (tid == 0) total = S;
+        __syncthreads();
+        S = total;
+        // pass 3: outputs
+        for (int i = tid; i < n; i += kRowBlock)
+            out[i] = BWD ? __fmul_rn(x[i], __fsub_rn(dp[i], S)) : __fdiv_rn(sm_exp(__fsub_rn(x[i], m)), S);
+        __syncthreads();   // `total` is rewritten by the next row
+    });
 }
 
 template <bool BWD>
 int launch(spmm_b200_t h, const float *x, const float *y, float *out, cudaStream_t s) {
-    int dev = 0, sms = 0;
-    SB_CUDA(cudaGetDevice(&dev));
-    SB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (sms <= 0) sms = 1;
+    RowGrid gr;
+    const int rc = row_grid(h->num_v, h->num_e, &gr);
+    if (rc) return rc;
     SoftmaxArgs a;
     a.ptr = h->d_ptr;
     a.a = x;
     a.b = y;
     a.out = out;
     a.num_v = h->num_v;
-    const long long d = (long long)h->num_e + h->num_v;
-    const long long target = (long long)sms * 32 * kWarpWaves;
-    a.chunk = (d + target - 1) / target;
-    if (a.chunk < kMinChunk) a.chunk = kMinChunk;
-    const long long warps = (d + a.chunk - 1) / a.chunk;
-    softmax_warp_kernel<BWD><<<(unsigned)((warps + kWarps - 1) / kWarps), kBlock, 0, s>>>(a);
+    a.chunk = gr.chunk;
+    softmax_warp_kernel<BWD><<<gr.warp_blocks, kRowBlock, 0, s>>>(a);
     SB_CUDA(cudaGetLastError());
-    const long long stripes = ((long long)h->num_v + kBlock - 1) / kBlock;
-    const long long grid = stripes < (long long)sms * 4 ? stripes : (long long)sms * 4;
-    softmax_long_kernel<BWD><<<(unsigned)grid, kBlock, 0, s>>>(a);
+    softmax_long_kernel<BWD><<<gr.long_blocks, kRowBlock, 0, s>>>(a);
     SB_CUDA(cudaGetLastError());
     return 0;
 }

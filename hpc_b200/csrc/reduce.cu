@@ -25,29 +25,26 @@
 //
 // Work split (forward and backward alike): lane groups of L lanes cover one slice of the columns (L lanes x VEC units
 // of W = 4 or 1 columns, the lane shape of sddmm); K % 4 == 0 and K <= 512 is one slice, wider or scalar K loops over
-// slices. Warps take contiguous row ranges of equal rows + nonzeros (binary search over ptr[r] + r). Forward: the 32 / L
-// groups of a warp take interleaved nonzeros of one row, keep a running (value, position) per column in registers and
-// fold with shuffles. Backward: the groups take different rows of Aᵀ, since each tile is one in-order chain. Rows longer
-// than a threshold go to a second launch, one CTA per row: forward warps interleave nonzeros and fold through shared
-// memory; backward lane groups take whole tiles round-robin and the tile sums are added in tile order through shared
-// memory. Built -ftz=true. No atomics, no workspace, no allocation.
+// slices. dval's bits rely on L being sddmm's: both take it from pow2_lanes / fast_lane_shape (common.h). Rows are split
+// as rows.cuh describes, at kWarpMax (forward) and kBwdWarpMax (backward) nonzeros. Forward: the 32 / L groups of a warp
+// take interleaved nonzeros of one row, keep a running (value, position) per column in registers and fold with
+// shuffles. Backward: the groups take different rows of Aᵀ, since each tile is one in-order chain. Long rows, one CTA
+// each: forward warps interleave nonzeros and fold through shared memory; backward lane groups take whole tiles
+// round-robin and the tile sums are added in tile order through shared memory. Built -ftz=true. No atomics, no
+// workspace, no allocation.
 #include <cstdint>
 
-#include "common.h"
+#include "rows.cuh"
 
 namespace spmm_b200 {
 
 namespace {
 
 constexpr unsigned kFull = 0xffffffffu;
-constexpr int kBlock = 256;
-constexpr int kWarps = kBlock / 32;
 constexpr int kWarpMax = 2048;          // forward: rows with more nonzeros go to the CTA path
 constexpr int kTile = 1024;             // T of the backward order (tests/reduce_oracle.c: REDUCE_TILE)
 constexpr int kBwdWarpMax = 4 * kTile;  // backward: longer Aᵀ rows go to the CTA path
 constexpr int kMaxSlice = 512;          // columns per slice at most (32 lanes x 4 float4)
-constexpr int kWarpWaves = 4;           // row ranges per resident warp (32 per SM assumed): a short tail
-constexpr long long kMinChunk = 256;    // rows + nonzeros per warp at least
 
 struct ReduceArgs {
     const int *ptr, *idx;
@@ -115,17 +112,6 @@ __device__ __forceinline__ bool beats(float v1, int p1, float v2, int p2, bool a
     if (n1 != n2) return n1;
     if (!n1 && v1 != v2) return amax ? v1 > v2 : v1 < v2;
     return p1 < p2;
-}
-
-// first row r in [0, num_v] with ptr[r] + r >= d
-__device__ int first_row(const int *ptr, int num_v, long long d) {
-    int lo = 0, hi = num_v;
-    while (lo < hi) {
-        const int mid = (lo + hi) >> 1;
-        if ((long long)__ldg(ptr + mid) + mid >= d) hi = mid;
-        else lo = mid + 1;
-    }
-    return lo;
 }
 
 // ---- forward ---------------------------------------------------------------------------------------------------
@@ -223,12 +209,11 @@ __device__ __forceinline__ void fold_groups(float (&v)[VEC][W], int (&p)[VEC][W]
 
 // Rows of at most kWarpMax nonzeros: one warp per row of its range, the groups interleaving the row's nonzeros.
 template <int W, int VEC, int U>
-__global__ void __launch_bounds__(kBlock) reduce_warp_kernel(const __grid_constant__ ReduceArgs a) {
+__global__ void __launch_bounds__(kRowBlock) reduce_warp_kernel(const __grid_constant__ ReduceArgs a) {
     const int lane = threadIdx.x & 31, L = a.lanes, G = 32 / L;
     const int l = lane % L, g = lane / L;
-    const long long w = (long long)blockIdx.x * kWarps + (threadIdx.x >> 5);
-    const int r0 = first_row(a.ptr, a.num_v, w * a.chunk);
-    const int r1 = first_row(a.ptr, a.num_v, (w + 1) * a.chunk);
+    int r0, r1;
+    warp_rows(a, r0, r1);
     const size_t row_units = (size_t)(a.feat / W);
     const int slice_units = L * VEC;
     for (int r = r0; r < r1; ++r) {
@@ -258,80 +243,68 @@ __global__ void __launch_bounds__(kBlock) reduce_warp_kernel(const __grid_consta
     }
 }
 
-// Rows of more than kWarpMax nonzeros, one CTA each: CTA b scans row stripes b, b + gridDim.x, ... of kBlock rows and
-// takes the long rows of a stripe in row order. The warps interleave the row's nonzeros; their winners meet in shared
-// memory.
+// Rows of more than kWarpMax nonzeros, one CTA each (the long-row launch of rows.cuh). The warps interleave the row's
+// nonzeros; their winners meet in shared memory.
 template <int W, int VEC, int U>
-__global__ void __launch_bounds__(kBlock) reduce_long_kernel(const __grid_constant__ ReduceArgs a) {
-    __shared__ unsigned long_mask[kWarps];
-    __shared__ float red_v[kWarps][kMaxSlice];
-    __shared__ int red_p[kWarps][kMaxSlice];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, L = a.lanes, G = 32 / L;
+__global__ void __launch_bounds__(kRowBlock) reduce_long_kernel(const __grid_constant__ ReduceArgs a) {
+    __shared__ unsigned long_mask[kRowWarps];
+    __shared__ float red_v[kRowWarps][kMaxSlice];
+    __shared__ int red_p[kRowWarps][kMaxSlice];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, L = a.lanes, G = 32 / L;
     const int l = lane % L, g = lane / L;
     const size_t row_units = (size_t)(a.feat / W);
     const int slice_units = L * VEC;
-    for (long long r0 = (long long)blockIdx.x * kBlock; r0 < a.num_v; r0 += (long long)gridDim.x * kBlock) {
-        const long long rr = r0 + threadIdx.x;
-        const bool is_long = rr < a.num_v && __ldg(a.ptr + rr + 1) - __ldg(a.ptr + rr) > kWarpMax;
-        const unsigned bm = __ballot_sync(kFull, is_long);
-        if (lane == 0) long_mask[warp] = bm;
-        __syncthreads();
-        for (int sw = 0; sw < kWarps; ++sw) {
-            for (unsigned rest = long_mask[sw]; rest; rest &= rest - 1) {
-                const int r = (int)r0 + sw * 32 + __ffs(rest) - 1;
-                const int rb = __ldg(a.ptr + r);
-                const int pb = __ldg(a.s0 + r), pe = __ldg(a.s1 + r);
-                if (pb == pe) {
-                    if (a.band == 0) fwd_store_empty<W>(a, (size_t)r * row_units, (size_t)(r + 1) * row_units, threadIdx.x, kBlock);
-                    continue;
-                }
-                const bool combine = a.band > 0 && pb > rb;
-                for (int s = 0; s < a.n_slices; ++s) {
-                    const size_t u0 = (size_t)s * slice_units + l;
-                    bool ok[VEC];
+    for_long_rows(a, kWarpMax, long_mask, [&](int r) {
+        const int rb = __ldg(a.ptr + r);
+        const int pb = __ldg(a.s0 + r), pe = __ldg(a.s1 + r);
+        if (pb == pe) {
+            if (a.band == 0) fwd_store_empty<W>(a, (size_t)r * row_units, (size_t)(r + 1) * row_units, tid, kRowBlock);
+            return;
+        }
+        const bool combine = a.band > 0 && pb > rb;
+        for (int s = 0; s < a.n_slices; ++s) {
+            const size_t u0 = (size_t)s * slice_units + l;
+            bool ok[VEC];
 #pragma unroll
-                    for (int i = 0; i < VEC; ++i) ok[i] = u0 + i * L < row_units;
-                    float v[VEC][W];
-                    int p[VEC][W];
-                    fwd_walk<W, VEC, U>(a, pb, pe, warp * G + g, kWarps * G, u0, ok, v, p);
-                    fold_groups<W, VEC>(v, p, L, a.amax);
-                    if (g == 0) {
+            for (int i = 0; i < VEC; ++i) ok[i] = u0 + i * L < row_units;
+            float v[VEC][W];
+            int p[VEC][W];
+            fwd_walk<W, VEC, U>(a, pb, pe, warp * G + g, kRowWarps * G, u0, ok, v, p);
+            fold_groups<W, VEC>(v, p, L, a.amax);
+            if (g == 0) {
 #pragma unroll
-                        for (int i = 0; i < VEC; ++i)
+                for (int i = 0; i < VEC; ++i)
 #pragma unroll
-                            for (int t = 0; t < W; ++t) {
-                                const int j = (l + i * L) * W + t;   // column inside the slice
-                                red_v[warp][j] = v[i][t];
-                                red_p[warp][j] = p[i][t];
-                            }
+                    for (int t = 0; t < W; ++t) {
+                        const int j = (l + i * L) * W + t;   // column inside the slice
+                        red_v[warp][j] = v[i][t];
+                        red_p[warp][j] = p[i][t];
                     }
-                    __syncthreads();
-                    const int cols = slice_units * W;
-                    const size_t c0 = (size_t)s * cols;
-                    for (int j = threadIdx.x; j < cols && c0 + j < (size_t)a.feat; j += kBlock) {
-                        float bv = red_v[0][j];
-                        int bp = red_p[0][j];
-                        for (int k = 1; k < kWarps; ++k)
-                            if (beats(red_v[k][j], red_p[k][j], bv, bp, a.amax)) bv = red_v[k][j], bp = red_p[k][j];
-                        const size_t o = (size_t)r * a.feat + c0 + j;
-                        if (!combine || later_wins(bv, a.vout[o], a.amax)) {
-                            a.vout[o] = bv;
-                            if (a.arg) a.arg[o] = bp;
-                        }
-                    }
-                    __syncthreads();   // red_v / red_p are rewritten by the next slice or row
+            }
+            __syncthreads();
+            const int cols = slice_units * W;
+            const size_t c0 = (size_t)s * cols;
+            for (int j = tid; j < cols && c0 + j < (size_t)a.feat; j += kRowBlock) {
+                float bv = red_v[0][j];
+                int bp = red_p[0][j];
+                for (int k = 1; k < kRowWarps; ++k)
+                    if (beats(red_v[k][j], red_p[k][j], bv, bp, a.amax)) bv = red_v[k][j], bp = red_p[k][j];
+                const size_t o = (size_t)r * a.feat + c0 + j;
+                if (!combine || later_wins(bv, a.vout[o], a.amax)) {
+                    a.vout[o] = bv;
+                    if (a.arg) a.arg[o] = bp;
                 }
             }
+            __syncthreads();   // red_v / red_p are rewritten by the next slice or row
         }
-        __syncthreads();   // long_mask is rewritten by the next stripe
-    }
+    });
 }
 
 // ---- backward --------------------------------------------------------------------------------------------------
 
 // One tile [kb, ke) of an Aᵀ row c, for the slice at unit u0 (+ the lane's units l + v*L): s = the tile's chain per
 // column (db). With x (vin[c]'s slice, the whole row: one slice) also dval of every entry, in sddmm's order over the
-// group's L lanes (gmask).
+// group's L lanes (gmask); that order holds only while layout() takes L from sddmm's lane rule (common.h).
 template <int W, int VEC, int U>
 __device__ __forceinline__ void bwd_tile(const BwdArgs &a, int kb, int ke, size_t u0, const bool (&ok)[VEC],
                                          float (&s)[VEC][W], const float (&x)[VEC][W], bool with_dval, int l,
@@ -419,13 +392,12 @@ __device__ __forceinline__ void bwd_dval_walk(const BwdArgs &a, int c, int kb, i
 // Aᵀ rows of at most kBwdWarpMax entries: the warp's groups take the rows of its range round-robin, each row walked
 // tile by tile by one group.
 template <int W, int VEC, int U>
-__global__ void __launch_bounds__(kBlock) reduce_bwd_warp_kernel(const __grid_constant__ BwdArgs a) {
+__global__ void __launch_bounds__(kRowBlock) reduce_bwd_warp_kernel(const __grid_constant__ BwdArgs a) {
     const int lane = threadIdx.x & 31, L = a.lanes, G = 32 / L;
     const int l = lane % L, g = lane / L;
     const unsigned gmask = L == 32 ? kFull : ((1u << L) - 1) << (g * L);
-    const long long w = (long long)blockIdx.x * kWarps + (threadIdx.x >> 5);
-    const int r0 = first_row(a.ptr, a.num_v, w * a.chunk);
-    const int r1 = first_row(a.ptr, a.num_v, (w + 1) * a.chunk);
+    int r0, r1;
+    warp_rows(a, r0, r1);
     const size_t row_units = (size_t)(a.feat / W);
     const int slice_units = L * VEC;
     const bool fused = a.n_slices == 1;
@@ -461,96 +433,80 @@ __global__ void __launch_bounds__(kBlock) reduce_bwd_warp_kernel(const __grid_co
     }
 }
 
-// Aᵀ rows of more than kBwdWarpMax entries, one CTA each (found as in reduce_long_kernel). The CTA's lane groups take
-// the tiles round-robin, kWarps * G tiles per round; the tile sums of a round are added in tile order through shared
+// Aᵀ rows of more than kBwdWarpMax entries, one CTA each (the long-row launch of rows.cuh). The CTA's lane groups take
+// the tiles round-robin, kRowWarps * G tiles per round; the tile sums of a round are added in tile order through shared
 // memory.
 template <int W, int VEC, int U>
-__global__ void __launch_bounds__(kBlock, 1) reduce_bwd_long_kernel(const __grid_constant__ BwdArgs a) {
-    constexpr int kSumCols = kWarps * 32 * VEC * W;   // workers (kWarps * G) x slice columns (L * VEC * W)
-    __shared__ unsigned long_mask[kWarps];
+__global__ void __launch_bounds__(kRowBlock, 1) reduce_bwd_long_kernel(const __grid_constant__ BwdArgs a) {
+    constexpr int kSumCols = kRowWarps * 32 * VEC * W;   // workers (kRowWarps * G) x slice columns (L * VEC * W)
+    __shared__ unsigned long_mask[kRowWarps];
     __shared__ float tsum[kSumCols];
     __shared__ float acc[kMaxSlice];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, L = a.lanes, G = 32 / L;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, L = a.lanes, G = 32 / L;
     const int l = lane % L, g = lane / L;
-    const int worker = warp * G + g, n_workers = kWarps * G;
+    const int worker = warp * G + g, n_workers = kRowWarps * G;
     const unsigned gmask = L == 32 ? kFull : ((1u << L) - 1) << (g * L);
     const size_t row_units = (size_t)(a.feat / W);
     const int slice_units = L * VEC, cols = slice_units * W;
     const bool fused = a.n_slices == 1;
-    for (long long r0 = (long long)blockIdx.x * kBlock; r0 < a.num_v; r0 += (long long)gridDim.x * kBlock) {
-        const long long rr = r0 + threadIdx.x;
-        const bool is_long = rr < a.num_v && __ldg(a.ptr + rr + 1) - __ldg(a.ptr + rr) > kBwdWarpMax;
-        const unsigned bm = __ballot_sync(kFull, is_long);
-        if (lane == 0) long_mask[warp] = bm;
-        __syncthreads();
-        for (int sw = 0; sw < kWarps; ++sw) {
-            for (unsigned rest = long_mask[sw]; rest; rest &= rest - 1) {
-                const int c = (int)r0 + sw * 32 + __ffs(rest) - 1;
-                const int kb = __ldg(a.ptr + c), ke = __ldg(a.ptr + c + 1);
-                const int nt = (ke - kb + kTile - 1) / kTile;
-                if (a.db || (fused && a.dval)) {
-                    for (int s = 0; s < a.n_slices; ++s) {
-                        const size_t u0 = (size_t)s * slice_units + l;
-                        const size_t c0 = (size_t)s * cols;
-                        bool ok[VEC];
-                        float x[VEC][W], ts[VEC][W];
+    for_long_rows(a, kBwdWarpMax, long_mask, [&](int c) {
+        const int kb = __ldg(a.ptr + c), ke = __ldg(a.ptr + c + 1);
+        const int nt = (ke - kb + kTile - 1) / kTile;
+        if (a.db || (fused && a.dval)) {
+            for (int s = 0; s < a.n_slices; ++s) {
+                const size_t u0 = (size_t)s * slice_units + l;
+                const size_t c0 = (size_t)s * cols;
+                bool ok[VEC];
+                float x[VEC][W], ts[VEC][W];
 #pragma unroll
-                        for (int i = 0; i < VEC; ++i) {
-                            ok[i] = u0 + i * L < row_units;
+                for (int i = 0; i < VEC; ++i) {
+                    ok[i] = u0 + i * L < row_units;
 #pragma unroll
-                            for (int t = 0; t < W; ++t) x[i][t] = 0.0f;
-                            if (ok[i] && fused && a.dval) ldf<W>(x[i], a.vin, (size_t)c * row_units + u0 + i * L);
-                        }
-                        for (int j = threadIdx.x; j < cols; j += kBlock) acc[j] = 0.0f;
-                        for (int t0 = 0; t0 < nt; t0 += n_workers) {
-                            const int t = t0 + worker;
-                            if (t < nt) {
-                                bwd_tile<W, VEC, U>(a, kb + t * kTile, min(ke, kb + (t + 1) * kTile), u0, ok, ts, x,
-                                                    fused && a.dval, l, gmask);
-#pragma unroll
-                                for (int i = 0; i < VEC; ++i)
-#pragma unroll
-                                    for (int q = 0; q < W; ++q) tsum[worker * cols + (l + i * L) * W + q] = ts[i][q];
-                            }
-                            __syncthreads();
-                            const int n_here = min(n_workers, nt - t0);
-                            for (int j = threadIdx.x; j < cols; j += kBlock)
-                                for (int k = 0; k < n_here; ++k) acc[j] = __fadd_rn(acc[j], tsum[k * cols + j]);
-                            __syncthreads();
-                        }
-                        if (a.db)
-                            for (int j = threadIdx.x; j < cols && c0 + j < (size_t)a.feat; j += kBlock)
-                                a.db[(size_t)c * a.feat + c0 + j] = acc[j];
-                        __syncthreads();   // acc is reset by the next slice or row
-                    }
+                    for (int t = 0; t < W; ++t) x[i][t] = 0.0f;
+                    if (ok[i] && fused && a.dval) ldf<W>(x[i], a.vin, (size_t)c * row_units + u0 + i * L);
                 }
-                if (a.dval && !fused) bwd_dval_walk<W>(a, c, kb, ke, worker, n_workers, l, gmask);
+                for (int j = tid; j < cols; j += kRowBlock) acc[j] = 0.0f;
+                for (int t0 = 0; t0 < nt; t0 += n_workers) {
+                    const int t = t0 + worker;
+                    if (t < nt) {
+                        bwd_tile<W, VEC, U>(a, kb + t * kTile, min(ke, kb + (t + 1) * kTile), u0, ok, ts, x,
+                                            fused && a.dval, l, gmask);
+#pragma unroll
+                        for (int i = 0; i < VEC; ++i)
+#pragma unroll
+                            for (int q = 0; q < W; ++q) tsum[worker * cols + (l + i * L) * W + q] = ts[i][q];
+                    }
+                    __syncthreads();
+                    const int n_here = min(n_workers, nt - t0);
+                    for (int j = tid; j < cols; j += kRowBlock)
+                        for (int k = 0; k < n_here; ++k) acc[j] = __fadd_rn(acc[j], tsum[k * cols + j]);
+                    __syncthreads();
+                }
+                if (a.db)
+                    for (int j = tid; j < cols && c0 + j < (size_t)a.feat; j += kRowBlock)
+                        a.db[(size_t)c * a.feat + c0 + j] = acc[j];
+                __syncthreads();   // acc is reset by the next slice or row
             }
         }
-        __syncthreads();   // long_mask is rewritten by the next stripe
-    }
+        if (a.dval && !fused) bwd_dval_walk<W>(a, c, kb, ke, worker, n_workers, l, gmask);
+    });
 }
 
 // ---- host --------------------------------------------------------------------------------------------------------
 
-int pow2_lanes(int q) {
-    int l = 1;
-    while (l < q && l < 32) l <<= 1;
-    return l;
-}
-
-// The lane shape: W columns per unit, L lanes, VEC units per lane and slice. K % 4 == 0, K <= 512: sddmm's fast shape
-// (one slice); K % 4 == 0, K > 512: 32 lanes x 4 float4; K % 4 != 0: sddmm's scalar lane count, 4 columns per lane.
+// The lane shape: W columns per unit, L lanes, VEC units per lane and slice. L is sddmm's (common.h), which dval's bits
+// rely on. K % 4 == 0, K <= 512: sddmm's fast shape (one slice); K % 4 == 0, K > 512: 32 lanes x 4 float4; K % 4 != 0:
+// sddmm's scalar lane count, 4 columns per lane.
 struct Layout {
     int w, lanes, vec, n_slices;
 };
 Layout layout(int K) {
     Layout s;
     if (K % 4 == 0 && K <= 512) {
-        const int q = K / 4, l = pow2_lanes(q), need = (q + l - 1) / l;
-        s = {4, l, need <= 1 ? 1 : need <= 2 ? 2 : 4, 1};
+        const LaneShape f = fast_lane_shape(K);
+        s = {4, f.lanes, f.vec, 1};
     } else if (K % 4 == 0) {
-        s = {4, 32, 4, 0};
+        s = {4, pow2_lanes(K / 4), 4, 0};
     } else {
         s = {1, pow2_lanes(K), 4, 0};
     }
@@ -559,36 +515,16 @@ Layout layout(int K) {
     return s;
 }
 
-struct Grid {
-    unsigned warp_blocks, long_blocks;
-    long long chunk;
-};
-int grid_for(int num_v, long long num_e, Grid *gr) {
-    int dev = 0, sms = 0;
-    SB_CUDA(cudaGetDevice(&dev));
-    SB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (sms <= 0) sms = 1;
-    const long long d = num_e + num_v;
-    const long long target = (long long)sms * 32 * kWarpWaves;
-    gr->chunk = (d + target - 1) / target;
-    if (gr->chunk < kMinChunk) gr->chunk = kMinChunk;
-    const long long warps = (d + gr->chunk - 1) / gr->chunk;
-    gr->warp_blocks = (unsigned)((warps + kWarps - 1) / kWarps);
-    const long long stripes = ((long long)num_v + kBlock - 1) / kBlock;
-    gr->long_blocks = (unsigned)(stripes < (long long)sms * 4 ? stripes : (long long)sms * 4);
-    return 0;
+template <int W, int VEC, int U>
+void launch_fwd(const ReduceArgs &a, const RowGrid &gr, cudaStream_t s) {
+    reduce_warp_kernel<W, VEC, U><<<gr.warp_blocks, kRowBlock, 0, s>>>(a);
+    reduce_long_kernel<W, VEC, U><<<gr.long_blocks, kRowBlock, 0, s>>>(a);
 }
 
 template <int W, int VEC, int U>
-void launch_fwd(const ReduceArgs &a, const Grid &gr, cudaStream_t s) {
-    reduce_warp_kernel<W, VEC, U><<<gr.warp_blocks, kBlock, 0, s>>>(a);
-    reduce_long_kernel<W, VEC, U><<<gr.long_blocks, kBlock, 0, s>>>(a);
-}
-
-template <int W, int VEC, int U>
-void launch_bwd(const BwdArgs &a, const Grid &gr, cudaStream_t s) {
-    reduce_bwd_warp_kernel<W, VEC, U><<<gr.warp_blocks, kBlock, 0, s>>>(a);
-    reduce_bwd_long_kernel<W, VEC, U><<<gr.long_blocks, kBlock, 0, s>>>(a);
+void launch_bwd(const BwdArgs &a, const RowGrid &gr, cudaStream_t s) {
+    reduce_bwd_warp_kernel<W, VEC, U><<<gr.warp_blocks, kRowBlock, 0, s>>>(a);
+    reduce_bwd_long_kernel<W, VEC, U><<<gr.long_blocks, kRowBlock, 0, s>>>(a);
 }
 
 // the four instantiations: (W, VEC) = (4, 1), (4, 2), (4, 4), (1, 4); U = entries in flight per lane group
@@ -633,8 +569,8 @@ extern "C" int spmm_b200_reduce(spmm_b200_t h, int op, const float *vin, float *
     }
     cudaStream_t s = (cudaStream_t)stream;
     const Layout ly = layout(K);
-    Grid gr;
-    int rc = grid_for(h->num_v, h->num_e, &gr);
+    RowGrid gr;
+    int rc = row_grid(h->num_v, h->num_e, &gr);
     if (rc) return rc;
     const Plan &p = h->plan;
     const int nb = p.n_col_blocks > 1 ? p.n_col_blocks : 1;
@@ -689,8 +625,8 @@ extern "C" int spmm_b200_reduce_backward(spmm_b200_t t, const float *dc, const i
     }
     cudaStream_t s = (cudaStream_t)stream;
     const Layout ly = layout(K);
-    Grid gr;
-    int rc = grid_for(t->num_v, t->num_e, &gr);
+    RowGrid gr;
+    int rc = row_grid(t->num_v, t->num_e, &gr);
     if (rc) return rc;
     BwdArgs a;
     a.ptr = t->t_ptr;

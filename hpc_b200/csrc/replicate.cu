@@ -73,11 +73,8 @@ int launch_push_rows(const float *src, long long off, long long count, int n, fl
     }
     PtrTable tg;
     for (int t = 0; t < kMaxGather; ++t) tg.p[t] = t < n ? targets[t] : nullptr;
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-        cudaGetLastError();
-        sms = 148;
-    }
+    int sms = sm_count();
+    if (sms <= 0) sms = 148;
     const long long n4 = count / 4;
     long long blocks = (n4 + 255) / 256;
     if (blocks > 8ll * sms) blocks = 8ll * sms;

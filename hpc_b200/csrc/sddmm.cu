@@ -211,31 +211,16 @@ bool walk_banded(const spmm_b200_handle *h) {
     return h->plan.n_col_blocks > 1 && (long long)h->plan.n_col_blocks * h->num_v + 1 <= (long long)INT_MAX;
 }
 
-int pow2_lanes(int q) {
-    int l = 1;
-    while (l < q && l < 32) l <<= 1;
-    return l;
-}
-
-// the fast kernel's shape for K % 4 == 0, K <= 512: lanes = L, vec = float4 per lane (1, 2 or 4), u = entries in flight
-struct Shape {
-    int lanes, vec, u;
-};
-Shape fast_shape(int K) {
-    const int q = K / 4, l = pow2_lanes(q);
-    const int need = (q + l - 1) / l;
-    const int vec = need <= 1 ? 1 : need <= 2 ? 2 : 4;
-    return {l, vec, vec == 4 ? 2 : 4};
-}
-
 template <int LANES, int VEC, int U>
 void *fast_fn() {
     return reinterpret_cast<void *>(&sddmm_kernel<LANES, VEC, U>);
 }
+// The kernel for width K, for both the occupancy query and the launch: sddmm_kernel<L, VEC, U> with (L, VEC) =
+// fast_lane_shape(K) and U = entries in flight per lane group, or a generic kernel. NULL: no kernel for K.
 void *kernel_fn(int K) {
     if (K % 4 != 0) return reinterpret_cast<void *>(&sddmm_generic_kernel<false>);
     if (K > 512) return reinterpret_cast<void *>(&sddmm_generic_kernel<true>);
-    const Shape sh = fast_shape(K);
+    const LaneShape sh = fast_lane_shape(K);
     switch (sh.lanes * 10 + sh.vec) {
         case 11: return fast_fn<1, 1, 4>();
         case 21: return fast_fn<2, 1, 4>();
@@ -278,15 +263,14 @@ int prepare(spmm_b200_handle *h, cudaStream_t stream) {
         p.d_sddmm_vp = vp;
     }
     if (p.sddmm_chunk == 0) {
-        int per_sm = 0, dev = 0, sms = 0;
+        int per_sm = 0, sms = 0;
         void *fn = kernel_fn(K);
         if (!fn) {
             set_error("spmm_b200_sddmm: no kernel for feat_in = %d", K);
             return SPMM_B200_EINVAL;
         }
         SB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kBlock, 0));
-        SB_CUDA(cudaGetDevice(&dev));
-        SB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        SB_CUDA(query_sm_count(&sms));
         const long long warps = (long long)(per_sm > 0 ? per_sm : 1) * (kBlock / 32) * (sms > 0 ? sms : 1);
         long long chunk = (h->num_e + kWaves * warps - 1) / (kWaves * warps);
         if (chunk < kMinChunk) chunk = kMinChunk;
@@ -344,26 +328,11 @@ extern "C" int spmm_b200_sddmm(spmm_b200_t h, const float *x_row, const float *x
     a.chunk = p.sddmm_chunk;
     const long long warps = ((long long)h->num_e + a.chunk - 1) / a.chunk;
     const unsigned grid = (unsigned)((warps + kBlock / 32 - 1) / (kBlock / 32));
-    if (K % 4 != 0) {
-        sddmm_generic_kernel<false><<<grid, kBlock, 0, s>>>(a, pow2_lanes(K));
-    } else if (K > 512) {
-        sddmm_generic_kernel<true><<<grid, kBlock, 0, s>>>(a, pow2_lanes(K / 4));
-    } else {
-        const Shape sh = fast_shape(K);
-        switch (sh.lanes * 10 + sh.vec) {
-            case 11: sddmm_kernel<1, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 21: sddmm_kernel<2, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 41: sddmm_kernel<4, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 81: sddmm_kernel<8, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 161: sddmm_kernel<16, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 321: sddmm_kernel<32, 1, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 322: sddmm_kernel<32, 2, 4><<<grid, kBlock, 0, s>>>(a); break;
-            case 324: sddmm_kernel<32, 4, 2><<<grid, kBlock, 0, s>>>(a); break;
-            default:
-                set_error("spmm_b200_sddmm: unsupported shape lanes=%d vec=%d", sh.lanes, sh.vec);
-                return SPMM_B200_EINVAL;
-        }
-    }
+    int lanes = pow2_lanes(K % 4 != 0 ? K : K / 4);   // the generic kernels' second parameter
+    void *args[] = {&a, &lanes};
+    // kernel_fn(K) is not NULL: prepare checked it. As after <<< >>>, cudaGetLastError reports a failed launch and
+    // clears it, so the caller's next cudaGetLastError does not see it again.
+    cudaLaunchKernel(kernel_fn(K), grid, kBlock, args, 0, s);
     SB_CUDA(cudaGetLastError());
     return 0;
 }

@@ -605,15 +605,6 @@ int ctas_per_sm(int lanes, int vec, int tune, int block) {
     }
 }
 
-int sm_count() {
-    int dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return sms;
-}
-
 void fill_common(CommonArgs &c, const spmm_b200_handle *h, const float *vin, float *vout, float *cfinal) {
     const Plan &p = h->plan;
     c.idx = h->d_idx;
@@ -712,13 +703,8 @@ int resident_warps(int lanes, int vec, int tune, int block) {
 
 // grid cap for the grid-stride support kernels: 16 CTAs per SM of the current device
 static long long stride_grid_cap() {
-    int dev = 0, sms = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-        sms <= 0) {
-        cudaGetLastError();
-        sms = 148;   // B200
-    }
-    return 16ll * sms;
+    const int sms = sm_count();
+    return 16ll * (sms > 0 ? sms : 148);   // 148: B200
 }
 
 int launch_check_cols(const int *d_idx, long long nnz, int b_rows, int *d_bad, cudaStream_t stream) {

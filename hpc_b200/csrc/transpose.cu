@@ -59,11 +59,8 @@ __global__ void __launch_bounds__(256) gather_t_kernel(const int *perm, const in
 }
 
 int grid_for(long long n) {
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-        cudaGetLastError();
-        sms = 148;
-    }
+    int sms = sm_count();
+    if (sms <= 0) sms = 148;
     long long blocks = (n + 255) / 256;
     if (blocks > 16ll * sms) blocks = 16ll * sms;
     return (int)(blocks < 1 ? 1 : blocks);

@@ -172,7 +172,7 @@ def test_cpp_adapter_sddmm_compiles(tmp_path):
 # ---- dispatch coverage of the GPU tests ----------------------------------------------------------------------------
 
 def _pow2_lanes(q):
-    """pow2_lanes of sddmm.cu"""
+    """pow2_lanes of common.h (the lane count of sddmm.cu and reduce.cu)"""
     lanes = 1
     while lanes < q and lanes < 32:
         lanes <<= 1
@@ -180,7 +180,7 @@ def _pow2_lanes(q):
 
 
 def _fast_shape(k):
-    """fast_shape of sddmm.cu: (lanes, float4 per lane) of sddmm_kernel for K % 4 == 0, K <= 512"""
+    """fast_lane_shape of common.h: (lanes, float4 per lane) of sddmm_kernel for K % 4 == 0, K <= 512"""
     q = k // 4
     lanes = _pow2_lanes(q)
     need = -(-q // lanes)
