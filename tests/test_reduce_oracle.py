@@ -265,3 +265,36 @@ def test_gpu_widths_reach_every_reduce_dispatch_case():
     assert {lanes for w, lanes, _, _ in shapes if w == 1} == {1, 2, 4, 8, 16, 32}
     assert {(w, n > 1) for w, _, _, n in shapes} == {(4, False), (4, True), (1, False), (1, True)}
     assert 1024 in RG.WIDTHS and 516 in RG.WIDTHS
+
+
+def test_path_tests_reach_every_reduce_boundary():
+    """tests/test_reduce_paths_gpu.py reaches, with the thresholds read from reduce.cu and rows.cuh: every (W, VEC)
+    instantiation of the forward (its CTA kernel included) at every float4 lane count, one- and several-slice layouts;
+    rows on each side of kWarpMax; Aᵀ rows on each side of kTile and kBwdWarpMax; and a second round of the backward
+    CTA's lane groups at L = 1, 4, 8 and 32, ending partway through it."""
+    import test_reduce_paths_gpu as RP
+    src = open(os.path.join(ROOT, "hpc_b200", "csrc", "reduce.cu")).read()
+    rows_src = open(os.path.join(ROOT, "hpc_b200", "csrc", "rows.cuh")).read()
+    c = RP.source_constants()
+    assert f"constexpr int kWarpMax = {c['kWarpMax']};" in src and f"constexpr int kTile = {c['kTile']};" in src
+    assert "constexpr int kBwdWarpMax = 4 * kTile;" in src and c["kBwdWarpMax"] == 4 * c["kTile"]
+    assert f"constexpr int kRowBlock = {c['kRowBlock']};" in rows_src and c["kRowWarps"] == c["kRowBlock"] // 32
+    table = {(int(w), int(v)) for w, v in re.findall(r"launch_fwd<(\d+), (\d+), \d+>\(a, gr, s\)", src)}
+    fwd = [_layout(k) for k in RP.FWD_WIDTHS]
+    assert {(w, v) for w, _, v, _ in fwd} == table
+    assert {lanes for w, lanes, _, _ in fwd if w == 4} == {1, 2, 4, 8, 16, 32}
+    assert {lanes for w, lanes, _, _ in fwd if w == 1} >= {1, 32}
+    assert {(w, n > 1) for w, _, _, n in fwd} == {(4, False), (4, True), (1, False), (1, True)}
+    lens = set(RP.FWD_ROW_LENGTHS)
+    assert {c["kWarpMax"] - 1, c["kWarpMax"], c["kWarpMax"] + 1} <= lens and max(lens) >= 30 * c["kWarpMax"]
+    cols = RP.BWD_COLUMN_LENGTHS
+    T, W = c["kTile"], c["kBwdWarpMax"]
+    assert {T - 1, T, T + 1, W, W + 1} <= set(cols)
+    bwd_lanes = {_layout(k)[1] for k in RP.BWD_WIDTHS}
+    assert bwd_lanes >= {1, 4, 8, 32}
+    assert any(_layout(k)[3] > 1 for k in RP.BWD_WIDTHS)                 # the separate dval walk
+    for lanes in (1, 4, 8, 32):
+        workers = c["kRowWarps"] * 32 // lanes
+        tiles = [-(-n // T) for n in cols]
+        assert any(t > workers and t % workers for t in tiles), lanes     # a second round, the last one partial
+    assert c["kRowWarps"] * 32 // 32 * T in cols                          # exactly one full round at L = 32
