@@ -44,6 +44,7 @@ SIGNATURES = {
     "spmm_b200_preprocess": (_I, [_P, _P, _P, _P]),
     "spmm_b200_refresh_values": (_I, [_P, _P]),
     "spmm_b200_run": (_I, [_P, _P, _P, _P]),
+    "spmm_b200_run_values": (_I, [_P, _P, _P, _P, _P]),
     "spmm_b200_run_profiled": (_I, [_P, _P, _P, _P, C.POINTER(C.c_float)]),
     "spmm_b200_create_transposed": (_I, [_P, _I, _P, C.POINTER(_P)]),
     "spmm_b200_sddmm": (_I, [_P, _P, _P, _P, _P]),

@@ -6,7 +6,7 @@ which also records the winning nonzero of every output, and the backward is `red
 operator; reduce="mean" divides the sum by the row's nonzero count.
 
 GraphAttention: scores = sddmm(q, k), alpha = edge_softmax(scores), out = A_alpha·v, with A_alpha the graph's pattern
-carrying alpha as edge values; every step differentiable.
+carrying alpha as edge values (run_values on live-value operators); every step differentiable.
 """
 from __future__ import annotations
 
@@ -147,13 +147,6 @@ class GraphSpMM:
             pass
 
 
-def _stage(mod, values, op):
-    """Puts `values` into the attention module's edge-value buffer and re-stages `op`'s panels from it. Done before every
-    run: autograd interleaves the backwards of several calls, so nothing can be assumed about what is staged."""
-    mod._val.copy_(values)
-    op.refresh_values()
-
-
 class _ScoresFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mod, q, k):
@@ -171,13 +164,10 @@ class _ScoresFn(torch.autograd.Function):
         dq = dk = None
         if ctx.needs_input_grad[1]:   # dq = S_ds·k
             dq = torch.empty_like(q)
-            _stage(mod, ds, mod.op)
-            mod.op.run(k, dq)
+            mod.op.run_values(ds, k, dq)
         if ctx.needs_input_grad[2]:   # dk = S_dsᵀ·q
             dk = torch.empty_like(k)
-            t = mod.transposed()
-            _stage(mod, ds, t)
-            t.run(q, dk)
+            mod.transposed().run_values(ds, q, dk)
         return None, dq, dk
 
 
@@ -202,9 +192,7 @@ class _AggregateFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mod, alpha, v):
         out = torch.empty((mod.g.num_v, mod.feat_in), dtype=torch.float32, device=v.device)
-        op = mod._op()
-        _stage(mod, alpha, op)
-        op.run(v, out)
+        mod._op().run_values(alpha, v, out)
         ctx.mod = mod
         ctx.save_for_backward(alpha, v)
         return out
@@ -220,9 +208,7 @@ class _AggregateFn(torch.autograd.Function):
             mod.op.sddmm(dout, v, dalpha)
         if ctx.needs_input_grad[2]:   # dv = A_alphaᵀ·dout
             dv = torch.empty_like(v)
-            t = mod.transposed()
-            _stage(mod, alpha, t)
-            t.run(dout, dv)
+            mod.transposed().run_values(alpha, dout, dv)
         return None, dalpha, dv
 
 
@@ -231,16 +217,16 @@ class GraphAttention:
     q: num_v x feat_in, k and v: b_rows x feat_in (CUDA float32). Differentiable in q, k and v, and through the separate
     steps scores / softmax / aggregate (e.g. GAT scores built in torch, then softmax and aggregate). The caller scales q.
 
-    Uses g.ptr / g.idx only: the edge values of every run are the module's own buffer, so g.val is never read or
-    written. options are passed to the forward operator (SpMMB200), e.g. b_rows for a row block. The forward operator
-    is planned on first use, the transposed one is created when a gradient first needs it. Call close() when done (or
-    rely on garbage collection)."""
+    The operators are built over g with live values: every run takes its edge values (alpha, or the score gradient) as
+    an argument and reads them in the kernel, so nothing is staged between runs and g.val is never written. The
+    transposed operator reads the same arrays, in g's CSR positions. options are passed to the forward operator
+    (SpMMB200), e.g. b_rows for a row block. The forward operator is planned on first use, the transposed one is created
+    when a gradient first needs it. Call close() when done (or rely on garbage collection)."""
 
     def __init__(self, g: CSR, feat_in: int, **options):
         self.g = g
         self.feat_in = int(feat_in)
-        self._val = torch.zeros(g.num_e, dtype=torch.float32, device=g.ptr.device)
-        self.op = SpMMB200(CSR(g.num_v, g.num_e, g.ptr, g.idx, self._val), self.feat_in, **options)
+        self.op = SpMMB200(g, self.feat_in, live_values=1, **options)
         self._t = None
         self._prepared = False
 
@@ -255,11 +241,11 @@ class GraphAttention:
         return self.op
 
     def transposed(self) -> SpMMB200:
-        """The operator over the pattern's transpose (created and planned on first use); it reads the module's edge-value
-        buffer through refresh_values."""
+        """The operator over the pattern's transpose (created and planned on first use); run_values on it takes edge
+        values in g's CSR positions."""
         if self._t is None:
             op = self._op()
-            self._t = op.transposed(self.feat_in)
+            self._t = op.transposed(self.feat_in, live_values=1)
             dev = self.g.ptr.device
             dc = torch.empty((op.num_v, self.feat_in), dtype=torch.float32, device=dev)
             db = torch.empty((op.b_rows, self.feat_in), dtype=torch.float32, device=dev)

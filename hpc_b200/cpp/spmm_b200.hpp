@@ -76,6 +76,10 @@ class SpMMB200 : public SpMM {
     virtual void preprocess(float *vin, float *vout) { check(spmm_b200_preprocess(h_, vin, vout, stream_), "preprocess"); }
     // asynchronous on the stream (default stream unless set_stream), like SpMMRef::run (spmm_ref.cu:27-30)
     virtual void run(float *vin, float *vout) { check(spmm_b200_run(h_, vin, vout, stream_), "run"); }
+    // run with this call's edge values (val: the source operator's num_e floats); needs option live_values = 1
+    void run_values(const float *val, const float *vin, float *vout) {
+        check(spmm_b200_run_values(h_, val, vin, vout, stream_), "run_values");
+    }
 
     // re-stage the plan's copy of idx / val after the caller changed the edge values in place (the reference's
     // SpMMOpt::run reads them live, PA4/workspace/src/spmm_opt.cu:22-25)

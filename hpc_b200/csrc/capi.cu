@@ -84,6 +84,7 @@ int spmm_b200_set_option(spmm_b200_t h, const char *name, long long value) {
     else if (!strcmp(name, "row_groups") && value >= 0 && value <= kMaxRowGroups) h->opt_row_groups = value;
     else if (!strcmp(name, "split_streams") && value >= -1 && value <= 1) h->opt_split_streams = value;
     else if (!strcmp(name, "host_bands") && (value == 0 || value == 1 || (value >= 10 && value <= 90))) h->opt_host_bands = value;
+    else if (!strcmp(name, "live_values") && value >= 0 && value <= 1) h->opt_live_values = value;
     else if (!strcmp(name, "zero_copy") && value >= 0 && value <= 1) {
         h->opt_zero_copy = value;   // run_host only; not part of the plan
         return 0;
@@ -173,6 +174,20 @@ int spmm_b200_run(spmm_b200_t h, const float *vin, float *vout, void *stream) {
     int rc = check_run_args("spmm_b200_run", h, vin, vout);
     if (rc) return rc;
     return launch_spmm(h, vin, vout, (cudaStream_t)stream, &h->plan.launches);
+}
+
+int spmm_b200_run_values(spmm_b200_t h, const float *val, const float *vin, float *vout, void *stream) {
+    int rc = check_run_args("spmm_b200_run_values", h, vin, vout);
+    if (rc) return rc;
+    if (!h->plan.live) {
+        set_error("spmm_b200_run_values: the plan stages its values; set option live_values = 1 before preprocess");
+        return SPMM_B200_ESTATE;
+    }
+    if (h->num_e > 0 && !val) {
+        set_error("spmm_b200_run_values: null val");
+        return SPMM_B200_EINVAL;
+    }
+    return launch_spmm(h, vin, vout, (cudaStream_t)stream, &h->plan.launches, nullptr, nullptr, val);
 }
 
 int spmm_b200_run_profiled(spmm_b200_t h, const float *vin, float *vout, void *stream, float *ms) {

@@ -41,7 +41,8 @@ constexpr int kMaxRowGroups = 64;
 // What every pass of a run shares.
 struct CommonArgs {
     const int *idx;           // scalar fallback kernel only (the vectorised kernels read the staged panels)
-    const float *val;
+    const float *val;         // scalar kernel; with live values also the vectorised kernels: val[panel .y word]
+    const int *perm;          // live values on a derived handle (scalar kernel): the weight of position i is val[perm[i]]
     const float *vin;
     float *vout;              // C: partial chains between column-block passes, and final rows unless cfinal differs
     float *cfinal;            // where FINAL rows are stored (= vout, or device-mapped pinned host memory: run_host's zero-copy output)
@@ -63,6 +64,7 @@ struct BandArgs {
                               // for a light-stream task, {-1 - segment, 0} for a heavy segment
     int n_utask;
     const int2 *lpanel;       // light rows as a stream: header {0x80000000|row, 0}, then {col, val}..., nop = {-1, -1}
+                              // (live values: {col, position} instead of {col, val})
     const SegDesc *seg_desc;
     const int *seg_hrow;      // segment -> index of its row in heavy_rows
     const int *heavy_seg0;    // heavy row -> first segment (prefix, n_heavy + 1)
@@ -98,6 +100,7 @@ struct Plan {
     int device = -1;   // the device the plan's arrays live on (the current device at preprocess)
     int seg_len = 0, kslice = 0, n_slices = 0, block = 128, lanes = 0, vec = 0, tune = 0, light_steps = 0;
     bool scalar = false;   // K % 4 != 0: scalar fallback kernel, no segments
+    bool live = false;     // option "live_values": panels stage positions, runs read the weights from a value array
     int n_col_blocks = 1;
     long long slots = 0;   // warps the device keeps resident for the chosen kernel shape
     int *d_split = nullptr;   // [(n_col_blocks+1)][num_v] start of each column block inside each row
@@ -123,7 +126,7 @@ struct spmm_b200_handle {
     const float *d_val = nullptr;
     int num_v = 0, num_e = 0, feat = 0;
     long long opt_seg_len = 0, opt_kslice = 0, opt_block = 128, opt_reorder = -1, opt_tune = 0, opt_col_blocks = 0, opt_light_steps = 0,
-              opt_zero_copy = 1, opt_row_groups = 0, opt_split_streams = -1, opt_host_bands = 0;
+              opt_zero_copy = 1, opt_row_groups = 0, opt_split_streams = -1, opt_host_bands = 0, opt_live_values = 0;
     int plan_select = 0;   // which column block plan_info / plan_copy describe
     spmm_b200::Plan plan;
     float *d_stage_in = nullptr, *d_stage_out = nullptr;
@@ -171,18 +174,22 @@ int refresh_panels(spmm_b200_handle *h, cudaStream_t stream);
 // (run_host uploads B band by band on a second stream while earlier passes compute)
 // cfinal: NULL, or where the final rows go instead of vout (the last pass stores them there; earlier passes keep
 // their partial chains in vout)
+// val: a live plan's value array (spmm_b200_run_values); NULL = the handle's value source (d_val, or t_src's on a
+// derived handle). Ignored by a snapshot plan.
 int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t stream,
-                int *launches, const cudaEvent_t *band_ready = nullptr, float *cfinal = nullptr);
+                int *launches, const cudaEvent_t *band_ready = nullptr, float *cfinal = nullptr, const float *val = nullptr);
 int resident_warps(int lanes, int vec, int tune, int block);
 int launch_check_cols(const int *d_idx, long long nnz, int b_rows, int *d_bad, cudaStream_t stream);
 // band_begin[0..n_col_blocks]: first B row of every column block (band_begin[n] = b_rows), at most kMaxSplitBands blocks
 constexpr int kMaxSplitBands = 64;
 int launch_split_rows(const int *d_ptr, const int *d_idx, int num_v, int n_col_blocks, const int *band_begin,
                       int *d_split, int *d_unsorted, cudaStream_t stream);
+// The .y word of a staged entry: the value bits of d_val[i] (live = false), or the position i — perm[i] when perm is
+// non-NULL — (live = true, d_val is not read).
 int launch_build_lpanel(const int4 *d_light_desc, int n_light, int groups, int k4, const int *d_idx, const float *d_val,
-                        int2 *d_lpanel, cudaStream_t stream);
+                        const int *perm, bool live, int2 *d_lpanel, cudaStream_t stream);
 int launch_build_panel(const SegDesc *d_seg, int n_seg, int k4, int pad, const int *d_idx, const float *d_val,
-                       int2 *d_panel, cudaStream_t stream);
+                       const int *perm, bool live, int2 *d_panel, cudaStream_t stream);
 int launch_fill_normal(float *d_dst, long long n, uint64_t seed, uint64_t stream_id, float mean,
                        float stddev, cudaStream_t stream);
 int launch_valid(const float *d_y, const float *d_y2, long long num, unsigned long long *d_count,

@@ -618,6 +618,7 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
     free_plan(p);
     tr.lap("free the previous plan");
     h->plan_select = 0;
+    p.live = h->opt_live_values != 0;
     const int M = h->num_v, K = h->feat;
     const int b_rows = h->b_rows > 0 ? h->b_rows : M;
     if (K == 0 || M == 0) {
@@ -667,17 +668,20 @@ int build_plan(spmm_b200_handle *h, cudaStream_t stream) {
 }
 
 // Stage the {col, val} panels from the caller's idx/val (asynchronous on `stream`): at preprocess, and at refresh_values, as
-// the plan's structure (row order, segments, tasks, slots) depends on ptr only: new edge values need no new plan.
+// the plan's structure (row order, segments, tasks, slots) depends on ptr only: new edge values need no new plan. A live plan
+// stages {col, position} instead — the position in the value source's CSR (t_perm on a derived handle) — and reads no val.
 int refresh_panels(spmm_b200_handle *h, cudaStream_t stream) {
     Plan &p = h->plan;
     if (p.scalar || h->feat == 0 || h->num_v == 0) return 0;   // the scalar kernel reads idx/val at run time
     const int groups = 32 / p.lanes, pad = 4 * groups, k4 = h->feat / 4;
+    const int *perm = p.live && h->t_src ? h->t_perm : nullptr;
     for (BlockPlan &bp : p.blocks) {
         int rc;
         if (bp.n_ltask > 0 &&
-            (rc = launch_build_lpanel(bp.d_light_desc, bp.n_light, groups, k4, h->d_idx, h->d_val, bp.d_lpanel, stream)))
+            (rc = launch_build_lpanel(bp.d_light_desc, bp.n_light, groups, k4, h->d_idx, h->d_val, perm, p.live, bp.d_lpanel, stream)))
             return rc;
-        if (bp.n_seg > 0 && (rc = launch_build_panel(bp.d_seg_desc, bp.n_seg, k4, pad, h->d_idx, h->d_val, bp.d_panel, stream)))
+        if (bp.n_seg > 0 &&
+            (rc = launch_build_panel(bp.d_seg_desc, bp.n_seg, k4, pad, h->d_idx, h->d_val, perm, p.live, bp.d_panel, stream)))
             return rc;
     }
     return 0;

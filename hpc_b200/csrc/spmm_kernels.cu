@@ -125,6 +125,8 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst, const void *src, uint32_
 // L2::evict_last on B rows; gathering B rows into a shared-memory ring with cp.async or with one 1-D TMA copy
 // per row (both ~35 % slower than register gathers on every shape).
 // FULL: every lane's columns are inside the slice (K a multiple of the slice width): no column predicates.
+// LIVE (option "live_values"): a staged entry's .y word is the nonzero's position p and the weight is c.val[p], loaded in
+// the same batch as the entry's B-row gather (both depend on the staged entry alone). Headers and nops load nothing.
 template <int TUNE, int VEC>
 struct Tune {
     static constexpr int kMinBlocks = (TUNE == 0 && VEC == 2) ? 3 : 4;
@@ -174,7 +176,7 @@ __device__ __forceinline__ const int2 *pipe_wait(const Pipe &p, int k) {
 // and one in-order FMA, a nop is padding. Rows never span lane groups, so every row is still one FMA chain in
 // CSR order (bit-exact), but gathers stay in flight across row boundaries and no load depends on a
 // per-row descriptor.
-template <int LANES, int VEC, int TUNE, bool FULL>
+template <int LANES, int VEC, int TUNE, bool FULL, bool LIVE>
 __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs &bd, bool accumulate, bool final, int slice, int2 td,
                                              int lane, const Pipe &pipe) {
     constexpr int GROUPS = 32 / LANES;
@@ -218,11 +220,13 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
         for (int t0 = 0; t0 < n; t0 += GROUPS * U, ep += GROUPS * U) {
             float4 b[U][VEC];
             int2 cv[U];
+            float lw[U];   // LIVE: the weights, defined for nonzero entries only
 #pragma unroll
             for (int u = 0; u < U; ++u) {
                 cv[u] = ep[u * GROUPS];   // in range: a task is padded to a multiple of 4 steps
                 if (cv[u].x >= 0) {
                     const float4 *brow = bbase + (unsigned)cv[u].x;
+                    if (LIVE) lw[u] = ld_stream_f32(c.val + (unsigned)cv[u].y);
 #pragma unroll
                     for (int v = 0; v < VEC; ++v)
                         if (colok[v]) b[u][v] = __ldg(brow + v * LANES);
@@ -235,7 +239,7 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
                 // common case for long rows: nonzeros (and padding) only — straight-line predicated FMAs
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
-                    const float w = __int_as_float(cv[u].y);
+                    const float w = LIVE ? lw[u] : __int_as_float(cv[u].y);
 #pragma unroll
                     for (int v = 0; v < VEC; ++v)
                         if (cv[u].x >= 0 && colok[v]) fma4(acc[v], b[u][v], w);
@@ -244,7 +248,7 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
                     if (cv[u].x >= 0) {
-                        const float w = __int_as_float(cv[u].y);
+                        const float w = LIVE ? lw[u] : __int_as_float(cv[u].y);
 #pragma unroll
                         for (int v = 0; v < VEC; ++v)
                             if (colok[v]) fma4(acc[v], b[u][v], w);   // CSR order within the row: bit-exact chain
@@ -272,7 +276,7 @@ __device__ __forceinline__ void light_stream(const CommonArgs &c, const BandArgs
     flush_row();
 }
 
-template <int LANES, int VEC, int TUNE, bool FULL>
+template <int LANES, int VEC, int TUNE, bool FULL, bool LIVE>
 __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArgs &bd, bool accumulate, bool final, int slice, int seg,
                                               int lane, const Pipe &pipe) {
     constexpr int GROUPS = 32 / LANES;
@@ -313,13 +317,14 @@ __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArg
             for (int u = 0; u < U; ++u) {
                 const int2 cv = e[t0 + u * GROUPS + g];   // in range: the span is padded to whole batches
                 ok[u] = cv.x >= 0;                        // nop entries are {-1, 0}
-                wt[u] = __int_as_float(cv.y);
                 // a nop gathers row 0 (always a valid address) and is ignored below: every b[u][v] is defined in every
                 // iteration, which keeps the register allocator from carrying the batch across iterations
                 const float4 *brow = bbase + (ok[u] ? (unsigned)cv.x : 0u);
 #pragma unroll
                 for (int v = 0; v < VEC; ++v)
                     if (colok[v]) b[u][v] = __ldg(brow + v * LANES);
+                if (LIVE) wt[u] = ok[u] ? ld_stream_f32(c.val + (unsigned)cv.y) : 0.f;   // a nop loads nothing
+                else wt[u] = __int_as_float(cv.y);
             }
 #pragma unroll
             for (int u = 0; u < U; ++u) {
@@ -385,7 +390,7 @@ __device__ __forceinline__ void heavy_segment(const CommonArgs &c, const BandArg
     }
 }
 
-template <int LANES, int VEC, int TUNE, bool FULL>
+template <int LANES, int VEC, int TUNE, bool FULL, bool LIVE>
 __global__ void __launch_bounds__(256, Tune<TUNE, VEC>::kMinBlocks) spmm_kernel(const __grid_constant__ RunArgs a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int warp = threadIdx.x >> 5;
@@ -399,11 +404,12 @@ __global__ void __launch_bounds__(256, Tune<TUNE, VEC>::kMinBlocks) spmm_kernel(
     const Pipe pipe = {reinterpret_cast<int2 *>(smem_raw) + (size_t)warp * kStages * kChunk,
                        reinterpret_cast<uint64_t *>(smem_raw + (size_t)nwarps * kStages * kChunk * sizeof(int2)) + warp * kStages};
     pipe_init(pipe, lane);
-    if (td.x < 0) heavy_segment<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, -1 - td.x, lane, pipe);
-    else light_stream<LANES, VEC, TUNE, FULL>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, td, lane, pipe);
+    if (td.x < 0) heavy_segment<LANES, VEC, TUNE, FULL, LIVE>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, -1 - td.x, lane, pipe);
+    else light_stream<LANES, VEC, TUNE, FULL, LIVE>(a.c, a.b, a.b.accumulate != 0, a.b.final != 0, slice, td, lane, pipe);
 }
 
-// K % 4 != 0: scalar lanes over the feature columns, one warp per row, same in-order chain.
+// K % 4 != 0: scalar lanes over the feature columns, one warp per row, same in-order chain. It reads idx/val at run time;
+// with live values on a derived handle the weight of position i is val[perm[i]].
 __global__ void __launch_bounds__(256) spmm_scalar_kernel(const __grid_constant__ RunArgs ra) {
     const CommonArgs &a = ra.c;
     const int lane = threadIdx.x & 31;
@@ -419,8 +425,9 @@ __global__ void __launch_bounds__(256) spmm_scalar_kernel(const __grid_constant_
             int c = 0;
             float w = 0.f;
             if (base + lane < deg) {
-                c = ld_stream_s32(a.idx + begin + base + lane);
-                w = ld_stream_f32(a.val + begin + base + lane);
+                const int i = begin + base + lane;
+                c = ld_stream_s32(a.idx + i);
+                w = ld_stream_f32(a.val + (a.perm ? ld_stream_s32(a.perm + i) : i));
             }
             const int n = min(32, deg - base);
             for (int t = 0; t < n; ++t) {
@@ -479,21 +486,28 @@ __global__ void __launch_bounds__(256) check_cols_kernel(const int *idx, long lo
     if (__any_sync(kFull, any) && (threadIdx.x & 31) == 0) atomicExch(bad, 1);
 }
 
+// The .y word of the staged entry of CSR position i: the value bits, or (live values) the position the run reads its
+// weight from — i itself, or perm[i] on a derived handle (a position in the source handle's CSR).
+__device__ __forceinline__ int staged_word(int i, const float *val, const int *perm, bool live) {
+    return live ? (perm ? perm[i] : i) : __float_as_int(val[i]);
+}
+
 // one warp per light row: header at its slot, nonzeros at stride `groups` after it (the panel was preset to nops)
 __global__ void __launch_bounds__(256) build_lpanel_kernel(const int4 *light_desc, int n_light, int groups, int k4,
-                                                           const int *idx, const float *val, int2 *lpanel) {
+                                                           const int *idx, const float *val, const int *perm, bool live,
+                                                           int2 *lpanel) {
     const long long gw = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (gw >= n_light) return;
     const int4 d = light_desc[gw];   // {row, begin, deg, dst}
     if (lane == 0) lpanel[d.w] = make_int2((int)(0x80000000u | (unsigned)d.x), 0);
     for (int t = lane; t < d.z; t += 32)
-        lpanel[(size_t)d.w + (size_t)(1 + t) * groups] = make_int2(idx[d.y + t] * k4, __float_as_int(val[d.y + t]));
+        lpanel[(size_t)d.w + (size_t)(1 + t) * groups] = make_int2(idx[d.y + t] * k4, staged_word(d.y + t, val, perm, live));
 }
 
 // one warp per segment: gather its {col * k4, val} pairs into the panel, nop entries in the padding
 __global__ void __launch_bounds__(256) build_panel_kernel(const SegDesc *seg, int n_seg, int k4, int pad, const int *idx,
-                                                          const float *val, int2 *panel) {
+                                                          const float *val, const int *perm, bool live, int2 *panel) {
     const long long gw = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (gw >= n_seg) return;
@@ -501,7 +515,7 @@ __global__ void __launch_bounds__(256) build_panel_kernel(const SegDesc *seg, in
     const int padded = (d.len + pad - 1) / pad * pad;
     for (int t = lane; t < padded; t += 32) {
         int2 e = make_int2(-1, 0);
-        if (t < d.len) e = make_int2(idx[d.nnz_begin + t] * k4, __float_as_int(val[d.nnz_begin + t]));
+        if (t < d.len) e = make_int2(idx[d.nnz_begin + t] * k4, staged_word(d.nnz_begin + t, val, perm, live));
         panel[(size_t)d.panel_off + t] = e;
     }
 }
@@ -545,33 +559,39 @@ __global__ void __launch_bounds__(256) valid_kernel(const float *y, const float 
 // per warp: kStages chunks + their mbarriers
 size_t task_smem(int block) { return (size_t)(block / 32) * kStages * (kChunk * sizeof(int2) + sizeof(uint64_t)); }
 
-template <int LANES, int VEC, int TUNE, bool FULL>
+template <int LANES, int VEC, int TUNE, bool FULL, bool LIVE>
 void launch_tuned(const RunArgs &a, int block, cudaStream_t stream) {
     const int warps = block / 32;
     const long long tasks = (long long)a.b.n_utask * a.c.n_slices;
-    spmm_kernel<LANES, VEC, TUNE, FULL><<<(unsigned)((tasks + warps - 1) / warps), block, task_smem(block), stream>>>(a);
+    spmm_kernel<LANES, VEC, TUNE, FULL, LIVE><<<(unsigned)((tasks + warps - 1) / warps), block, task_smem(block), stream>>>(a);
+}
+
+template <int LANES, int VEC, bool LIVE>
+void launch_shape(const RunArgs &a, int block, int tune, bool full, cudaStream_t stream) {
+    if (tune == 1) {
+        if (full) launch_tuned<LANES, VEC, 1, true, LIVE>(a, block, stream);
+        else launch_tuned<LANES, VEC, 1, false, LIVE>(a, block, stream);
+    } else {
+        if (full) launch_tuned<LANES, VEC, 0, true, LIVE>(a, block, stream);
+        else launch_tuned<LANES, VEC, 0, false, LIVE>(a, block, stream);
+    }
 }
 
 template <int LANES, int VEC>
-void launch_shape(const RunArgs &a, int block, int tune, bool full, cudaStream_t stream) {
-    if (tune == 1) {
-        if (full) launch_tuned<LANES, VEC, 1, true>(a, block, stream);
-        else launch_tuned<LANES, VEC, 1, false>(a, block, stream);
-    } else {
-        if (full) launch_tuned<LANES, VEC, 0, true>(a, block, stream);
-        else launch_tuned<LANES, VEC, 0, false>(a, block, stream);
-    }
+void launch_shape(const RunArgs &a, const Plan &p, bool full, cudaStream_t stream) {
+    if (p.live) launch_shape<LANES, VEC, true>(a, p.block, p.tune, full, stream);
+    else launch_shape<LANES, VEC, false>(a, p.block, p.tune, full, stream);
 }
 
 int launch_lanes(const Plan &p, const RunArgs &a, bool full, cudaStream_t stream) {
     switch (p.lanes * 10 + p.vec) {
-        case 11: launch_shape<1, 1>(a, p.block, p.tune, full, stream); break;
-        case 21: launch_shape<2, 1>(a, p.block, p.tune, full, stream); break;
-        case 41: launch_shape<4, 1>(a, p.block, p.tune, full, stream); break;
-        case 81: launch_shape<8, 1>(a, p.block, p.tune, full, stream); break;
-        case 161: launch_shape<16, 1>(a, p.block, p.tune, full, stream); break;
-        case 321: launch_shape<32, 1>(a, p.block, p.tune, full, stream); break;
-        case 322: launch_shape<32, 2>(a, p.block, p.tune, full, stream); break;
+        case 11: launch_shape<1, 1>(a, p, full, stream); break;
+        case 21: launch_shape<2, 1>(a, p, full, stream); break;
+        case 41: launch_shape<4, 1>(a, p, full, stream); break;
+        case 81: launch_shape<8, 1>(a, p, full, stream); break;
+        case 161: launch_shape<16, 1>(a, p, full, stream); break;
+        case 321: launch_shape<32, 1>(a, p, full, stream); break;
+        case 322: launch_shape<32, 2>(a, p, full, stream); break;
         default:
             set_error("unsupported kernel shape lanes=%d vec=%d", p.lanes, p.vec);
             return SPMM_B200_EINVAL;
@@ -583,8 +603,9 @@ template <int LANES, int VEC>
 int slots_shape(int block, int tune) {
     int nb = 0;
     const size_t smem = task_smem(block);
-    const cudaError_t e = tune == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 1, true>, block, smem)
-                                    : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 0, true>, block, smem);
+    // the LIVE instances keep the same register caps (DESIGN.md §3), so the snapshot kernel's occupancy stands for both
+    const cudaError_t e = tune == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 1, true, false>, block, smem)
+                                    : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, spmm_kernel<LANES, VEC, 0, true, false>, block, smem);
     if (e != cudaSuccess) {
         cudaGetLastError();
         return 0;
@@ -605,10 +626,15 @@ int ctas_per_sm(int lanes, int vec, int tune, int block) {
     }
 }
 
-void fill_common(CommonArgs &c, const spmm_b200_handle *h, const float *vin, float *vout, float *cfinal) {
+void fill_common(CommonArgs &c, const spmm_b200_handle *h, const float *vin, float *vout, float *cfinal, const float *val) {
     const Plan &p = h->plan;
     c.idx = h->d_idx;
     c.val = h->d_val;
+    c.perm = nullptr;
+    if (p.live) {   // positions index the value source: the handle's own CSR, or the source's on a derived handle
+        c.val = val ? val : h->t_src ? h->t_src->d_val : h->d_val;
+        c.perm = h->t_src ? h->t_perm : nullptr;
+    }
     c.vin = vin;
     c.vout = vout;
     c.cfinal = cfinal ? cfinal : vout;
@@ -641,7 +667,7 @@ void fill_band(BandArgs &b, const Plan &p, int blk) {
 }  // namespace
 
 int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t stream,
-                int *launches, const cudaEvent_t *band_ready, float *cfinal) {
+                int *launches, const cudaEvent_t *band_ready, float *cfinal, const float *val) {
     const Plan &p = h->plan;
     *launches = 0;
     if (h->num_v == 0 || h->feat == 0) return 0;
@@ -668,7 +694,7 @@ int launch_spmm(spmm_b200_handle *h, const float *vin, float *vout, cudaStream_t
         }
         if (bp.n_light == 0 && bp.n_seg == 0) continue;
         RunArgs a;
-        fill_common(a.c, h, vin, vout, cfinal);
+        fill_common(a.c, h, vin, vout, cfinal, val);
         fill_band(a.b, p, blk);
         if (p.scalar) {
             const int warps = p.block / 32;
@@ -733,21 +759,21 @@ int launch_split_rows(const int *d_ptr, const int *d_idx, int num_v, int n_col_b
 }
 
 int launch_build_lpanel(const int4 *d_light_desc, int n_light, int groups, int k4, const int *d_idx, const float *d_val,
-                        int2 *d_lpanel, cudaStream_t stream) {
+                        const int *perm, bool live, int2 *d_lpanel, cudaStream_t stream) {
     if (n_light == 0) return 0;
     const long long threads = (long long)n_light * 32;
     build_lpanel_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(d_light_desc, n_light, groups, k4, d_idx,
-                                                                              d_val, d_lpanel);
+                                                                              d_val, perm, live, d_lpanel);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
 
 int launch_build_panel(const SegDesc *d_seg, int n_seg, int k4, int pad, const int *d_idx, const float *d_val,
-                       int2 *d_panel, cudaStream_t stream) {
+                       const int *perm, bool live, int2 *d_panel, cudaStream_t stream) {
     if (n_seg == 0) return 0;
     const long long threads = (long long)n_seg * 32;
-    build_panel_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(d_seg, n_seg, k4, pad, d_idx, d_val,
-                                                                             d_panel);
+    build_panel_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(d_seg, n_seg, k4, pad, d_idx, d_val, perm,
+                                                                             live, d_panel);
     SB_CUDA(cudaGetLastError());
     return 0;
 }

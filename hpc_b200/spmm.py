@@ -143,6 +143,14 @@ class SpMMB200(SpMM):
         self._check_io(vin, vout)
         check(lib.spmm_b200_run(self._h, _ptr(vin), _ptr(vout), _stream()))
 
+    def run_values(self, val, vin, vout) -> None:
+        """run with the edge values `val` (spmm_b200_run_values): C = A_val·B, val[p] the value of the nonzero at CSR
+        position p — on an operator from transposed() / column_sorted(), a position of the source operator, whose num_e
+        values val holds. Needs the option live_values=1. Asynchronous on the current stream."""
+        self._check_io(vin, vout)
+        self._check_dense("val", val, self.num_e)
+        check(lib.spmm_b200_run_values(self._h, _ptr(val), _ptr(vin), _ptr(vout), _stream()))
+
     def sddmm(self, x_row, x_col, out) -> None:
         """SDDMM over this operator's pattern (spmm_b200_sddmm): out[e] = <x_row[row(e)], x_col[idx[e]]> for every
         nonzero e, in CSR position order. x_row: num_v x feat_in, x_col: b_rows x feat_in, out: >= num_e floats.

@@ -64,6 +64,11 @@ int spmm_b200_set_feat(spmm_b200_t h, int feat_in);
  *   "zero_copy" run_host / run_host_sharded: 1 (default) = when the output buffer is pinned host memory the last pass
  *               stores final rows straight into it (no separate device-to-host copy), 0 = always copy
  *   "tune"      measured kernel variant, 0 (default) or 1, see hpc_b200/csrc/spmm_kernels.cu
+ *   "live_values" 0 (default) = the plan stages the edge values (SNAPSHOT, see preprocess); 1 = the plan stages each
+ *               nonzero's position instead and every run reads the weights at run time from a value array
+ *               (spmm_b200_run_values). On a handle from create_transposed / create_column_sorted the positions are
+ *               those of the source handle's CSR, so one value array drives both. Part of the plan: changing it
+ *               invalidates the plan
  *   "b_rows"    rows of B when A is a row block of a larger graph (0 = num_v). Part of the plan (column bounds
  *               check, 32-bit offset guard, column-block bands, run_host's copy of B): changing it after
  *               preprocess invalidates the plan
@@ -80,12 +85,14 @@ int spmm_b200_set_option(spmm_b200_t h, const char *name, long long value);
  * copy — unlike the reference's SpMMOpt::run, which reads idx/val at run time (PA4/workspace/src/spmm_opt.cu:22-25).
  * A caller that rewrites d_val in place afterwards (or d_idx, if the plan has a single column block and no row changes
  * its length) must call spmm_b200_refresh_values before the next run; any other change of the structure needs a new
- * preprocess. */
+ * preprocess. With option live_values = 1 run, run_host and run_host_sharded instead read the values at run time, as
+ * the reference does: d_val, or on a derived handle the source handle's d_val (refresh_values is then needed only after
+ * d_idx changes). */
 int spmm_b200_preprocess(spmm_b200_t h, const float *vin, float *vout, void *stream);
 
 /* Re-stages the plan's {col, val} panels from the caller's current d_idx / d_val (same ptr), asynchronously on
  * `stream`: two small kernels per column block, no host work, no new plan (GNN edge re-weighting between layers).
- * No reference counterpart (the reference reads idx/val live). */
+ * No reference counterpart (the reference reads idx/val live). On a live_values plan it re-stages idx and the positions. */
 int spmm_b200_refresh_values(spmm_b200_t h, void *stream);
 
 /* SpMM::run(float *vin, float *vout)  (spmm_base.h:32; PA4/handout/src/spmm_ref.cu:27-30).
@@ -96,6 +103,16 @@ int spmm_b200_refresh_values(spmm_b200_t h, void *stream);
  * joined back to `stream` by events inside the call: to the caller everything is ordered on `stream` (also under
  * CUDA-graph capture). */
 int spmm_b200_run(spmm_b200_t h, const float *vin, float *vout, void *stream);
+
+/* C = A_val * B: run with the edge values of this call (no reference counterpart; DGL's u_mul_e_sum). val[p] is the
+ * value of the nonzero at CSR position p, a device array of num_e floats — on a handle from create_transposed /
+ * create_column_sorted, p is a position in the SOURCE handle's CSR and val holds the source's num_e floats. Needs a
+ * plan built with option live_values = 1 (SPMM_B200_ESTATE otherwise, and without preprocess); val == NULL while
+ * num_e > 0: SPMM_B200_EINVAL. Everything else is run's: asynchronous on `stream`, fully overwrites vout, column
+ * blocks, two-stream launches, the stacked-layer epilogue and the alignment rules; capturable into a CUDA graph (the
+ * graph reads val's contents at replay). The bits equal those of a snapshot plan with the same options after its
+ * values are set to val and refreshed. */
+int spmm_b200_run_values(spmm_b200_t h, const float *val, const float *vin, float *vout, void *stream);
 
 /* run, plus the device time of its kernel in milliseconds (CUDA events on `stream` around the
  * launch). Synchronises. Counterpart of getCUDATime (PA4/handout/include/util.h:131-139). */

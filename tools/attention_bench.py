@@ -8,8 +8,8 @@ For each workload:
     flushed (256 MiB write outside the event pair) before every call when the working set is below 2x L2. Bytes:
     forward 8 nnz + 4 (M+1), backward 12 nnz + 4 (M+1), copy 8 nnz.
   - one GraphAttention forward + backward step, phase by phase (the calls the module makes, each between events):
-    sddmm, softmax, staging (value copy + refresh_values), runs (forward and transposed operator); and the same step
-    through the module and autograd, timed as a whole.
+    sddmm, softmax, runs (run_values on the forward and the transposed operator); and the same step through the module
+    and autograd, timed as a whole.
   - the timed softmax outputs against the CPU restatement on a seeded sample of rows (bit for bit).
   - the device name and power limit, read in the same process.
 With --out, line i is also written to DIR/r04_attention_<workload>.json.
@@ -110,18 +110,12 @@ def bench(name, steps):
     # one attention step, phase by phase: the calls GraphAttention makes
     out, dout = torch.empty(M, K, device=dev), w
     dalpha, dq, dk, dv = torch.empty(nnz, device=dev), torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
-    val = att._val
-
-    def stage(x, o):
-        val.copy_(x)
-        o.refresh_values()
-
     phases = [("sddmm", lambda: op.sddmm(q, k, s)), ("softmax", lambda: op.edge_softmax(s, p)),
-              ("staging", lambda: stage(p, op)), ("runs", lambda: op.run(v, out)),
-              ("sddmm", lambda: op.sddmm(dout, v, dalpha)), ("staging", lambda: stage(p, t)),
-              ("runs", lambda: t.run(dout, dv)), ("softmax", lambda: op.edge_softmax_backward(p, dalpha, ds)),
-              ("staging", lambda: stage(ds, op)), ("runs", lambda: op.run(k, dq)),
-              ("staging", lambda: stage(ds, t)), ("runs", lambda: t.run(q, dk))]
+              ("runs", lambda: op.run_values(p, v, out)),
+              ("sddmm", lambda: op.sddmm(dout, v, dalpha)),
+              ("runs", lambda: t.run_values(p, dout, dv)), ("softmax", lambda: op.edge_softmax_backward(p, dalpha, ds)),
+              ("runs", lambda: op.run_values(ds, k, dq)),
+              ("runs", lambda: t.run_values(ds, q, dk))]
     for _, fn in phases:
         fn()
     torch.cuda.synchronize()
