@@ -66,7 +66,55 @@ class _GraphSpMMReduceFn(torch.autograd.Function):
 REDUCTIONS = ("sum", "mean", "amax", "amin")
 
 
-class GraphSpMM:
+class _Operators:
+    """What GraphSpMM and GraphAttention share: the forward operator over g, planned on first use, and the operator over
+    Aᵀ, created on first use and planned when the module runs on it. Plans live in the library's pool; close() releases
+    both operators."""
+
+    def __init__(self, g: CSR, feat_in: int, shared: dict, **options):
+        """shared: the options of both operators; options: those of the forward one alone."""
+        self.g = g
+        self.feat_in = int(feat_in)
+        self.op = SpMMB200(g, self.feat_in, **shared, **options)
+        self._shared = shared
+        self._t = None
+        self._planned = False
+
+    def _runs(self) -> bool:
+        """Whether the module runs its operators (run / run_values, which need a plan on the transposed one too)."""
+        return True
+
+    def _op(self) -> SpMMB200:
+        """The forward operator, planned on first use."""
+        if not self._planned:
+            self.op._plan()
+            self._planned = True
+        return self.op
+
+    def transposed(self) -> SpMMB200:
+        """The operator over Aᵀ (created on first use; planned when the module runs on it). On a live-value module its
+        run_values takes edge values in g's CSR positions."""
+        if self._t is None:
+            self._t = self.op.transposed(self.feat_in, **self._shared)
+            if self._runs():
+                self._t._plan()
+        return self._t
+
+    def close(self) -> None:
+        """Releases the transposed operator, then the forward one."""
+        if self._t is not None:
+            self._t.close()
+            self._t = None
+        self.op.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:   # interpreter shutdown: the library may already be gone
+            pass
+
+
+class GraphSpMM(_Operators):
     """C = A·B for the CSR `g` (num_v x b_rows) and a dense B (b_rows x feat_in), differentiable in B and in g.val.
 
     reduce (torch.sparse.mm's names): "sum" (default), "mean" (the sum over the row's nonzero count; empty rows give 0),
@@ -81,39 +129,23 @@ class GraphSpMM:
     def __init__(self, g: CSR, feat_in: int, reduce: str = "sum", **options):
         if reduce not in REDUCTIONS:
             raise ValueError(f"reduce must be one of {REDUCTIONS}, got {reduce!r}")
-        self.g = g
-        self.feat_in = int(feat_in)
+        super().__init__(g, feat_in, {}, **options)
         self.reduce = reduce
-        self.op = SpMMB200(g, self.feat_in, **options)
-        self._t = None
         self._staged = None
-        self._prepared = False
         self._deg = None
 
-    def _staged_values(self) -> bool:
-        """run reads the plan's copy of the values; reduce / reduce_backward read g.val itself."""
+    def _runs(self) -> bool:
+        """run reads the plan's copy of the values; reduce / reduce_backward read g.val itself, and reduce_backward
+        needs no plan."""
         return self.reduce in ("sum", "mean")
 
-    def transposed(self) -> SpMMB200:
-        """The operator over Aᵀ (created on first use; planned when its run is needed)."""
-        if self._t is None:
-            self._t = self.op.transposed(self.feat_in)
-            if self._staged_values():
-                dc = torch.empty((self.op.num_v, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
-                db = torch.empty((self.op.b_rows, self.feat_in), dtype=torch.float32, device=self.g.ptr.device)
-                self._t.preprocess(dc, db)
-        return self._t
-
-    def _stage(self, b: torch.Tensor) -> None:
+    def _stage(self) -> None:
         version = self.g.val._version
-        if not self._prepared:
-            c = torch.empty((self.g.num_v, self.feat_in), dtype=torch.float32, device=b.device)
-            self.op.preprocess(b, c)
-            self._prepared = True
-        elif version != self._staged and self._staged_values():
+        if self._planned and version != self._staged and self._runs():
             self.op.refresh_values()
             if self._t is not None:
                 self._t.refresh_values()
+        self._op()
         self._staged = version
 
     def _degrees(self) -> torch.Tensor:
@@ -127,24 +159,11 @@ class GraphSpMM:
         if b.dtype != torch.float32 or not b.is_cuda or b.shape != (self.op.b_rows, self.feat_in):
             raise ValueError(f"B: need a CUDA float32 tensor of shape ({self.op.b_rows}, {self.feat_in})")
         b = b.contiguous()
-        self._stage(b)
+        self._stage()
         if self.reduce in ("amax", "amin"):
             return _GraphSpMMReduceFn.apply(self, b, self.g.val)
         c = _GraphSpMMFn.apply(self, b, self.g.val)
         return c / self._degrees() if self.reduce == "mean" else c
-
-    def close(self) -> None:
-        """Releases the transposed operator, then the forward one."""
-        if self._t is not None:
-            self._t.close()
-            self._t = None
-        self.op.close()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:   # interpreter shutdown: the library may already be gone
-            pass
 
 
 class _ScoresFn(torch.autograd.Function):
@@ -212,7 +231,7 @@ class _AggregateFn(torch.autograd.Function):
         return None, dalpha, dv
 
 
-class GraphAttention:
+class GraphAttention(_Operators):
     """Dot-product attention over the CSR pattern of `g` (num_v x b_rows): out = softmax_row(<q_r, k_c>)·v, with
     q: num_v x feat_in, k and v: b_rows x feat_in (CUDA float32). Differentiable in q, k and v, and through the separate
     steps scores / softmax / aggregate (e.g. GAT scores built in torch, then softmax and aggregate). The caller scales q.
@@ -224,33 +243,7 @@ class GraphAttention:
     when a gradient first needs it. Call close() when done (or rely on garbage collection)."""
 
     def __init__(self, g: CSR, feat_in: int, **options):
-        self.g = g
-        self.feat_in = int(feat_in)
-        self.op = SpMMB200(g, self.feat_in, live_values=1, **options)
-        self._t = None
-        self._prepared = False
-
-    def _op(self) -> SpMMB200:
-        """The forward operator, planned on first use."""
-        if not self._prepared:
-            dev = self.g.ptr.device
-            b = torch.empty((self.op.b_rows, self.feat_in), dtype=torch.float32, device=dev)
-            c = torch.empty((self.g.num_v, self.feat_in), dtype=torch.float32, device=dev)
-            self.op.preprocess(b, c)
-            self._prepared = True
-        return self.op
-
-    def transposed(self) -> SpMMB200:
-        """The operator over the pattern's transpose (created and planned on first use); run_values on it takes edge
-        values in g's CSR positions."""
-        if self._t is None:
-            op = self._op()
-            self._t = op.transposed(self.feat_in, live_values=1)
-            dev = self.g.ptr.device
-            dc = torch.empty((op.num_v, self.feat_in), dtype=torch.float32, device=dev)
-            db = torch.empty((op.b_rows, self.feat_in), dtype=torch.float32, device=dev)
-            self._t.preprocess(dc, db)
-        return self._t
+        super().__init__(g, feat_in, {"live_values": 1}, **options)
 
     def _dense(self, name, t, rows):
         if not isinstance(t, torch.Tensor) or t.dtype != torch.float32 or not t.is_cuda or t.shape != (rows, self.feat_in):
@@ -280,16 +273,3 @@ class GraphAttention:
 
     def __call__(self, q: torch.Tensor, k: torch.Tensor, v: torch.Tensor) -> torch.Tensor:
         return self.aggregate(self.softmax(self.scores(q, k)), v)
-
-    def close(self) -> None:
-        """Releases the transposed operator, then the forward one."""
-        if self._t is not None:
-            self._t.close()
-            self._t = None
-        self.op.close()
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:   # interpreter shutdown: the library may already be gone
-            pass

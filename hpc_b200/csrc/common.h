@@ -228,6 +228,14 @@ inline int sm_count() {
     return sms;
 }
 
+// Grid of a grid-stride support kernel of 256-thread blocks over n elements: one block per 256, at most 16 per SM of the
+// current device (148 SMs, a B200's, when it cannot be queried), at least 1.
+inline int stride_grid(long long n) {
+    const int sms = sm_count();
+    const long long cap = 16ll * (sms > 0 ? sms : 148), blocks = (n + 255) / 256;
+    return (int)(blocks < 1 ? 1 : blocks < cap ? blocks : cap);
+}
+
 // Lanes per row slice of q units (float4 or columns): the power of two >= q, at most 32. This is the L of sddmm's
 // summation order (sddmm.cu), which reduce_backward's dval (reduce.cu) must follow bit for bit.
 inline int pow2_lanes(int q) {

@@ -727,17 +727,9 @@ int resident_warps(int lanes, int vec, int tune, int block) {
     return ctas_per_sm(lanes, vec, tune, block) * (block / 32) * sm_count();
 }
 
-// grid cap for the grid-stride support kernels: 16 CTAs per SM of the current device
-static long long stride_grid_cap() {
-    const int sms = sm_count();
-    return 16ll * (sms > 0 ? sms : 148);   // 148: B200
-}
-
 int launch_check_cols(const int *d_idx, long long nnz, int b_rows, int *d_bad, cudaStream_t stream) {
     if (nnz == 0) return 0;
-    const long long blocks = (nnz + 255) / 256;
-    const long long cap = stride_grid_cap();
-    check_cols_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(d_idx, nnz, b_rows, d_bad);
+    check_cols_kernel<<<stride_grid(nnz), 256, 0, stream>>>(d_idx, nnz, b_rows, d_bad);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -790,9 +782,7 @@ int launch_fill_normal(float *d_dst, long long n, uint64_t seed, uint64_t stream
     };
     const uint64_t key = hmix(seed ^ hmix(stream_id * 0x632BE59BD9B4E019ull + 0x1234567ull));
     const float scale = (float)((double)stddev / 53510.0);
-    const long long blocks = (n + 255) / 256;
-    const long long cap = stride_grid_cap();
-    fill_normal_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(d_dst, n, key, scale, mean);
+    fill_normal_kernel<<<stride_grid(n), 256, 0, stream>>>(d_dst, n, key, scale, mean);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -800,9 +790,7 @@ int launch_fill_normal(float *d_dst, long long n, uint64_t seed, uint64_t stream
 int launch_valid(const float *d_y, const float *d_y2, long long num, unsigned long long *d_count,
                  cudaStream_t stream) {
     if (num <= 0) return 0;
-    const long long blocks = (num + 255) / 256;
-    const long long cap = stride_grid_cap();
-    valid_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, stream>>>(d_y, d_y2, num, d_count);
+    valid_kernel<<<stride_grid(num), 256, 0, stream>>>(d_y, d_y2, num, d_count);
     SB_CUDA(cudaGetLastError());
     return 0;
 }

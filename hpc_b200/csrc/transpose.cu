@@ -58,12 +58,72 @@ __global__ void __launch_bounds__(256) gather_t_kernel(const int *perm, const in
     }
 }
 
-int grid_for(long long n) {
-    int sms = sm_count();
-    if (sms <= 0) sms = 148;
-    long long blocks = (n + 255) / 256;
-    if (blocks > 16ll * sms) blocks = 16ll * sms;
-    return (int)(blocks < 1 ? 1 : blocks);
+// Radix key bits that cover [0, n): at least 1, at most 31.
+int key_bits(long long n) {
+    int bits = 1;
+    while (bits < 31 && (1ll << bits) < n) ++bits;
+    return bits;
+}
+
+// Pool blocks (pool.cu) that one construction borrows, stream-ordered on `s`; create_derived frees them however it ends.
+struct Scratch {
+    cudaStream_t s;
+    void *p[5] = {};   // the most one construction borrows (the transposed one)
+    int n = 0;
+    template <class T>
+    cudaError_t alloc(T **ptr, size_t bytes) {
+        const cudaError_t e = pool_alloc((void **)ptr, bytes, s);
+        if (e == cudaSuccess) p[n++] = *ptr;
+        return e;
+    }
+    void drop() {
+        for (int i = 0; i < n; ++i) pool_free(p[i], s);
+    }
+};
+
+// What the transposed and the column-sorted handle share: the argument check, a new handle whose t_idx / t_val / t_perm
+// (max(1, nnz) each) come from the current device's pool, one failure path that leaves no handle and no scratch behind,
+// and the synchronise before the handle is returned. build(t, scratch) queues the rest on the stream and sets t's d_ptr,
+// num_v and b_rows; it returns 0 or a status code.
+template <class Build>
+int create_derived(spmm_b200_handle *h, int feat_in, void *stream, spmm_b200_t *out, const char *who, Build build) {
+    if (!h || !out || feat_in < 0) {
+        set_error("%s: bad arguments", who);
+        return SPMM_B200_EINVAL;
+    }
+    spmm_b200_handle *t = new (std::nothrow) spmm_b200_handle();
+    if (!t) {
+        set_error("%s: out of host memory", who);
+        return SPMM_B200_ENOMEM;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    Scratch scratch{s};
+    const int rc = [&]() {
+        const size_t cnt = (size_t)std::max<long long>(1, h->num_e);
+        SB_CUDA(cudaGetDevice(&t->t_device));
+        SB_CUDA(pool_alloc((void **)&t->t_idx, sizeof(int) * cnt, s));
+        SB_CUDA(pool_alloc((void **)&t->t_val, sizeof(float) * cnt, s));
+        SB_CUDA(pool_alloc((void **)&t->t_perm, sizeof(int) * cnt, s));
+        const int rc = build(t, scratch);
+        if (rc) return rc;
+        SB_CUDA(cudaStreamSynchronize(s));
+        return 0;
+    }();
+    if (rc) {
+        cudaStreamSynchronize(s);   // whatever was queued may still read the scratch
+        cudaGetLastError();
+        scratch.drop();
+        spmm_b200_destroy(t);
+        return rc;
+    }
+    scratch.drop();
+    t->d_idx = t->t_idx;
+    t->d_val = t->t_val;
+    t->num_e = h->num_e;
+    t->feat = feat_in;
+    t->t_src = h;
+    *out = t;
+    return 0;
 }
 
 }  // namespace
@@ -71,7 +131,7 @@ int grid_for(long long n) {
 // values of the transposed CSR from the source handle's current val (spmm_b200_refresh_values on a transposed handle)
 int regather_transposed_values(spmm_b200_handle *t, cudaStream_t stream) {
     if (!t->t_src || t->num_e == 0) return 0;
-    gather_t_kernel<<<grid_for(t->num_e), 256, 0, stream>>>(t->t_perm, nullptr, t->t_src->d_val, t->num_e, nullptr, t->t_val);
+    gather_t_kernel<<<stride_grid(t->num_e), 256, 0, stream>>>(t->t_perm, nullptr, t->t_src->d_val, t->num_e, nullptr, t->t_val);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -81,93 +141,50 @@ int regather_transposed_values(spmm_b200_handle *t, cudaStream_t stream) {
 using namespace spmm_b200;
 
 extern "C" int spmm_b200_create_transposed(spmm_b200_t h, int feat_in, void *stream, spmm_b200_t *out) {
-    if (!h || !out || feat_in < 0) {
-        set_error("spmm_b200_create_transposed: bad arguments");
-        return SPMM_B200_EINVAL;
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    const int rows_t = h->b_rows > 0 ? h->b_rows : h->num_v;   // rows of A^T = columns of A = rows of B
-    const long long nnz = h->num_e;
-    spmm_b200_handle *t = new (std::nothrow) spmm_b200_handle();
-    if (!t) {
-        set_error("spmm_b200_create_transposed: out of host memory");
-        return SPMM_B200_ENOMEM;
-    }
-    int *row_of = nullptr, *pos = nullptr, *keys_out = nullptr, *bad = nullptr;
-    void *tmp = nullptr;
-    // scratch and the new CSR come from the library's pool (pool.cu), stream-ordered on `s`
-    auto drop_scratch = [&]() {
-        pool_free(row_of, s);
-        pool_free(pos, s);
-        pool_free(keys_out, s);
-        pool_free(tmp, s);
-        pool_free(bad, s);
-    };
-    auto fail = [&](int rc) {
-        cudaStreamSynchronize(s);   // whatever was queued may still read the scratch
-        cudaGetLastError();
-        drop_scratch();
-        spmm_b200_destroy(t);
-        return rc;
-    };
-#define TR_CUDA(call)                                                                    \
-    do {                                                                                 \
-        cudaError_t e__ = (call);                                                        \
-        if (e__ != cudaSuccess) return fail(cuda_fail(e__, #call, __FILE__, __LINE__)); \
-    } while (0)
-    TR_CUDA(cudaGetDevice(&t->t_device));
-    TR_CUDA(pool_alloc((void **)&t->t_ptr, sizeof(int) * ((size_t)rows_t + 1), s));
-    TR_CUDA(pool_alloc((void **)&t->t_idx, sizeof(int) * (size_t)std::max<long long>(1, nnz), s));
-    TR_CUDA(pool_alloc((void **)&t->t_val, sizeof(float) * (size_t)std::max<long long>(1, nnz), s));
-    TR_CUDA(pool_alloc((void **)&t->t_perm, sizeof(int) * (size_t)std::max<long long>(1, nnz), s));
-    TR_CUDA(cudaMemsetAsync(t->t_ptr, 0, sizeof(int) * ((size_t)rows_t + 1), s));
-    if (nnz > 0) {
+    return create_derived(h, feat_in, stream, out, "spmm_b200_create_transposed", [&](spmm_b200_handle *t, Scratch &scratch) {
+        cudaStream_t s = scratch.s;
+        const int rows_t = h->b_rows > 0 ? h->b_rows : h->num_v;   // rows of A^T = columns of A = rows of B
+        const long long nnz = h->num_e;
+        SB_CUDA(pool_alloc((void **)&t->t_ptr, sizeof(int) * ((size_t)rows_t + 1), s));
+        SB_CUDA(cudaMemsetAsync(t->t_ptr, 0, sizeof(int) * ((size_t)rows_t + 1), s));
+        t->d_ptr = t->t_ptr;
+        t->num_v = rows_t;
+        t->b_rows = h->num_v;   // A^T gathers rows of dC, which has as many rows as A
+        if (nnz == 0) return 0;
         // a column outside [0, rows_t) would corrupt the histogram: same check as preprocess
-        int h_bad = 0;
-        TR_CUDA(pool_alloc((void **)&bad, sizeof(int), s));
-        TR_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), s));
-        int rc = launch_check_cols(h->d_idx, nnz, rows_t, bad, s);
-        if (rc) return fail(rc);
-        TR_CUDA(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
-        TR_CUDA(cudaStreamSynchronize(s));
+        int *bad = nullptr, *row_of = nullptr, *pos = nullptr, *keys_out = nullptr, h_bad = 0;
+        void *tmp = nullptr;
+        SB_CUDA(scratch.alloc(&bad, sizeof(int)));
+        SB_CUDA(cudaMemsetAsync(bad, 0, sizeof(int), s));
+        const int rc = launch_check_cols(h->d_idx, nnz, rows_t, bad, s);
+        if (rc) return rc;
+        SB_CUDA(cudaMemcpyAsync(&h_bad, bad, sizeof(int), cudaMemcpyDeviceToHost, s));
+        SB_CUDA(cudaStreamSynchronize(s));
         if (h_bad) {
             set_error("CSR idx holds a column outside [0, %d)", rows_t);
-            return fail(SPMM_B200_EINVAL);
+            return SPMM_B200_EINVAL;
         }
-        TR_CUDA(pool_alloc((void **)&row_of, sizeof(int) * (size_t)nnz, s));
-        TR_CUDA(pool_alloc((void **)&pos, sizeof(int) * (size_t)nnz, s));
-        TR_CUDA(pool_alloc((void **)&keys_out, sizeof(int) * (size_t)nnz, s));
+        SB_CUDA(scratch.alloc(&row_of, sizeof(int) * (size_t)nnz));
+        SB_CUDA(scratch.alloc(&pos, sizeof(int) * (size_t)nnz));
+        SB_CUDA(scratch.alloc(&keys_out, sizeof(int) * (size_t)nnz));
         // ptr of A^T: counts shifted by one, then an inclusive scan in place == exclusive scan of the counts
-        col_histogram_kernel<<<grid_for(nnz), 256, 0, s>>>(h->d_idx, nnz, t->t_ptr + 1);
-        TR_CUDA(cudaGetLastError());
+        col_histogram_kernel<<<stride_grid(nnz), 256, 0, s>>>(h->d_idx, nnz, t->t_ptr + 1);
+        SB_CUDA(cudaGetLastError());
         size_t scan_bytes = 0, sort_bytes = 0;
-        TR_CUDA(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, t->t_ptr + 1, t->t_ptr + 1, rows_t, s));
-        int bits = 1;
-        while (bits < 31 && (1ll << bits) < (long long)rows_t) ++bits;
-        TR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, h->d_idx, keys_out, pos, t->t_perm, (int)nnz, 0, bits, s));
-        TR_CUDA(pool_alloc(&tmp, std::max(scan_bytes, sort_bytes), s));
-        TR_CUDA(cub::DeviceScan::InclusiveSum(tmp, scan_bytes, t->t_ptr + 1, t->t_ptr + 1, rows_t, s));
+        SB_CUDA(cub::DeviceScan::InclusiveSum(nullptr, scan_bytes, t->t_ptr + 1, t->t_ptr + 1, rows_t, s));
+        const int bits = key_bits(rows_t);
+        SB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, h->d_idx, keys_out, pos, t->t_perm, (int)nnz, 0, bits, s));
+        SB_CUDA(scratch.alloc(&tmp, std::max(scan_bytes, sort_bytes)));
+        SB_CUDA(cub::DeviceScan::InclusiveSum(tmp, scan_bytes, t->t_ptr + 1, t->t_ptr + 1, rows_t, s));
         const long long threads = (long long)h->num_v * 32;
         if (h->num_v > 0) expand_rows_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(h->d_ptr, h->num_v, row_of, pos);
-        TR_CUDA(cudaGetLastError());
+        SB_CUDA(cudaGetLastError());
         // stable: equal columns keep A's storage order, i.e. ascending row of A
-        TR_CUDA(cub::DeviceRadixSort::SortPairs(tmp, sort_bytes, h->d_idx, keys_out, pos, t->t_perm, (int)nnz, 0, bits, s));
-        gather_t_kernel<<<grid_for(nnz), 256, 0, s>>>(t->t_perm, row_of, h->d_val, nnz, t->t_idx, t->t_val);
-        TR_CUDA(cudaGetLastError());
-    }
-    TR_CUDA(cudaStreamSynchronize(s));
-#undef TR_CUDA
-    drop_scratch();
-    t->d_ptr = t->t_ptr;
-    t->d_idx = t->t_idx;
-    t->d_val = t->t_val;
-    t->num_v = rows_t;
-    t->num_e = (int)nnz;
-    t->feat = feat_in;
-    t->b_rows = h->num_v;   // A^T gathers rows of dC, which has as many rows as A
-    t->t_src = h;
-    *out = t;
-    return 0;
+        SB_CUDA(cub::DeviceRadixSort::SortPairs(tmp, sort_bytes, h->d_idx, keys_out, pos, t->t_perm, (int)nnz, 0, bits, s));
+        gather_t_kernel<<<stride_grid(nnz), 256, 0, s>>>(t->t_perm, row_of, h->d_val, nnz, t->t_idx, t->t_val);
+        SB_CUDA(cudaGetLastError());
+        return 0;
+    });
 }
 
 // The column-sorted operator: a second handle over the SAME matrix whose rows are stored in ascending column order
@@ -177,72 +194,31 @@ extern "C" int spmm_b200_create_transposed(spmm_b200_t h, int feat_in, void *str
 // column order, i.e. they equal the reference run on the sorted CSR bit for bit and the reference run on the original
 // order within the split-row tolerance. Shares ptr with `h` (borrowed), owns idx / val / perm (pool.cu).
 extern "C" int spmm_b200_create_column_sorted(spmm_b200_t h, int feat_in, void *stream, spmm_b200_t *out) {
-    if (!h || !out || feat_in < 0) {
-        set_error("spmm_b200_create_column_sorted: bad arguments");
-        return SPMM_B200_EINVAL;
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    const long long nnz = h->num_e;
-    spmm_b200_handle *t = new (std::nothrow) spmm_b200_handle();
-    if (!t) {
-        set_error("spmm_b200_create_column_sorted: out of host memory");
-        return SPMM_B200_ENOMEM;
-    }
-    unsigned long long *key_in = nullptr, *key_out = nullptr;
-    int *pos = nullptr;
-    void *tmp = nullptr;
-    auto drop_scratch = [&]() {
-        pool_free(key_in, s);
-        pool_free(key_out, s);
-        pool_free(pos, s);
-        pool_free(tmp, s);
-    };
-    auto fail = [&](int rc) {
-        cudaStreamSynchronize(s);
-        cudaGetLastError();
-        drop_scratch();
-        spmm_b200_destroy(t);
-        return rc;
-    };
-#define TR_CUDA(call)                                                                    \
-    do {                                                                                 \
-        cudaError_t e__ = (call);                                                        \
-        if (e__ != cudaSuccess) return fail(cuda_fail(e__, #call, __FILE__, __LINE__)); \
-    } while (0)
-    TR_CUDA(cudaGetDevice(&t->t_device));
-    const size_t cnt = (size_t)std::max<long long>(1, nnz);
-    TR_CUDA(pool_alloc((void **)&t->t_idx, sizeof(int) * cnt, s));
-    TR_CUDA(pool_alloc((void **)&t->t_val, sizeof(float) * cnt, s));
-    TR_CUDA(pool_alloc((void **)&t->t_perm, sizeof(int) * cnt, s));
-    if (nnz > 0) {
-        TR_CUDA(pool_alloc((void **)&key_in, sizeof(unsigned long long) * cnt, s));
-        TR_CUDA(pool_alloc((void **)&key_out, sizeof(unsigned long long) * cnt, s));
-        TR_CUDA(pool_alloc((void **)&pos, sizeof(int) * cnt, s));
+    return create_derived(h, feat_in, stream, out, "spmm_b200_create_column_sorted", [&](spmm_b200_handle *t, Scratch &scratch) {
+        cudaStream_t s = scratch.s;
+        const long long nnz = h->num_e;
+        t->d_ptr = h->d_ptr;   // same rows, same lengths
+        t->num_v = h->num_v;
+        t->b_rows = h->b_rows;
+        if (nnz == 0) return 0;
+        unsigned long long *key_in = nullptr, *key_out = nullptr;
+        int *pos = nullptr;
+        void *tmp = nullptr;
+        SB_CUDA(scratch.alloc(&key_in, sizeof(unsigned long long) * (size_t)nnz));
+        SB_CUDA(scratch.alloc(&key_out, sizeof(unsigned long long) * (size_t)nnz));
+        SB_CUDA(scratch.alloc(&pos, sizeof(int) * (size_t)nnz));
         const long long threads = (long long)h->num_v * 32;
         row_col_keys_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(h->d_ptr, h->d_idx, h->num_v, key_in, pos);
-        TR_CUDA(cudaGetLastError());
-        int row_bits = 1;
-        while (row_bits < 31 && (1ll << row_bits) < (long long)h->num_v) ++row_bits;
+        SB_CUDA(cudaGetLastError());
+        const int bits = 32 + key_bits(h->num_v);
         size_t sort_bytes = 0;
-        TR_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, key_in, key_out, pos, t->t_perm, (int)nnz, 0, 32 + row_bits, s));
-        TR_CUDA(pool_alloc(&tmp, sort_bytes, s));
+        SB_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, key_in, key_out, pos, t->t_perm, (int)nnz, 0, bits, s));
+        SB_CUDA(scratch.alloc(&tmp, sort_bytes));
         // stable: nonzeros of one row with the same column keep their storage order
-        TR_CUDA(cub::DeviceRadixSort::SortPairs(tmp, sort_bytes, key_in, key_out, pos, t->t_perm, (int)nnz, 0, 32 + row_bits, s));
+        SB_CUDA(cub::DeviceRadixSort::SortPairs(tmp, sort_bytes, key_in, key_out, pos, t->t_perm, (int)nnz, 0, bits, s));
         // idx_sorted[k] = idx[perm[k]], val_sorted[k] = val[perm[k]]
-        gather_t_kernel<<<grid_for(nnz), 256, 0, s>>>(t->t_perm, h->d_idx, h->d_val, nnz, t->t_idx, t->t_val);
-        TR_CUDA(cudaGetLastError());
-    }
-    TR_CUDA(cudaStreamSynchronize(s));
-#undef TR_CUDA
-    drop_scratch();
-    t->d_ptr = h->d_ptr;   // same rows, same lengths
-    t->d_idx = t->t_idx;
-    t->d_val = t->t_val;
-    t->num_v = h->num_v;
-    t->num_e = (int)nnz;
-    t->feat = feat_in;
-    t->b_rows = h->b_rows;
-    t->t_src = h;
-    *out = t;
-    return 0;
+        gather_t_kernel<<<stride_grid(nnz), 256, 0, s>>>(t->t_perm, h->d_idx, h->d_val, nnz, t->t_idx, t->t_val);
+        SB_CUDA(cudaGetLastError());
+        return 0;
+    });
 }

@@ -29,6 +29,14 @@ def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
 
+def _check_tensor(name, t, n, dtype=torch.float32, cuda=True):
+    """Raises ValueError naming `name` unless t is a contiguous tensor of `dtype` with >= n elements, on a CUDA device
+    (cuda=True) or on the host (cuda=False)."""
+    if t.is_cuda != cuda or t.dtype != dtype or not t.is_contiguous() or t.numel() < n:
+        kind, dt = "CUDA" if cuda else "host", str(dtype).removeprefix("torch.")
+        raise ValueError(f"{name}: need a contiguous {kind} {dt} tensor of >= {n} elements")
+
+
 @dataclass
 class CSR:
     """struct CSR: device pointers, int32 indices (util.h:120-129)."""
@@ -40,11 +48,9 @@ class CSR:
     val: torch.Tensor  # float32[num_e]
 
     def __post_init__(self):
-        for name, t, dt, n in (("ptr", self.ptr, torch.int32, self.num_v + 1),
-                               ("idx", self.idx, torch.int32, self.num_e),
-                               ("val", self.val, torch.float32, self.num_e)):
-            if not t.is_cuda or t.dtype != dt or not t.is_contiguous() or t.numel() < n:
-                raise ValueError(f"CSR.{name}: need a contiguous CUDA {dt} tensor of >= {n} elements")
+        _check_tensor("CSR.ptr", self.ptr, self.num_v + 1, torch.int32)
+        _check_tensor("CSR.idx", self.idx, self.num_e, torch.int32)
+        _check_tensor("CSR.val", self.val, self.num_e)
 
 
 class SpMM:
@@ -87,10 +93,13 @@ class SpMMB200(SpMM):
         super().set_feat(feat_in)
         check(lib.spmm_b200_set_feat(self._h, self.feat_in))
 
-    def _check_io(self, vin, vout):
-        for name, t, n in (("vin", vin, self.b_rows * self.feat_in), ("vout", vout, self.num_v * self.feat_in)):
-            if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < n:
-                raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {n} elements")
+    def _check_io(self, vin, vout, prefix="", cuda=True):
+        _check_tensor(prefix + "vin", vin, self.b_rows * self.feat_in, cuda=cuda)
+        _check_tensor(prefix + "vout", vout, self.num_v * self.feat_in, cuda=cuda)
+
+    def _check_edges(self, **arrays):
+        for name, t in arrays.items():
+            _check_tensor(name, t, self.num_e)
 
     def set_gather(self, targets, row_offset: int, multicast: int = 0) -> None:
         """Stacked-layer epilogue: finished C rows also go to `targets` (device pointers as ints, or CUDA
@@ -101,39 +110,36 @@ class SpMMB200(SpMM):
 
     def preprocess(self, vin, vout) -> None:
         self._check_io(vin, vout)
-        check(lib.spmm_b200_preprocess(self._h, _ptr(vin), _ptr(vout), _stream()))
+        self._plan()
 
-    def transposed(self, feat_in: int | None = None, **options) -> "SpMMB200":
-        """The operator over A^T (spmm_b200_create_transposed): run(dC[num_v x K], dB[b_rows x K]) computes the gradient
-        of this operator with respect to its input. The new operator owns its CSR; close it before this one."""
+    def _plan(self) -> None:
+        """preprocess without vin / vout: the library takes them as hints only and reads neither."""
+        check(lib.spmm_b200_preprocess(self._h, None, None, _stream()))
+
+    def _derived(self, create, num_v: int, b_rows: int, feat_in: int | None, options: dict) -> "SpMMB200":
+        """The operator that the C constructor `create` builds from this one's handle, with the given shape."""
         t = object.__new__(SpMMB200)
         t.g = None
-        t.num_e = self.num_e
-        t.num_v, t.b_rows = self.b_rows, self.num_v
+        t.num_v, t.num_e, t.b_rows = num_v, self.num_e, b_rows
         t.feat_in = self.feat_in if feat_in is None else int(feat_in)
         h = C.c_void_p()
-        check(lib.spmm_b200_create_transposed(self._h, t.feat_in, _stream(), C.byref(h)))
+        check(create(self._h, t.feat_in, _stream(), C.byref(h)))
         t._h = h
         t._parent = self   # keeps the source operator (and the arrays it borrows) alive
         for k, v in options.items():
             t.set_option(k, v)
         return t
 
+    def transposed(self, feat_in: int | None = None, **options) -> "SpMMB200":
+        """The operator over A^T (spmm_b200_create_transposed): run(dC[num_v x K], dB[b_rows x K]) computes the gradient
+        of this operator with respect to its input. The new operator owns its CSR; close it before this one."""
+        return self._derived(lib.spmm_b200_create_transposed, self.b_rows, self.num_v, feat_in, options)
+
     def column_sorted(self, feat_in: int | None = None, **options) -> "SpMMB200":
         """The operator over the same matrix with every row in ascending column order (spmm_b200_create_column_sorted): for
         CSR inputs whose rows are not column-sorted, which otherwise stay in one column block. Results associate in column
         order. The new operator borrows ptr, owns idx / val; close it before this one."""
-        t = object.__new__(SpMMB200)
-        t.g = None
-        t.num_e, t.num_v, t.b_rows = self.num_e, self.num_v, self.b_rows
-        t.feat_in = self.feat_in if feat_in is None else int(feat_in)
-        h = C.c_void_p()
-        check(lib.spmm_b200_create_column_sorted(self._h, t.feat_in, _stream(), C.byref(h)))
-        t._h = h
-        t._parent = self   # the C side copies b_rows from the source handle
-        for k, v in options.items():
-            t.set_option(k, v)
-        return t
+        return self._derived(lib.spmm_b200_create_column_sorted, self.num_v, self.b_rows, feat_in, options)
 
     def refresh_values(self) -> None:
         """Re-stage the plan's copy of idx/val after the caller changed them in place (same ptr)."""
@@ -148,23 +154,17 @@ class SpMMB200(SpMM):
         position p — on an operator from transposed() / column_sorted(), a position of the source operator, whose num_e
         values val holds. Needs the option live_values=1. Asynchronous on the current stream."""
         self._check_io(vin, vout)
-        self._check_dense("val", val, self.num_e)
+        _check_tensor("val", val, self.num_e)
         check(lib.spmm_b200_run_values(self._h, _ptr(val), _ptr(vin), _ptr(vout), _stream()))
 
     def sddmm(self, x_row, x_col, out) -> None:
         """SDDMM over this operator's pattern (spmm_b200_sddmm): out[e] = <x_row[row(e)], x_col[idx[e]]> for every
         nonzero e, in CSR position order. x_row: num_v x feat_in, x_col: b_rows x feat_in, out: >= num_e floats.
         With x_row = dC and x_col = B, out is dL/dval of C = A·B. Asynchronous on the current stream."""
-        for name, t, n in (("x_row", x_row, self.num_v * self.feat_in), ("x_col", x_col, self.b_rows * self.feat_in),
-                           ("out", out, self.num_e)):
-            if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < n:
-                raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {n} elements")
+        _check_tensor("x_row", x_row, self.num_v * self.feat_in)
+        _check_tensor("x_col", x_col, self.b_rows * self.feat_in)
+        _check_tensor("out", out, self.num_e)
         check(lib.spmm_b200_sddmm(self._h, _ptr(x_row), _ptr(x_col), _ptr(out), _stream()))
-
-    def _check_edges(self, **arrays):
-        for name, t in arrays.items():
-            if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < self.num_e:
-                raise ValueError(f"{name}: need a contiguous CUDA float32 tensor of >= {self.num_e} elements")
 
     def edge_softmax(self, scores, out) -> None:
         """Softmax over each row's nonzeros (spmm_b200_edge_softmax), in CSR position order: out[e] = exp(s[e] - m_r) /
@@ -181,11 +181,6 @@ class SpMMB200(SpMM):
 
     REDUCE_OPS = {"amax": 1, "amin": 2}   # SPMM_B200_REDUCE_AMAX / _AMIN
 
-    @staticmethod
-    def _check_dense(name, t, n, dtype=torch.float32):
-        if not t.is_cuda or t.dtype != dtype or not t.is_contiguous() or t.numel() < n:
-            raise ValueError(f"{name}: need a contiguous CUDA {dtype} tensor of >= {n} elements")
-
     def reduce(self, op: str, vin, vout, arg=None) -> None:
         """amax / amin aggregation over this operator's rows (spmm_b200_reduce): vout[r, j] = the winning message
         val[e] * vin[idx[e], j] over the nonzeros e of row r, arg[r, j] = e (int32, optional). NaN wins; ties go to the
@@ -193,10 +188,9 @@ class SpMMB200(SpMM):
         Reads the current g.val (no refresh_values needed). Asynchronous on the current stream."""
         if op not in self.REDUCE_OPS:
             raise ValueError(f"reduce: op must be one of {sorted(self.REDUCE_OPS)}, got {op!r}")
-        self._check_dense("vin", vin, self.b_rows * self.feat_in)
-        self._check_dense("vout", vout, self.num_v * self.feat_in)
+        self._check_io(vin, vout)
         if arg is not None:
-            self._check_dense("arg", arg, self.num_v * self.feat_in, torch.int32)
+            _check_tensor("arg", arg, self.num_v * self.feat_in, torch.int32)
         check(lib.spmm_b200_reduce(self._h, self.REDUCE_OPS[op], _ptr(vin), _ptr(vout), _ptr(arg), _stream()))
 
     def reduce_backward(self, dc, arg, db=None, dval=None, vin=None) -> None:
@@ -205,15 +199,15 @@ class SpMMB200(SpMM):
         each optional, from dC and the forward's arg (both the source's num_v x feat_in). vin (the forward's B) is
         needed only with dval. Asynchronous on the current stream."""
         src_rows = self.b_rows   # this operator is Aᵀ: its b_rows are the source's rows
-        self._check_dense("dc", dc, src_rows * self.feat_in)
-        self._check_dense("arg", arg, src_rows * self.feat_in, torch.int32)
+        _check_tensor("dc", dc, src_rows * self.feat_in)
+        _check_tensor("arg", arg, src_rows * self.feat_in, torch.int32)
         if db is not None:
-            self._check_dense("db", db, self.num_v * self.feat_in)
+            _check_tensor("db", db, self.num_v * self.feat_in)
         if dval is not None:
-            self._check_dense("dval", dval, self.num_e)
+            _check_tensor("dval", dval, self.num_e)
             if vin is None:
                 raise ValueError("reduce_backward: dval needs vin (the forward's B)")
-            self._check_dense("vin", vin, self.num_v * self.feat_in)
+            _check_tensor("vin", vin, self.num_v * self.feat_in)
         check(lib.spmm_b200_reduce_backward(self._h, _ptr(dc), _ptr(arg), _ptr(vin), _ptr(db), _ptr(dval), _stream()))
 
     def run_profiled(self, vin, vout) -> float:
@@ -225,9 +219,7 @@ class SpMMB200(SpMM):
 
     def run_host(self, h_vin: torch.Tensor, h_vout: torch.Tensor) -> None:
         """H2D(vin) -> run -> D2H(vout) -> sync, host (ideally pinned) float32 tensors."""
-        for name, t, n in (("h_vin", h_vin, self.b_rows * self.feat_in), ("h_vout", h_vout, self.num_v * self.feat_in)):
-            if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < n:
-                raise ValueError(f"{name}: need a contiguous host float32 tensor of >= {n} elements")
+        self._check_io(h_vin, h_vout, "h_", cuda=False)
         check(lib.spmm_b200_run_host(self._h, C.c_void_p(h_vin.data_ptr()), C.c_void_p(h_vout.data_ptr()),
                                      _stream()))
 
@@ -242,9 +234,7 @@ class SpMMB200(SpMM):
         """Collective over the ranks: upload this rank's share of B (h_vin is the whole B on the host), replicate it
         over NVLink, run, deliver the local block of C into h_vout, synchronise (spmm_b200_run_host_sharded).
         Returns the host-to-device bytes this rank copied."""
-        for name, t, n in (("h_vin", h_vin, self.b_rows * self.feat_in), ("h_vout", h_vout, self.num_v * self.feat_in)):
-            if t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous() or t.numel() < n:
-                raise ValueError(f"{name}: need a contiguous host float32 tensor of >= {n} elements")
+        self._check_io(h_vin, h_vout, "h_", cuda=False)
         check(lib.spmm_b200_run_host_sharded(self._h, C.c_void_p(h_vin.data_ptr()), C.c_void_p(h_vout.data_ptr()), _stream()))
         return int(lib.spmm_b200_replicate_h2d_bytes(self._h))
 
@@ -310,8 +300,7 @@ def trim_memory() -> None:
 
 def fill_normal(t: torch.Tensor, seed: int, stream_id: int, mean: float = 0.0, stddev: float = 0.1) -> torch.Tensor:
     """Counter-based N(mean, stddev) fill (the engine's stand-in for curandGenerateNormal, data.h:31)."""
-    if not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous():
-        raise ValueError("fill_normal: need a contiguous CUDA float32 tensor")
+    _check_tensor("fill_normal: t", t, 0)
     check(lib.spmm_b200_fill_normal(_ptr(t), t.numel(), seed, stream_id, mean, stddev, _stream()))
     return t
 

@@ -85,8 +85,7 @@ def bench(name, steps):
     g = H.CSR(M, nnz, torch.from_numpy(ptr).cuda(), torch.from_numpy(idx).cuda(), H.fill_normal(torch.empty(nnz, device=dev), 123, 1))
     q, k, v, w = (H.fill_normal(torch.empty(M * K, device=dev), 123, 2 + i).reshape(M, K) for i in range(4))
     att = H.GraphAttention(g, K)
-    op = att.op
-    t = att.transposed()   # plans the forward operator, then the transposed one
+    op, t = att._op(), att.transposed()   # both planned
     s = torch.empty(nnz, device=dev)
     op.sddmm(q, k, s)
     dp = H.fill_normal(torch.empty(nnz, device=dev), 123, 7)
